@@ -25,6 +25,9 @@ Beside the main line's keys the JSON carries:
 contiguous time spans (strong scaling: the whole job is fixed), encode + full-tile window decode.
 
 --impl reference times the oracle on all host cores (one full 64-instant slice of the 721x1440 grid per worker).
+
+--dump-outputs DIR writes a seeded sample of the last timed step's result as .npy files (see dump_outputs); the inputs
+are the same on every run with the same arguments, so two builds of the project can be compared output for output.
 """
 import argparse
 import json
@@ -293,6 +296,35 @@ def encode_leg(ctx, data, levels, steps, warmup, world, dev, stream, clock_index
             "clocks": sampler.summary() if sampler else None}
 
 
+def dump_outputs(sc, out_dir, n_bytes=8192, n_cells=1 << 18, seed=0xDCDF0D):
+    """Writes what the last timed Superchunk.build returned as .npy files, so that two builds of the project can be
+    compared output for output: every slice's info and root-node references, a sample of its stored bytes, and the
+    values decoded at a sample of cells.  Sample positions depend on `seed` and the sizes alone; about 25 MB for the
+    workload's 137 slices."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(seed)
+    info, refs, sample = [], [], []
+    for s in range(sc.n_slices):
+        i = sc.info(s)
+        st = i.stats
+        info.append([*i.shape, i.sidelen, i.chunks_sidelen, i.subsidelen, i.levels, i.encoding, i.fractional_bits, i.n_refs,
+                     i.max_dac_bytes, i.min_dac_bytes, i.chunk_bytes, st.size, st.elided, st.local, st.external, st.snapshots, st.logs])
+        refs.append(np.stack(sc.refs(s), axis=1))  # per subchunk slot: kind, offset, size, fractional bits
+        for which in range(3):  # the slice's stored Chunks back to back, its max DAC, its min DAC
+            blob = np.frombuffer(sc.bytes(s, which), np.uint8)
+            at = (rng.random(n_bytes) * len(blob)).astype(np.int64)
+            sample.append(blob[at] if len(blob) else np.zeros(n_bytes, np.uint8))
+    T, rows, cols = sc.shape
+    irc = np.stack([rng.integers(0, n, n_cells) for n in (T, rows, cols)], axis=1)
+    outputs = {"slice_info": np.array(info, np.float64), "root_refs": np.stack(refs).astype(np.float64),
+               "stored_bytes_sample": np.stack(sample).reshape(sc.n_slices, 3, n_bytes).astype(np.float32),
+               "cells_sample_irc": irc.astype(np.float64), "cells_sample_values": sc.get_batch(irc).astype(np.float32)}
+    for name, a in outputs.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+    return {"dir": out_dir, "bytes": int(sum(a.nbytes for a in outputs.values()))}
+
+
 def decode_leg(ctx, sc, data, tspan, stream, s_out_total, T_total, peak, reps=3):
     """Full-extent window decode of the first `tspan` instants, f32 output resident in HBM, checked against the input."""
     import torch
@@ -413,6 +445,8 @@ def run_ours(args):
     free, total = torch.cuda.mem_get_info(dev)
     need = 4 * T * rows * cols * 2.2
     if need > free:
+        if args.dump_outputs:  # a shorter raster would make the outputs incomparable with another run's
+            raise SystemExit(f"--dump-outputs: {T} instants need {need / 1e9:.0f} GB, {free / 1e9:.0f} GB free on {dev}")
         T = int(free / (4 * rows * cols * 2.2)) // CHUNK_SIZE * CHUNK_SIZE
     raw_bytes = 4 * T * rows * cols
     data = torch.empty((T, rows, cols), device=dev, dtype=torch.float32)
@@ -432,6 +466,7 @@ def run_ours(args):
     step_ms = _max_over_ranks(enc["step_ms"], world, dev)
     total_raw = _sum_over_ranks(raw_bytes, world, dev)
     value = total_raw / (step_ms * 1e-3) / 1e9
+    dumped = dump_outputs(sc, args.dump_outputs) if args.dump_outputs and rank == 0 else None
 
     # ---- CPU path beside it (rank 0, N == 1): one slice through the oracle, all four legs + sector densities
     cpu, oracle_ref, oracle_search = None, None, None
@@ -657,7 +692,7 @@ def run_ours(args):
                          "frac_of_whole_step": algo / (step_ms * 1e-3) / 1e9 / peak},
             "cpu_baseline": (dict(cpu["encode"], decode=cpu.get("decode"), cell=cpu.get("cell"), search=cpu.get("search")) if cpu and "encode" in cpu else cpu),
             "e2e": e2e, "decode": dec, "queries": queries, "extras": extras, "gpu_launches": int(enc["launches"]), "clocks": enc["clocks"],
-            "wall_ms_per_step": enc["wall_ms"], "device_ms_per_step": enc["dev_ms"],
+            "wall_ms_per_step": enc["wall_ms"], "device_ms_per_step": enc["dev_ms"], "dumped_outputs": dumped,
         }
         try:  # DRAM traffic of the dominant kernel from the committed ncu capture (bytes per (unit, instant)), scaled to this launch
             tj = json.load(open(os.path.join(ROOT, "profiles", "r2_traffic.json")))
@@ -782,7 +817,13 @@ def main():
     ap.add_argument("--c5-slab-slices", type=int, default=18)
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write a seeded sample of what the last "
+                    "step's Superchunk.build returned (rank 0) to DIR/<name>.npy; default config and impl only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.config != "c2"):
+        ap.error("--dump-outputs applies to the default --impl ours --config c2 run")
     if args.no_e2e:
         args.sections = ",".join(s for s in args.sections.split(",") if s != "e2e")
     if args.no_cpu:

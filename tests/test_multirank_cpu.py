@@ -1,6 +1,7 @@
 """world_size-2 gloo test of the N > 1 host logic of bench.py (no GPU): every rank owns an independent time
 span, nothing is exchanged on the data path, and only the timing / byte totals are reduced."""
 import os
+import socket
 import sys
 
 import torch
@@ -30,9 +31,12 @@ def _worker(rank, world, port, out):
 
 def test_two_rank_reduction_of_timings_and_totals():
     world = 2
+    with socket.socket() as s:  # a free port chosen by the OS: a fixed one may be taken on a shared machine
+        s.bind(("127.0.0.1", 0))
+        port = s.getsockname()[1]
     with mp.Manager() as m:
         out = m.dict()
-        mp.spawn(_worker, args=(world, 29731, out), nprocs=world, join=True)
+        mp.spawn(_worker, args=(world, port, out), nprocs=world, join=True)
         res = dict(out)
     assert res[0] == res[1] == (15.0, 2 * 4 * 40 * 50 * 4.0)   # max over ranks, whole-job bytes
 
