@@ -111,6 +111,7 @@ def _declare(lib):
         "dcdf_superchunk_window": (i32, [vp, vp, _P(Cube), vp, i32, i32]),
         "dcdf_superchunk_window_batch": (i32, [vp, vp, u64, vp, vp, vp, i32, i32]),
         "dcdf_superchunk_search_batch": (i32, [vp, vp, u64, vp, vp, vp, vp, vp, u64, _P(u64), i32]),
+        "dcdf_superchunk_search_values": (i32, [vp, vp, u64, vp, vp, vp, vp, vp, u64, _P(u64), i32]),
         "dcdf_superchunk_save": (i32, [vp, vp, u32, _P(vp)]),
         "dcdf_saved_free": (i32, [vp]),
         "dcdf_saved_count": (i32, [vp, _P(u32)]),

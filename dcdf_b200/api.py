@@ -3,6 +3,7 @@
 Names and argument meaning follow the reference (paths relative to dcdf/src):
   Chunk.build / get / fill_cell / fill_window / iter_search / write_to / read_from   chunk.rs:42-278
   Superchunk.build / get / fill_cell / fill_window / search                          superchunk.rs:88-585
+  Superchunk.search_values (float bounds; mmarray.rs:407-417 is todo!() upstream)
   MMArray3.{shape,get,cell,window,search}                                            mmarray.rs:135-536,
                                                                 py-dcdf/src/lib.rs:411-581 (PyMMArray3*)
   to_fixed / from_fixed / suggest_fraction                                           fixed.rs:31-159
@@ -459,13 +460,27 @@ class Superchunk(_Queryable):
         return out, off
 
     def search_batch(self, cubes, lower, upper, want_cells=True):
+        return self._search(self.ctx._lib.dcdf_superchunk_search_batch, np.int64, cubes, lower, upper, want_cells)
+
+    def search(self, start, end, top, bottom, left, right, lower, upper):
+        return self.search_batch([[start, end, top, bottom, left, right]], lower, upper)[1]
+
+    def search_values_batch(self, cubes, lower, upper, want_cells=True):
+        """Value-range search with bounds in the array's own units (dcdf_superchunk_search_values): the cells whose decoded
+        value v has lower <= v <= upper, NaN never; exact where search_batch follows the reference's traversal.  Per window
+        counts and the (instant, row, col) cells, window after window."""
+        return self._search(self.ctx._lib.dcdf_superchunk_search_values, np.float64, cubes, lower, upper, want_cells)
+
+    def search_values(self, start, end, top, bottom, left, right, lower, upper):
+        return self.search_values_batch([[start, end, top, bottom, left, right]], lower, upper)[1]
+
+    def _search(self, fn, bound_type, cubes, lower, upper, want_cells):
         cubes = np.ascontiguousarray(cubes, dtype=np.int64).reshape(-1, 6)
         n = len(cubes)
-        lo = np.ascontiguousarray(np.broadcast_to(np.asarray(lower, np.int64), (n,)))
-        hi = np.ascontiguousarray(np.broadcast_to(np.asarray(upper, np.int64), (n,)))
+        lo = np.ascontiguousarray(np.broadcast_to(np.asarray(lower, bound_type), (n,)))
+        hi = np.ascontiguousarray(np.broadcast_to(np.asarray(upper, bound_type), (n,)))
         counts = np.zeros(n, np.uint64)
         found = C.c_uint64()
-        fn = self.ctx._lib.dcdf_superchunk_search_batch
         self.ctx.check(fn(self.ctx._h, self._h, n, _ptr(cubes), _ptr(lo), _ptr(hi), _ptr(counts), None, 0, C.byref(found), MEM_HOST))
         if not want_cells:
             return counts, None
@@ -473,9 +488,6 @@ class Superchunk(_Queryable):
         if found.value:
             self.ctx.check(fn(self.ctx._h, self._h, n, _ptr(cubes), _ptr(lo), _ptr(hi), _ptr(counts), _ptr(out), found.value, C.byref(found), MEM_HOST))
         return counts, out
-
-    def search(self, start, end, top, bottom, left, right, lower, upper):
-        return self.search_batch([[start, end, top, bottom, left, right]], lower, upper)[1]
 
     def close(self):
         if getattr(self, "_h", None):

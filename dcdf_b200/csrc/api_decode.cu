@@ -241,7 +241,7 @@ MetaBlock* super_meta(dcdf_ctx* ctx, const dcdf_superchunk* scc) {
           const u64 tbl0 = sc->slices[s].table_base + (u64)nd.tbl_off * (u64)m.instants + c;
           if (ch.kind == 2 && sc->nstate[s * n_nodes + ch.index].alive) {
             if (d.n_up >= 3) api_fail(DCDF_ERR_BAD_ARG, "superchunks nested more than four levels deep are not supported by the query kernels");
-            d.up_tbl0[d.n_up] = tbl0; d.up_stride[d.n_up] = nd.n_children; d.n_up++;
+            d.up_tbl0[d.n_up] = tbl0; d.up_stride[d.n_up] = nd.n_children; d.up_bits[d.n_up] = sc->nstate[s * n_nodes + node].bits; d.n_up++;
             node = (uint32_t)ch.index;
             continue;
           }
@@ -558,11 +558,24 @@ void do_window_batch(dcdf_ctx* ctx, MetaBlock* mb, uint64_t n, const dcdf_cube* 
   tcollect(ctx, KT_WINDOW);
 }
 
+// Fixed-point bounds (lower / upper), or, with strict, value bounds (vlower / vupper) that the kernels convert per subchunk
+// with its own fractional bits, with the exact hit set (the strict kernels: k_search_tiles4 / k_count_tiles4 / k_search
+// with ST = true).
 void do_search_batch(dcdf_ctx* ctx, MetaBlock* mb, uint64_t n, const dcdf_cube* bounds, const int64_t* lower, const int64_t* upper,
-                     uint64_t* counts, int64_t* out_irc, uint64_t cap, uint64_t* n_found, int32_t mem) {
+                     uint64_t* counts, int64_t* out_irc, uint64_t cap, uint64_t* n_found, int32_t mem, bool strict = false,
+                     const double* vlower = nullptr, const double* vupper = nullptr) {
   if (n_found) *n_found = 0;
   if (n == 0) return;
-  if (!bounds || !lower || !upper) api_fail(DCDF_ERR_BAD_ARG, "null search arguments");
+  if (!bounds || (strict ? !vlower || !vupper : !lower || !upper)) api_fail(DCDF_ERR_BAD_ARG, "null search arguments");
+  std::vector<double> vlo, vhi;
+  if (strict) {
+    vlo.assign(vlower, vlower + n);
+    vhi.assign(vupper, vupper + n);
+    for (uint64_t i = 0; i < n; i++) {
+      if (std::isnan(vlo[i]) || std::isnan(vhi[i])) api_fail(DCDF_ERR_BAD_ARG, "NaN search bound in window %llu", (unsigned long long)i);
+      if (vlo[i] > vhi[i]) std::swap(vlo[i], vhi[i]);  // helpers.rs:7-16 via chunk.rs:214
+    }
+  }
   cudaStream_t st = ctx->stream;
   std::vector<CubeDev> cubes(n);
   std::vector<u64> job_base(n + 1);
@@ -591,8 +604,11 @@ void do_search_batch(dcdf_ctx* ctx, MetaBlock* mb, uint64_t n, const dcdf_cube* 
   i64* d_hi = d_lo + n;
   CK(cudaMemcpyAsync(d_c, cubes.data(), sizeof(CubeDev) * n, cudaMemcpyHostToDevice, st));
   CK(cudaMemcpyAsync(d_jb, job_base.data(), sizeof(u64) * (n + 1), cudaMemcpyHostToDevice, st));
-  CK(cudaMemcpyAsync(d_lo, lower, sizeof(i64) * n, cudaMemcpyHostToDevice, st));
-  CK(cudaMemcpyAsync(d_hi, upper, sizeof(i64) * n, cudaMemcpyHostToDevice, st));
+  // the strict search's value bounds take the place of the fixed ones (both 8 bytes a window)
+  CK(cudaMemcpyAsync(d_lo, strict ? (const void*)vlo.data() : (const void*)lower, sizeof(i64) * n, cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(d_hi, strict ? (const void*)vhi.data() : (const void*)upper, sizeof(i64) * n, cudaMemcpyHostToDevice, st));
+  const double* d_vlo = reinterpret_cast<const double*>(d_lo);
+  const double* d_vhi = reinterpret_cast<const double*>(d_hi);
   const u64 n_scan_chunks = (n_jobs + SCAN_CHUNK - 1) / SCAN_CHUNK;
   ctx->query_aux.reserve(sizeof(u64) * (2 * n_jobs + 2) + sizeof(u64) * (n + 1) + sizeof(u64) * (2 * n_scan_chunks + 2));
   u64* d_counts = ctx->query_aux.as<u64>();
@@ -603,7 +619,7 @@ void do_search_batch(dcdf_ctx* ctx, MetaBlock* mb, uint64_t n, const dcdf_cube* 
   SearchParams SP;
   SP.Q = mb->Q;
   SP.cubes = d_c; SP.job_base = d_jb; SP.n_queries = n; SP.n_jobs = n_jobs;
-  SP.lower = d_lo; SP.upper = d_hi;
+  SP.lower = d_lo; SP.upper = d_hi; SP.vlower = d_vlo; SP.vupper = d_vhi;
   SP.counts = d_counts; SP.offsets = d_offsets;
   SP.out = nullptr; SP.cap = 0;
   const unsigned grid = (unsigned)((n_jobs + 127) / 128);
@@ -630,7 +646,7 @@ void do_search_batch(dcdf_ctx* ctx, MetaBlock* mb, uint64_t n, const dcdf_cube* 
     CK(cudaMemcpyAsync(ctx->query_aux2.p, tile_base.data(), sizeof(u64) * (n + 1), cudaMemcpyHostToDevice, st));
     CK(cudaStreamSynchronize(st));  // tile_base is a local
     TS.Q = mb->Q; TS.cubes = d_c; TS.job_base = d_jb; TS.tile_base = ctx->query_aux2.as<u64>();
-    TS.n_queries = n; TS.n_tiles = n_tiles; TS.lower = d_lo; TS.upper = d_hi;
+    TS.n_queries = n; TS.n_tiles = n_tiles; TS.lower = d_lo; TS.upper = d_hi; TS.vlower = d_vlo; TS.vupper = d_vhi;
     TS.counts = d_counts; TS.offsets = d_offsets; TS.out = nullptr; TS.cap = 0;
     // 1 KB per (window, subchunk, instant) keeps the counting pass's findings for the writing pass (up to 2 GB)
     TS.hit_cache = nullptr;
@@ -639,8 +655,13 @@ void do_search_batch(dcdf_ctx* ctx, MetaBlock* mb, uint64_t n, const dcdf_cube* 
       TS.hit_cache = ctx->search_cache.as<u32>();
     }
     tgrid = (unsigned)std::min<u64>(n_tiles, (u64)ctx->sm_count * 64);
-    CK(cudaFuncSetAttribute(k_search_tiles4<i64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Search4Smem<i64>)));
-    CK(cudaFuncSetAttribute(k_search_tiles4<int32_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Search4Smem<int32_t>)));
+    if (strict) {
+      CK(cudaFuncSetAttribute(k_search_tiles4<i64, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Search4Smem<i64>)));
+      CK(cudaFuncSetAttribute(k_search_tiles4<int32_t, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Search4Smem<int32_t>)));
+    } else {
+      CK(cudaFuncSetAttribute(k_search_tiles4<i64, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Search4Smem<i64>)));
+      CK(cudaFuncSetAttribute(k_search_tiles4<int32_t, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Search4Smem<int32_t>)));
+    }
   }
   // Counting pass with shared decodes (k_count_tiles4) when the windows of the batch overlap: every (time slice, tile) some
   // window touches is decoded once for all of them.  Worth it from a few windows per touched tile on (ctx option
@@ -681,9 +702,13 @@ void do_search_batch(dcdf_ctx* ctx, MetaBlock* mb, uint64_t n, const dcdf_cube* 
       std::vector<u64> fill(key_off.begin(), key_off.end() - 1);
       for_each_entry([&](uint64_t q, const CubeDev& c, i64 sl, i64 cr, i64 cc, i64 sub, i64 T_all, u64 key) {
         CountEntry E;
-        i64 lo = lower[q], hi = upper[q];
-        if (lo > hi) std::swap(lo, hi);  // helpers.rs:7-16 via chunk.rs:214
-        E.lower = lo; E.upper = hi;
+        if (strict) {
+          E.vlower = vlo[q]; E.vupper = vhi[q];
+        } else {
+          i64 lo = lower[q], hi = upper[q];
+          if (lo > hi) std::swap(lo, hi);  // helpers.rs:7-16 via chunk.rs:214
+          E.lower = lo; E.upper = hi;
+        }
         const i64 s0 = sl * ct, t_lo = std::max(c.start, s0), t_hi = std::min(c.end, s0 + ct);
         E.t0 = (uint16_t)(t_lo - s0); E.t1 = (uint16_t)(t_hi - s0);
         E.cnt_base = (i64)job_base[q] + sub * T_all + (s0 - c.start);
@@ -704,22 +729,29 @@ void do_search_batch(dcdf_ctx* ctx, MetaBlock* mb, uint64_t n, const dcdf_cube* 
       CK(cudaMemcpyAsync(d_cj, cjobs.data(), b_jobs, cudaMemcpyHostToDevice, st));
       TC.Q = mb->Q; TC.jobs = d_cj; TC.n_jobs = cjobs.size(); TC.entries = d_ent; TC.counts = d_counts;
       cgrid = (unsigned)std::min<u64>(cjobs.size(), (u64)ctx->sm_count * 64);
-      if (narrow) CK(cudaFuncSetAttribute(k_count_tiles4<int32_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Count4Smem<int32_t>)));
-      else CK(cudaFuncSetAttribute(k_count_tiles4<i64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Count4Smem<i64>)));
+      const void* kc = narrow ? (strict ? (const void*)k_count_tiles4<int32_t, true> : (const void*)k_count_tiles4<int32_t, false>)
+                              : (strict ? (const void*)k_count_tiles4<i64, true> : (const void*)k_count_tiles4<i64, false>);
+      CK(cudaFuncSetAttribute(kc, cudaFuncAttributeMaxDynamicSharedMemorySize, narrow ? (int)sizeof(Count4Smem<int32_t>) : (int)sizeof(Count4Smem<i64>)));
       TS.hit_cache = nullptr;  // the shared counting pass keeps no per-thread findings; the buffer holds its entries
     }
   }
   auto launch_search = [&](int write) {
     if (tiles && !write && shared_count) {
       CK(cudaMemsetAsync(d_counts, 0, sizeof(u64) * n_jobs, st));
-      if (narrow) k_count_tiles4<int32_t><<<cgrid, DT_THREADS, sizeof(Count4Smem<int32_t>), st>>>(TC);
-      else k_count_tiles4<i64><<<cgrid, DT_THREADS, sizeof(Count4Smem<i64>), st>>>(TC);
+      if (narrow && strict) k_count_tiles4<int32_t, true><<<cgrid, DT_THREADS, sizeof(Count4Smem<int32_t>), st>>>(TC);
+      else if (narrow) k_count_tiles4<int32_t, false><<<cgrid, DT_THREADS, sizeof(Count4Smem<int32_t>), st>>>(TC);
+      else if (strict) k_count_tiles4<i64, true><<<cgrid, DT_THREADS, sizeof(Count4Smem<i64>), st>>>(TC);
+      else k_count_tiles4<i64, false><<<cgrid, DT_THREADS, sizeof(Count4Smem<i64>), st>>>(TC);
     } else if (tiles) {
       if (!write) CK(cudaMemsetAsync(d_counts, 0, sizeof(u64) * n_jobs, st));  // the counting pass adds per warp
-      if (narrow) k_search_tiles4<int32_t><<<tgrid, DT_THREADS, sizeof(Search4Smem<int32_t>), st>>>(TS);
-      else k_search_tiles4<i64><<<tgrid, DT_THREADS, sizeof(Search4Smem<i64>), st>>>(TS);
+      if (narrow && strict) k_search_tiles4<int32_t, true><<<tgrid, DT_THREADS, sizeof(Search4Smem<int32_t>), st>>>(TS);
+      else if (narrow) k_search_tiles4<int32_t, false><<<tgrid, DT_THREADS, sizeof(Search4Smem<int32_t>), st>>>(TS);
+      else if (strict) k_search_tiles4<i64, true><<<tgrid, DT_THREADS, sizeof(Search4Smem<i64>), st>>>(TS);
+      else k_search_tiles4<i64, false><<<tgrid, DT_THREADS, sizeof(Search4Smem<i64>), st>>>(TS);
+    } else if (strict) {
+      k_search<true><<<grid, 128, 0, st>>>(SP, write);
     } else {
-      k_search<<<grid, 128, 0, st>>>(SP, write);
+      k_search<false><<<grid, 128, 0, st>>>(SP, write);
     }
   };
   tbegin(ctx, KT_SEARCH);
@@ -888,6 +920,15 @@ int32_t dcdf_superchunk_search_batch(dcdf_ctx* ctx, const dcdf_superchunk* sc, u
   return guarded(ctx, [&] {
     if (!sc) api_fail(DCDF_ERR_BAD_ARG, "null superchunk");
     do_search_batch(ctx, super_meta(ctx, sc), n, bounds, lower, upper, counts, out_irc, cap, n_found, mem);
+  });
+}
+
+int32_t dcdf_superchunk_search_values(dcdf_ctx* ctx, const dcdf_superchunk* sc, uint64_t n, const dcdf_cube* bounds,
+                                      const double* lower, const double* upper, uint64_t* counts, int64_t* out_irc,
+                                      uint64_t cap, uint64_t* n_found, int32_t mem) {
+  return guarded(ctx, [&] {
+    if (!sc) api_fail(DCDF_ERR_BAD_ARG, "null superchunk");
+    do_search_batch(ctx, super_meta(ctx, sc), n, bounds, nullptr, nullptr, counts, out_irc, cap, n_found, mem, true, lower, upper);
   });
 }
 

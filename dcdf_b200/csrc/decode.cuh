@@ -60,6 +60,7 @@ struct SlotDesc {
   u64 up_tbl0[3];
   u32 up_stride[3];
   int n_up;
+  int up_bits[3];  // fractional bits of those nodes (their tables are at these bits)
 };
 struct QuerySet {
   const u8* blob;
@@ -546,6 +547,76 @@ DCDF_DEVINL bool slot_has_cells_part(const QuerySet& Q, const SlotDesc& d, i64 t
   return any;
 }
 
+// ------------------------------------------------------------------ value bounds (dcdf_superchunk_search_values)
+// The value the window decoder writes for a code, as a double: from_fixed_dev in the encoding's float type, the stored
+// integer itself for integer encodings.  Code 0 of a float encoding is NaN and never a hit; it is given the value 0 here,
+// which lies between the values of codes -1 and 1, so that the map stays monotone non-decreasing in the code
+// (fixed.rs:81-86) and the codes of any value interval form one interval.  INT64_MIN, where n - 1 would wrap, takes the
+// value of INT64_MIN + 1.
+DCDF_DEVINL double code_value(i64 n, int bits, int enc) {
+  if (enc == 4 || enc == 8) return (double)n;
+  if (n == 0) return 0.0;
+  if (n == INT64_MIN) n++;
+  return enc == 32 ? (double)from_fixed_dev<float>(n, bits) : from_fixed_dev<double>(n, bits);
+}
+// Fixed-point band of the value interval [lo, hi] at `bits` fractional bits: a code n is a hit iff lower <= n <= upper
+// and not (nz && n == 0).  Both ends by binary search over all of i64 with code_value itself -- a closed form such as
+// 2 ceil(lo 2^bits) + 1 misses when the float rounding of n - 1 maps many codes to one value (codes past 2^24 in f32).
+struct FixedBand {
+  i64 lower, upper;
+  bool nz;
+};
+DCDF_DEVINL FixedBand value_band(double lo, double hi, int bits, int enc) {
+  constexpr u64 SIGN = 1ull << 63;  // code = (i64)(offset ^ SIGN): offsets 0 .. 2^64 - 1 run over the codes in order
+  FixedBand b{1, 0, false};         // empty
+  if (!(code_value(INT64_MAX, bits, enc) >= lo) || !(code_value(INT64_MIN, bits, enc) <= hi)) return b;
+  u64 a = 0, z = ~0ull;  // smallest code with value >= lo
+  while (a < z) {
+    const u64 mid = a + (z - a) / 2;
+    if (code_value((i64)(mid ^ SIGN), bits, enc) >= lo) z = mid; else a = mid + 1;
+  }
+  b.lower = (i64)(a ^ SIGN);
+  a = 0; z = ~0ull;      // largest code with value <= hi
+  while (a < z) {
+    const u64 mid = z - (z - a) / 2;
+    if (code_value((i64)(mid ^ SIGN), bits, enc) <= hi) a = mid; else z = mid - 1;
+  }
+  b.upper = (i64)(a ^ SIGN);
+  b.nz = (enc == 32 || enc == 64) && b.lower <= 0 && b.upper >= 0;
+  return b;
+}
+// Hit tests against a band: one code / every code of [mn, mx] / no code of [mn, mx].  With nz false they are the plain
+// interval tests of the fixed-bound search.
+DCDF_DEVINL bool band_hit(i64 v, i64 lower, i64 upper, bool nz) { return lower <= v && v <= upper && !(nz && v == 0); }
+DCDF_DEVINL bool band_all(i64 mn, i64 mx, i64 lower, i64 upper, bool nz) { return lower <= mn && mx <= upper && !(nz && mn <= 0 && mx >= 0); }
+DCDF_DEVINL bool band_none(i64 mn, i64 mx, i64 lower, i64 upper, bool nz) { return mn > upper || mx < lower || (nz && mn == 0 && mx == 0); }
+
+// slot_has_cells_part for value bounds [lo, hi].  A level's tables hold codes at that node's fractional bits nb
+// (App. B #11), while a stored subchunk below encodes at its own bits: rounded (round = true) there, a value can lie
+// outside the table's decoded bracket [from_fixed(min), from_fixed(max)] by less than one unit 2^-nb of the node's
+// bits, and the decoded value carries one more rounding to the output type (at most one ulp, < 2^-22 |x| for f32).  So
+// the bracket is widened by 2^-nb + 2^-22 |x| on each side before the test, and a table code 0 bounds nothing on its
+// side (min_max_float stores a min of code 0 for an instant with NaN cells, App. B #10).  Integer tables are exact.
+// Elided slots need no margin: their values are the table values, tested exactly by the caller.
+DCDF_DEVINL bool slot_may_hold_part(const QuerySet& Q, const SlotDesc& d, i64 t_lo, i64 t_hi, double lo, double hi, int first, int step,
+                                    int level) {
+  const u64 tbl0 = level < d.n_up ? d.up_tbl0[level] : d.tbl0;
+  const u64 stride = level < d.n_up ? d.up_stride[level] : d.stride;
+  const int nb = level < d.n_up ? d.up_bits[level] : d.bits;
+  const bool flt = Q.encoding == 32 || Q.encoding == 64;
+  const double unit = flt ? ldexp(1.0, -nb) : 0.0, rel = flt ? 0x1p-22 : 0.0;
+  bool any = false;
+  for (i64 t = t_lo + first; t < t_hi && !any; t += step) {
+    const u64 idx = tbl0 + (u64)t * stride;
+    const i64 cmin = Q.tbl_min[idx], cmax = Q.tbl_max[idx];
+    double vmin = -INFINITY, vmax = INFINITY;
+    if (!flt || cmin != 0) { vmin = code_value(cmin, nb, Q.encoding); vmin -= unit + rel * fabs(vmin); }
+    if (!flt || cmax != 0) { vmax = code_value(cmax, nb, Q.encoding); vmax += unit + rel * fabs(vmax); }
+    any = hi >= vmin && lo <= vmax;
+  }
+  return any;
+}
+
 template <typename OutT>
 DCDF_DEVINL void store_value(void* out, u64 i, i64 fixed, int bits, int out_enc) {
   if (out_enc == 8) static_cast<i64*>(out)[i] = fixed;
@@ -646,13 +717,14 @@ struct Sink {
 
 constexpr int SEARCH_DEPTH = 14;
 
+// nz: code 0 is no hit (the value bounds of a float encoding, see value_band); the tests are exact either way
 DCDF_DEVINL void snapshot_search(const ChunkView& cv, const InstDir& s, u32 top, u32 bottom, u32 left, u32 right, i64 lower,
-                                 i64 upper, Sink& sink) {  // snapshot.rs:310-421; bounds inclusive here
+                                 i64 upper, Sink& sink, bool nz = false) {  // snapshot.rs:310-421; bounds inclusive here
   BitMapRef nm{cv.chunk, s.nm_len, s.nm_base};
   DacRef mx{cv.chunk, &s.max}, mn{cv.chunk, &s.min};
   if (!nm.get(0)) {
     const i64 v = mx.get(0);
-    if (lower <= v && v <= upper) sink.push_rect(top, bottom, left, right, 0, 0);
+    if (band_hit(v, lower, upper, nz)) sink.push_rect(top, bottom, left, right, 0, 0);
     return;
   }
   struct Frame {
@@ -684,11 +756,11 @@ DCDF_DEVINL void snapshot_search(const ChunkView& cv, const InstDir& s, u32 top,
     const u32 index_ = f.index + i * 2u + j;
     const i64 maxv_ = f.maxv - mx.get(index_);
     if (index_ >= s.nm_len || !nm.get(index_)) {
-      if (lower <= maxv_ && maxv_ <= upper) sink.push_rect(top_, bottom_, left_, right_, top_off_, left_off_);
+      if (band_hit(maxv_, lower, upper, nz)) sink.push_rect(top_, bottom_, left_, right_, top_off_, left_off_);
     } else {
       const u32 rk = nm.rank(index_);
       const i64 minv_ = f.minv + mn.get(rk);
-      if (lower <= f.minv && maxv_ <= upper) {  // snapshot.rs:392 uses the parent's min (sic)
+      if (band_all(f.minv, maxv_, lower, upper, nz)) {  // snapshot.rs:392 uses the parent's min (sic)
         sink.push_rect(top_, bottom_, left_, right_, top_off_, left_off_);
       } else if (upper >= minv_ && lower <= maxv_) {
         if (sp + 1 >= SEARCH_DEPTH || sl < 2u) continue;  // malformed input guard
@@ -704,8 +776,10 @@ DCDF_DEVINL void snapshot_search(const ChunkView& cv, const InstDir& s, u32 top,
   }
 }
 
+// strict: the root is read as Log::get reads it (log.rs:180-186) instead of the reference's root test (SURVEY App. B #15),
+// so that the hit set is exact; nz as snapshot_search
 DCDF_DEVINL void log_search(const ChunkView& cv, const InstDir& l, const InstDir& s, u32 top, u32 bottom, u32 left, u32 right,
-                            i64 lower, i64 upper, Sink& sink) {  // log.rs:519-702 (reference behaviour incl. SURVEY B#15)
+                            i64 lower, i64 upper, Sink& sink, bool strict = false, bool nz = false) {  // log.rs:519-702 (reference behaviour incl. SURVEY B#15)
   BitMapRef nm_t{cv.chunk, l.nm_len, l.nm_base}, nm_s{cv.chunk, s.nm_len, s.nm_base};
   BitMapRef eq{cv.chunk, l.eq_len, l.eq_base};
   DacRef mx_t{cv.chunk, &l.max}, mx_s{cv.chunk, &s.max}, mn_t{cv.chunk, &l.min}, mn_s{cv.chunk, &s.min};
@@ -724,17 +798,27 @@ DCDF_DEVINL void log_search(const ChunkView& cv, const InstDir& l, const InstDir
     f.top_off = 0; f.left_off = 0;
     f.min_t = mn_t.get(0); f.min_s = mn_s.get(0); f.max_t = mx_t.get(0); f.max_s = mx_s.get(0);
     f.i = 0; f.j = 0;
+    if (strict) {
+      if (!(f.flags & 2u)) f.min_s = f.max_s;  // a single-node Snapshot has no min Dac: its one value is the max entry
+      if (!(f.flags & 1u)) {
+        if (!(f.flags & 2u) || !eq.get(0)) {  // a uniform single-node Log: every cell is max_s + max_t
+          if (band_hit(f.max_s + f.max_t, lower, upper, nz)) sink.push_rect(top, bottom, left, right, 0, 0);
+          return;
+        }
+        f.min_t = f.max_t;  // the snapshot plus a constant
+      }
+    }
   }
   while (sp >= 0) {
     Frame& f = st[sp];
     if (!(f.flags & 4u)) {
       // entry of _search_window (log.rs:576-591)
       const i64 maxv = f.max_s + f.max_t, minv = f.min_s + f.min_t;
-      if (minv >= lower && maxv <= upper) {
+      if (band_all(minv, maxv, lower, upper, nz)) {
         sink.push_rect(f.top, f.bottom, f.left, f.right, f.top_off, f.left_off);
         sp--;
         continue;
-      } else if (minv > upper || maxv < lower) {
+      } else if (band_none(minv, maxv, lower, upper, nz)) {
         sp--;
         continue;
       }
@@ -789,6 +873,8 @@ struct SearchParams {
   u64 n_queries, n_jobs;
   const i64* lower;       // per query
   const i64* upper;
+  const double* vlower;   // per query, value bounds of the strict search (dcdf_superchunk_search_values)
+  const double* vupper;
   u64* counts;            // [n_jobs]  pass 1 out
   const u64* offsets;     // [n_jobs]  pass 2 in
   i64* out;               // triplets
@@ -796,7 +882,9 @@ struct SearchParams {
 };
 
 // Job order inside a query: overlapped subchunks row-major (superchunk.rs:589-633), then instants ascending,
-// then the Snapshot / Log traversal order (chunk.rs:336-383).
+// then the Snapshot / Log traversal order (chunk.rs:336-383).  STRICT: value bounds, converted per job with the
+// subchunk's own fractional bits (value_band), and the exact hit set (log_search's strict root, code 0 never a hit).
+template <bool STRICT>
 __global__ void k_search(const SearchParams P, int write) {
   const u64 ji = (u64)blockIdx.x * blockDim.x + threadIdx.x;
   if (ji >= P.n_jobs) return;
@@ -822,8 +910,12 @@ __global__ void k_search(const SearchParams P, int write) {
   const i64 wl = max(chunk_left, c.left), wr = min(chunk_left + cs, c.right);
   const u32 top = (u32)(wt - chunk_top), bottom = (u32)(wb - chunk_top - 1);
   const u32 left = (u32)(wl - chunk_left), right = (u32)(wr - chunk_left - 1);
-  i64 lower = P.lower[q], upper = P.upper[q];
-  if (lower > upper) { const i64 t = lower; lower = upper; upper = t; }  // helpers.rs:7-16 via chunk.rs:214
+  i64 lower = 0, upper = 0;
+  if (!STRICT) {
+    lower = P.lower[q]; upper = P.upper[q];
+    if (lower > upper) { const i64 t = lower; lower = upper; upper = t; }  // helpers.rs:7-16 via chunk.rs:214
+  }
+  bool nz = false;
   Sink sink;
   sink.n = 0;
   sink.instant = instant;
@@ -840,11 +932,17 @@ __global__ void k_search(const SearchParams P, int write) {
   const u32 ti = (u32)(instant - sm.t0);
   const u32 slot = (u32)(cr * Q.subsidelen + cc);
   const int32_t u = Q.slot_unit[sm.slot_base + slot];
+  if (STRICT) {
+    const bool stored = u >= 0 && Q.units[u].stored;
+    const FixedBand b = value_band(P.vlower[q], P.vupper[q], stored ? Q.units[u].bits : Q.slot_desc[sm.slot_base + slot].bits, Q.encoding);
+    lower = b.lower; upper = b.upper; nz = b.nz;
+  }
   if (Q.tbl_min) {  // superchunk.rs:480-493: the subchunk is searched only if some instant of the window can have cells in range
     const SlotDesc sd = Q.slot_desc[sm.slot_base + slot];
     const i64 t_lo = max(c.start, sm.t0) - sm.t0, t_hi = min(c.end, sm.t0 + (i64)sm.instants) - sm.t0;
     for (int lv = 0; lv <= sd.n_up; lv++)
-      if (!slot_has_cells_part(Q, sd, t_lo, t_hi, lower, upper, 0, 1, lv)) {
+      if (STRICT ? !slot_may_hold_part(Q, sd, t_lo, t_hi, P.vlower[q], P.vupper[q], 0, 1, lv)
+                 : !slot_has_cells_part(Q, sd, t_lo, t_hi, lower, upper, 0, 1, lv)) {
         if (!write) P.counts[ji] = 0;
         return;
       }
@@ -855,8 +953,8 @@ __global__ void k_search(const SearchParams P, int write) {
     if (m.stored) {
       ChunkView cv{Q.blob + m.blob_off, Q.dir + m.dir_base, m.sidelen};
       const InstDir& d = cv.dir[ti];
-      if (d.snap == ti) snapshot_search(cv, d, top, bottom, left, right, lower, upper, sink);
-      else log_search(cv, d, cv.dir[d.snap], top, bottom, left, right, lower, upper, sink);
+      if (d.snap == ti) snapshot_search(cv, d, top, bottom, left, right, lower, upper, sink, nz);
+      else log_search(cv, d, cv.dir[d.snap], top, bottom, left, right, lower, upper, sink, STRICT, nz);
       done = true;
     }
   }
@@ -864,7 +962,7 @@ __global__ void k_search(const SearchParams P, int write) {
     // Elided subchunk: one value per instant from the max table (superchunk.rs:541-559)
     const SlotDesc sdsc = Q.slot_desc[sm.slot_base + slot];
     const i64 v = Q.tbl_max[sdsc.tbl0 + (u64)ti * sdsc.stride];
-    if (lower <= v && v <= upper) sink.push_rect(top, bottom, left, right, 0, 0);
+    if (band_hit(v, lower, upper, nz)) sink.push_rect(top, bottom, left, right, 0, 0);
   }
   if (!write) P.counts[ji] = sink.n;
 }

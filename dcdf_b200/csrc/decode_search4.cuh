@@ -21,6 +21,7 @@ struct SearchJob {
   i64 lower, upper;
   int top, bottom, left, right;  // window clipped to the tile, tile coordinates, exclusive ends
   i64 row0, col0;                // raster coordinates of the tile's origin
+  bool nz;                       // strict search: code 0 (NaN) is no hit although it lies in [lower, upper]
 };
 // per thread: its 4x4 block / some block of its warp touches the window -- the others never need their part of any
 // pyramid (a thread only reads what it wrote itself)
@@ -42,6 +43,7 @@ struct Search4Smem {
   u32 base[DT_THREADS];            // exclusive prefix of the per-thread hit counts of the current instant
   u32 wsum[DT_WARPS];
   SearchJob job;                   // the CTA's current job (uniform; kept here instead of in every thread's registers)
+  FixedBand band;                  // strict search: the job's band, converted once by thread 0
   __align__(16) InstDir dir[3];
   __align__(16) u8 stage[2][BUF + 32];
 };
@@ -54,11 +56,13 @@ struct Hit {
   u32 m16;
 };
 
-template <typename V>
-DCDF_DEVINL bool in_band(V v, const SearchJob& J) { return J.lower <= (i64)v && (i64)v <= J.upper; }
+// ST (strict, dcdf_superchunk_search_values): the band is the job's converted value bounds and the hit set is exact.  The
+// fixed-bound search compiles without the code-0 tests.
+template <bool ST, typename V>
+DCDF_DEVINL bool in_band(V v, const SearchJob& J) { return band_hit((i64)v, J.lower, J.upper, ST && J.nz); }
 
 // Snapshot: expansion of the pyramid (max, min, cells) and, with `search`, the tests of snapshot.rs:371-413 on the way.
-template <typename V, typename S_>
+template <typename V, typename S_, bool ST>
 DCDF_DEVINL Hit snapshot4s(const u8* chunk, const InstDir& d, int L, S_& S, bool search, const SearchJob& J, const SearchAct A) {
   const u32 p = threadIdx.x;
   RankTab& T = S.tab[threadIdx.x >> 5];
@@ -75,7 +79,7 @@ DCDF_DEVINL Hit snapshot4s(const u8* chunk, const InstDir& d, int L, S_& S, bool
   bool live = search;  // still descending
   if (search && !has) {  // single node (snapshot.rs:318-326)
     live = false;
-    h.e_lvl = in_band(val, J) ? 0 : -1;
+    h.e_lvl = in_band<ST>(val, J) ? 0 : -1;
   }
   const int lvp = L - 2;
   if (p >= (1u << (2 * lvp)) || !A.act) return Hit{-1, 0u};
@@ -88,8 +92,8 @@ DCDF_DEVINL Hit snapshot4s(const u8* chunk, const InstDir& d, int L, S_& S, bool
       has = cidx < nm_len && tab_bit(T, cidx);
       if (has) { r = tab_rank(T, cidx); mnv = pmin + dac_get1<V>(mn, r); } else mnv = val;
       if (live) {
-        if (!has) { live = false; if (in_band(val, J)) h.e_lvl = k; }                                  // leaf node
-        else if (J.lower <= (i64)pmin && (i64)val <= J.upper) { live = false; h.e_lvl = k; }             // parent's min (sic, :392)
+        if (!has) { live = false; if (in_band<ST>(val, J)) h.e_lvl = k; }                                  // leaf node
+        else if (band_all((i64)pmin, (i64)val, J.lower, J.upper, ST && J.nz)) { live = false; h.e_lvl = k; }  // parent's min (sic, :392)
         else if (!(J.upper >= (i64)mnv && J.lower <= (i64)val)) live = false;                            // pruned
       }
     } else {
@@ -124,12 +128,12 @@ DCDF_DEVINL Hit snapshot4s(const u8* chunk, const InstDir& d, int L, S_& S, bool
     for (int i = 0; i < 4; i++) q.c[i] = qv.c[c] - dd[i];
     reinterpret_cast<Quad<V>*>(S.cells)[4u * p + (u32)c] = q;
     if (live && has) {  // the block's node is a branch that was entered: its children are the quads
-      if (!qin) { if (in_band(qv.c[c], J)) h.m16 |= 15u << (4 * c); }
-      else if (J.lower <= (i64)mnv && (i64)qv.c[c] <= J.upper) h.m16 |= 15u << (4 * c);
+      if (!qin) { if (in_band<ST>(qv.c[c], J)) h.m16 |= 15u << (4 * c); }
+      else if (band_all((i64)mnv, (i64)qv.c[c], J.lower, J.upper, ST && J.nz)) h.m16 |= 15u << (4 * c);
       else if (J.upper >= (i64)qm.c[c] && J.lower <= (i64)qv.c[c]) {
 #pragma unroll
         for (int i = 0; i < 4; i++)
-          if (in_band(q.c[i], J)) h.m16 |= 1u << (4 * c + i);
+          if (in_band<ST>(q.c[i], J)) h.m16 |= 1u << (4 * c + i);
       }
     }
   }
@@ -137,16 +141,16 @@ DCDF_DEVINL Hit snapshot4s(const u8* chunk, const InstDir& d, int L, S_& S, bool
 }
 
 // One entry test of Log::_search_window (log.rs:576-591): +1 all inside, -1 disjoint, 0 descend
-template <typename V>
+template <bool ST, typename V>
 DCDF_DEVINL int log_test(V min_s, V min_t, V max_s, V max_t, const SearchJob& J) {
   const i64 mn = (i64)min_s + (i64)min_t, mx = (i64)max_s + (i64)max_t;
-  if (mn >= J.lower && mx <= J.upper) return 1;
-  if (mn > J.upper || mx < J.lower) return -1;
+  if (band_all(mn, mx, J.lower, J.upper, ST && J.nz)) return 1;
+  if (band_none(mn, mx, J.lower, J.upper, ST && J.nz)) return -1;
   return 0;
 }
 
 // Log: the recursion's state down the thread's path, against the snapshot pyramid in S (log.rs:593-700).
-template <typename V, typename S_>
+template <typename V, typename S_, bool ST>
 DCDF_DEVINL Hit log4s(const u8* chunk, const InstDir& d, int L, S_& S, const SearchJob& J, const SearchAct A) {
   const u32 p = threadIdx.x;
   RankTab& T = S.tab[threadIdx.x >> 5];
@@ -157,7 +161,16 @@ DCDF_DEVINL Hit log4s(const u8* chunk, const InstDir& d, int L, S_& S, const Sea
   // the root's test is the same for every thread: a disjoint root ends the instant for the whole CTA (e_lvl = -2)
   // before the rank table is built
   V max_t = dac_get1<V>(mx, 0), min_t = dac_get1<V>(mn, 0);
-  int st = log_test<V>(S.smin[0], min_t, S.sup[0], max_t, J);
+  V min_s0 = S.smin[0];
+  if (ST) {
+    // the root as Log::get / the window decoder read it (log4), not the reference's root test (SURVEY App. B #15)
+    if (S.single[0]) min_s0 = S.sup[0];  // a single-node Snapshot has no min Dac: its one value is the max entry
+    if (!bit_at(nmb, 0)) {
+      if (S.single[0] || !bit_at(eq, 0)) return in_band<ST>((V)(S.sup[0] + max_t), J) ? Hit{0, 0u} : Hit{-2, 0u};  // uniform
+      min_t = max_t;  // the snapshot plus a constant
+    }
+  }
+  int st = log_test<ST, V>(min_s0, min_t, S.sup[0], max_t, J);
   if (st < 0) return Hit{-2, 0u};
   if (!A.warp_act) return Hit{-1, 0u};
   build_rank(nmb, nm_len, T);
@@ -190,7 +203,7 @@ DCDF_DEVINL Hit log4s(const u8* chunk, const InstDir& d, int L, S_& S, const Sea
     const u32 pk = p >> (2 * (lvp - k));
     const V max_s = sup_at(S, k, pk), min_s = S.smin[off3(k) + pk];
     step(pk & 3u, min_s, max_s);
-    st = log_test<V>(min_s, min_t, max_s, max_t, J);
+    st = log_test<ST, V>(min_s, min_t, max_s, max_t, J);
     if (st > 0) h.e_lvl = k;
   }
   if (st != 0) return h;
@@ -204,7 +217,7 @@ DCDF_DEVINL Hit log4s(const u8* chunk, const InstDir& d, int L, S_& S, const Sea
   for (int c = 0; c < 4; c++) {
     has_t = b_has; r = b_r; max_t = b_max;
     step((u32)c, qn.c[c], qs.c[c]);
-    const int sq = log_test<V>(qn.c[c], min_t, qs.c[c], max_t, J);
+    const int sq = log_test<ST, V>(qn.c[c], min_t, qs.c[c], max_t, J);
     if (sq > 0) h.m16 |= 15u << (4 * c);
     if (sq != 0) continue;
     const Quad<V> q = reinterpret_cast<const Quad<V>*>(S.cells)[4u * p + (u32)c];
@@ -213,7 +226,7 @@ DCDF_DEVINL Hit log4s(const u8* chunk, const InstDir& d, int L, S_& S, const Sea
 #pragma unroll
     for (int i = 0; i < 4; i++) {
       const V mt = has_t ? dd[i] : max_t;
-      if (in_band((V)(q.c[i] + mt), J)) h.m16 |= 1u << (4 * c + i);
+      if (in_band<ST>((V)(q.c[i] + mt), J)) h.m16 |= 1u << (4 * c + i);
     }
   }
   return h;
@@ -288,14 +301,14 @@ DCDF_DEVINL void emit_hits(const Hit h, int L, S_& S, const SearchJob& J, i64 in
   }
 }
 
-template <typename V, typename S_>
+template <typename V, typename S_, bool ST>
 DCDF_DEVINL Hit instant4s(const u8* base, const InstDir& d, bool is_snap, bool search, int L, S_& S, const SearchJob& J, const SearchAct A) {
-  return is_snap ? snapshot4s<V, S_>(base, d, L, S, search, J, A) : log4s<V, S_>(base, d, L, S, J, A);
+  return is_snap ? snapshot4s<V, S_, ST>(base, d, L, S, search, J, A) : log4s<V, S_, ST>(base, d, L, S, J, A);
 }
 // structures that do not fit the staging buffer are read from global memory by an out-of-line copy of the same code
-template <typename V, typename S_>
+template <typename V, typename S_, bool ST>
 __device__ __noinline__ void instant4s_global(const u8* chunk, const InstDir* d, bool is_snap, bool search, int L, S_* S, int act, Hit* h) {
-  *h = instant4s<V, S_>(chunk, *d, is_snap, search, L, *S, S->job, SearchAct{(act & 1) != 0, (act & 2) != 0});
+  *h = instant4s<V, S_, ST>(chunk, *d, is_snap, search, L, *S, S->job, SearchAct{(act & 1) != 0, (act & 2) != 0});
 }
 
 struct TileSearchParams {
@@ -306,6 +319,8 @@ struct TileSearchParams {
   u64 n_queries, n_tiles;
   const i64* lower;
   const i64* upper;
+  const double* vlower;      // value bounds of the strict search (k_search_tiles4<V, true>)
+  const double* vupper;
   u64* counts;
   const u64* offsets;
   i64* out;                  // null in the counting pass
@@ -314,7 +329,7 @@ struct TileSearchParams {
                              // the writing pass then places the hits without staging or expanding anything again
 };
 
-template <typename V>
+template <typename V, bool ST>
 __global__ void __launch_bounds__(DT_THREADS, sizeof(V) == 4 ? 4 : 2) k_search_tiles4(const TileSearchParams P) {
   extern __shared__ __align__(16) unsigned char ds4_smem_raw[];
   typedef Search4Smem<V> SM;
@@ -341,9 +356,21 @@ __global__ void __launch_bounds__(DT_THREADS, sizeof(V) == 4 ? 4 : 2) k_search_t
     const i64 t_lo = max(c.start, sm.t0), t_hi = min(c.end, sm.t0 + (i64)sm.instants);
     if (t_hi <= t_lo) continue;
     const i64 chunk_top = cr * cs, chunk_left = cc * cs;
+    const u32 slot = (u32)(cr * Q.subsidelen + cc);
+    const int32_t u = Q.slot_unit[sm.slot_base + slot];
+    const UnitMeta m = u >= 0 ? Q.units[u] : UnitMeta{};
+    const bool stored = u >= 0 && m.stored;
     SearchJob J;  // local copy: the elided / tiny-tile paths use it, the walk reads the CTA's copy in shared memory
-    J.lower = P.lower[q]; J.upper = P.upper[q];
-    if (J.lower > J.upper) { const i64 t = J.lower; J.lower = J.upper; J.upper = t; }  // helpers.rs:7-16 via chunk.rs:214
+    if (ST) {
+      // the band of this subchunk's own fractional bits (an Elided slot: its node's); the binary search runs once per job
+      __syncthreads();  // everyone has read the previous job's band
+      if (tid == 0) S.band = value_band(P.vlower[q], P.vupper[q], stored ? m.bits : Q.slot_desc[sm.slot_base + slot].bits, Q.encoding);
+      __syncthreads();
+      J.lower = S.band.lower; J.upper = S.band.upper; J.nz = S.band.nz;
+    } else {
+      J.lower = P.lower[q]; J.upper = P.upper[q]; J.nz = false;
+      if (J.lower > J.upper) { const i64 t = J.lower; J.lower = J.upper; J.upper = t; }  // helpers.rs:7-16 via chunk.rs:214
+    }
     J.top = (int)(max(chunk_top, c.top) - chunk_top); J.bottom = (int)(min(chunk_top + cs, c.bottom) - chunk_top);
     J.left = (int)(max(chunk_left, c.left) - chunk_left); J.right = (int)(min(chunk_left + cs, c.right) - chunk_left);
     J.row0 = chunk_top; J.col0 = chunk_left;
@@ -356,19 +383,17 @@ __global__ void __launch_bounds__(DT_THREADS, sizeof(V) == 4 ? 4 : 2) k_search_t
     const int act_bits = (A.act ? 1 : 0) | (A.warp_act ? 2 : 0);
     const u64 T_all = (u64)(c.end - c.start);
     const u64 job0 = P.job_base[q] + sub * T_all;  // + (t - c.start)
-    const u32 slot = (u32)(cr * Q.subsidelen + cc);
     if (Q.tbl_min) {
       // Superchunk::search only looks into subchunks whose min / max entries say that some instant of the window can have
       // cells in range (superchunk.rs:480-493), at every level of a nested superchunk; the counts of a pruned job stay 0
       const SlotDesc sd = Q.slot_desc[sm.slot_base + slot];
       bool pruned = false;
       for (int lv = 0; lv <= sd.n_up; lv++)
-        if (!__syncthreads_or(slot_has_cells_part(Q, sd, t_lo - sm.t0, t_hi - sm.t0, J.lower, J.upper, tid, DT_THREADS, lv) ? 1 : 0)) pruned = true;
+        if (!__syncthreads_or((ST ? slot_may_hold_part(Q, sd, t_lo - sm.t0, t_hi - sm.t0, P.vlower[q], P.vupper[q], tid, DT_THREADS, lv)
+                                  : slot_has_cells_part(Q, sd, t_lo - sm.t0, t_hi - sm.t0, J.lower, J.upper, tid, DT_THREADS, lv)) ? 1 : 0))
+          pruned = true;
       if (pruned) continue;
     }
-    const int32_t u = Q.slot_unit[sm.slot_base + slot];
-    const UnitMeta m = u >= 0 ? Q.units[u] : UnitMeta{};
-    const bool stored = u >= 0 && m.stored;
     const int L = stored ? 31 - __clz(m.sidelen) : 0;
     if (!stored) {
       // Elided subchunk: one value per instant from the max table (superchunk.rs:541-559); the window's cells row-major
@@ -378,7 +403,7 @@ __global__ void __launch_bounds__(DT_THREADS, sizeof(V) == 4 ? 4 : 2) k_search_t
       for (i64 t = t_lo; t < t_hi; t++) {
         const u64 jb = job0 + (u64)(t - c.start);
         const i64 v = Q.tbl_max[sdsc.tbl0 + (u64)(t - sm.t0) * sdsc.stride];
-        const bool hit = J.lower <= v && v <= J.upper;
+        const bool hit = band_hit(v, J.lower, J.upper, ST && J.nz);
         if (!P.out) {
           if (tid == 0) P.counts[jb] = hit ? area : 0ull;
         } else if (hit) {
@@ -407,8 +432,8 @@ __global__ void __launch_bounds__(DT_THREADS, sizeof(V) == 4 ? 4 : 2) k_search_t
           const u32 ti = (u32)(t - sm.t0);
           ChunkView cv{Q.blob + m.blob_off, Q.dir + m.dir_base, m.sidelen};
           const InstDir& dd = cv.dir[ti];
-          if (dd.snap == ti) snapshot_search(cv, dd, (u32)J.top, (u32)(J.bottom - 1), (u32)J.left, (u32)(J.right - 1), J.lower, J.upper, sink);
-          else log_search(cv, dd, cv.dir[dd.snap], (u32)J.top, (u32)(J.bottom - 1), (u32)J.left, (u32)(J.right - 1), J.lower, J.upper, sink);
+          if (dd.snap == ti) snapshot_search(cv, dd, (u32)J.top, (u32)(J.bottom - 1), (u32)J.left, (u32)(J.right - 1), J.lower, J.upper, sink, ST && J.nz);
+          else log_search(cv, dd, cv.dir[dd.snap], (u32)J.top, (u32)(J.bottom - 1), (u32)J.left, (u32)(J.right - 1), J.lower, J.upper, sink, ST, ST && J.nz);
           if (!P.out) P.counts[jb] = sink.n;
         }
       }
@@ -441,8 +466,8 @@ __global__ void __launch_bounds__(DT_THREADS, sizeof(V) == 4 ? 4 : 2) k_search_t
       __syncthreads();
       u32 delta;
       Hit hg;
-      if (staged4<V>(chunk, S.dir[2], delta)) instant4s<V, SM>(S.stage[1] + (int32_t)delta, S.dir[2], true, false, L, S, JS, A);
-      else instant4s_global<V, SM>(chunk, &S.dir[2], true, false, L, &S, act_bits, &hg);
+      if (staged4<V>(chunk, S.dir[2], delta)) instant4s<V, SM, ST>(S.stage[1] + (int32_t)delta, S.dir[2], true, false, L, S, JS, A);
+      else instant4s_global<V, SM, ST>(chunk, &S.dir[2], true, false, L, &S, act_bits, &hg);
       __syncthreads();
     }
     prefetch_dir4<V, SM>(dir + ti0, S, 0);
@@ -468,8 +493,8 @@ __global__ void __launch_bounds__(DT_THREADS, sizeof(V) == 4 ? 4 : 2) k_search_t
       if (!want && !is_snap) continue;
       u32 delta;
       Hit h;
-      if (staged4<V>(chunk, D, delta)) h = instant4s<V, SM>(S.stage[b] + (int32_t)delta, D, is_snap, want, L, S, JS, A);
-      else instant4s_global<V, SM>(chunk, &D, is_snap, want, L, &S, act_bits, &h);
+      if (staged4<V>(chunk, D, delta)) h = instant4s<V, SM, ST>(S.stage[b] + (int32_t)delta, D, is_snap, want, L, S, JS, A);
+      else instant4s_global<V, SM, ST>(chunk, &D, is_snap, want, L, &S, act_bits, &h);
       if (!want) continue;
       if (h.e_lvl == -2) continue;  // CTA-uniform: nothing of this instant is inside the band (its count stays 0)
       if (!P.out && P.hit_cache) P.hit_cache[jb * DT_THREADS + (u64)tid] = ((u32)(h.e_lvl + 1) << 16) | (h.m16 & 0xffffu);

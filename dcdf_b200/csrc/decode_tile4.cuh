@@ -533,7 +533,7 @@ struct Count4Smem {
   CountShared<V> C;
 };
 
-template <typename V>
+template <typename V, bool ST>
 __global__ void __launch_bounds__(DT_THREADS, sizeof(V) == 4 ? 4 : 2) k_count_tiles4(const TileCountParams P) {
   extern __shared__ __align__(16) unsigned char dt4_smem_raw[];
   Count4Smem<V>& SS = *reinterpret_cast<Count4Smem<V>*>(dt4_smem_raw);
@@ -549,10 +549,15 @@ __global__ void __launch_bounds__(DT_THREADS, sizeof(V) == 4 ? 4 : 2) k_count_ti
     const bool stored = u >= 0 && m.stored;
     __syncthreads();  // the previous job is done with the entries, the counters and the staging buffers
     if (tid < (int)J.ent_count) {
-      const CountEntry E = P.entries[J.ent_first + (u32)tid];
+      CountEntry E = P.entries[J.ent_first + (u32)tid];
+      bool nz = false;
+      if (ST) {  // the band of this subchunk's own fractional bits (an Elided slot: its node's)
+        const FixedBand fb = value_band(E.vlower, E.vupper, stored ? m.bits : Q.slot_desc[sm.slot_base + J.slot].bits, Q.encoding);
+        E.lower = fb.lower; E.upper = fb.upper; nz = fb.nz;
+      }
       C.ent[tid] = E;
       C.cnt[0][tid] = 0; C.cnt[1][tid] = 0;
-      C.keep[tid] = 1;
+      C.keep[tid] = nz ? 3u : 1u;
       // the band in the expansion's type: values outside V's range cannot occur
       const i64 vlo = sizeof(V) == 4 ? (i64)INT32_MIN : INT64_MIN, vhi = sizeof(V) == 4 ? (i64)INT32_MAX : INT64_MAX;
       const bool empty = E.lower > vhi || E.upper < vlo || E.lower > E.upper;
@@ -569,9 +574,11 @@ __global__ void __launch_bounds__(DT_THREADS, sizeof(V) == 4 ? 4 : 2) k_count_ti
         const CountEntry& E = C.ent[e];
         i64 lo = E.lower, hi = E.upper;
         if (lo > hi) { const i64 x = lo; lo = hi; hi = x; }
+        const CountEntry& G = P.entries[J.ent_first + e];  // the strict search prunes with the value bounds
         bool ok = true;
         for (int lv = 0; lv <= sd.n_up; lv++)
-          ok = ok && __any_sync(0xffffffffu, slot_has_cells_part(Q, sd, (i64)E.t0, (i64)E.t1, lo, hi, lane, 32, lv));
+          ok = ok && __any_sync(0xffffffffu, ST ? slot_may_hold_part(Q, sd, (i64)E.t0, (i64)E.t1, G.vlower, G.vupper, lane, 32, lv)
+                                                : slot_has_cells_part(Q, sd, (i64)E.t0, (i64)E.t1, lo, hi, lane, 32, lv));
         if (lane == 0 && !ok) C.keep[e] = 0;
       }
       __syncthreads();
@@ -596,7 +603,7 @@ __global__ void __launch_bounds__(DT_THREADS, sizeof(V) == 4 ? 4 : 2) k_count_ti
         const u64 area = (u64)(E.bottom - E.top) * (u64)(E.right - E.left);
         for (u32 t = E.t0; t < E.t1; t++) {
           const i64 v = Q.tbl_max[sdsc.tbl0 + (u64)t * sdsc.stride];
-          if (E.lower <= v && v <= E.upper) P.counts[E.cnt_base + (i64)t] = area;
+          if (band_hit(v, E.lower, E.upper, ST && (C.keep[e] & 2u))) P.counts[E.cnt_base + (i64)t] = area;
         }
       }
       continue;
@@ -604,7 +611,7 @@ __global__ void __launch_bounds__(DT_THREADS, sizeof(V) == 4 ? 4 : 2) k_count_ti
     const u8* chunk = Q.blob + m.blob_off;
     const InstDir* dir = Q.dir + m.dir_base;
     const int L = 31 - __clz(m.sidelen);
-    CountOut<V> O;
+    CountOut<V, ST> O;
     O.C = &C; O.mine = mine; O.R0 = R0; O.C0 = C0; O.t = t_lo; O.buf = 0; O.is_log = false; O.min_t = 0; O.e_root = 0;
     const u32 ti0 = t_lo, n_t = t_hi - t_lo;
     const u32 snap0 = dir[ti0].snap;
@@ -629,8 +636,8 @@ __global__ void __launch_bounds__(DT_THREADS, sizeof(V) == 4 ? 4 : 2) k_count_ti
         const bool st = staged4<V>(chunk, S.dir[2], delta);
         const u8* base = st ? S.stage[1] + (int32_t)delta : chunk;
         snapshot_root(base, S.dir[2]);
-        const CountOut<V> O2 = O;
-        instant4_global<V, Tile4Smem<V>, CountOut<V>>(base, &S.dir[2], true, false, L, &S, &O2);
+        const CountOut<V, ST> O2 = O;
+        instant4_global<V, Tile4Smem<V>, CountOut<V, ST>>(base, &S.dir[2], true, false, L, &S, &O2);
       }
       __syncthreads();
     }
@@ -687,10 +694,10 @@ __global__ void __launch_bounds__(DT_THREADS, sizeof(V) == 4 ? 4 : 2) k_count_ti
         O.min_t = dac_get1<V>(dac4_of(base, &D.min), 0);
       }
       if (st) {
-        instant4<V, Tile4Smem<V>, CountOut<V>>(base, D, is_snap, true, L, S, O);
+        instant4<V, Tile4Smem<V>, CountOut<V, ST>>(base, D, is_snap, true, L, S, O);
       } else {
-        const CountOut<V> O2 = O;  // only the copy has its address taken
-        instant4_global<V, Tile4Smem<V>, CountOut<V>>(chunk, &D, is_snap, true, L, &S, &O2);
+        const CountOut<V, ST> O2 = O;  // only the copy has its address taken
+        instant4_global<V, Tile4Smem<V>, CountOut<V, ST>>(chunk, &D, is_snap, true, L, &S, &O2);
       }
     }
     __syncthreads();

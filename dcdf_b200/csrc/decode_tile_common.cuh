@@ -263,7 +263,10 @@ struct SeriesOut {
 // instants of the slice it covers and where its per-instant counts go.
 struct CountEntry {
   i64 cnt_base;          // counts[cnt_base + t] for the slice-local instant t
-  i64 lower, upper;
+  // the fixed band; for the strict search (k_count_tiles4<V, true>) the value bounds, converted to the tile's band when
+  // the entry is loaded into shared memory
+  union { i64 lower; double vlower; };
+  union { i64 upper; double vupper; };
   uint16_t t0, t1;       // slice-local instants [t0, t1)
   u8 top, bottom, left, right;  // tile coordinates, exclusive ends (<= 64)
 };
@@ -273,7 +276,8 @@ struct CountShared {
   CountEntry ent[CT_MAX];
   V lo[CT_MAX], hi[CT_MAX];  // the entry's band in the expansion's value type (clamped; lo > hi: no value can match)
   u32 cnt[2][CT_MAX];   // hits of the instant being decoded / of the previous one (flushed while the next one is decoded)
-  u32 keep[CT_MAX];     // 0: pruned by the superchunk's min / max tables (superchunk.rs:480-493)
+  u32 keep[CT_MAX];     // 0: pruned by the superchunk's min / max tables (superchunk.rs:480-493); else bit 0 set, and
+                        // bit 1 when code 0 (NaN) is no hit although it lies in the band (strict search)
   unsigned long long act[2];  // entries that cover the instant being decoded (by instant parity)
   V smin0, smax0;       // root of the block's snapshot
   u32 n;
@@ -286,9 +290,11 @@ struct CountShared {
 // a Log that is a single node itself (SURVEY App. B #15), are tested against a wrong lower bound; a single-node Log is
 // moreover read as "snapshot + root entry" whether or not its `equal` bit is set.  log4 builds those values
 // (search_quirk); the root test is applied per entry below, to every Log instant (it changes nothing when it is exact).
-template <typename V>
+// ST (strict, dcdf_superchunk_search_values): none of this -- the values are read as the window decoder reads them and the
+// hit set is exact; code 0 is no hit for the entries whose keep bit 1 is set.
+template <typename V, bool ST>
 struct CountOut {
-  static constexpr bool search_quirk = true;
+  static constexpr bool search_quirk = !ST;
   static constexpr bool vec4 = false;
   CountShared<V>* C;
   unsigned long long mine;  // entries whose rectangle touches the thread's block
@@ -310,7 +316,8 @@ struct CountOut {
       m &= m - 1ull;
       const V lo = C->lo[e], hi = C->hi[e];
       bool all = false, none = false;
-      if (is_log) {  // the traversal's root test (log.rs:527-548)
+      const bool nz = ST && (C->keep[e] & 2u);
+      if (!ST && is_log) {  // the traversal's root test (log.rs:527-548)
         const CountEntry& E = C->ent[e];
         const i64 mn = (i64)C->smin0 + (i64)min_t, mx = (i64)C->smax0 + (i64)e_root;
         all = mn >= E.lower && mx <= E.upper;
@@ -325,12 +332,12 @@ struct CountOut {
       const u32 in = rowm & colm;
       if (!in) continue;
       u32 hit = in;
-      if (!all && !(vmin >= lo && vmax <= hi)) {
+      if (!all && !(vmin >= lo && vmax <= hi && !(nz && vmin <= 0 && vmax >= 0))) {
         hit = 0;
 #pragma unroll
         for (int i = 0; i < 4; i++) {
-          if (a[i] >= lo && a[i] <= hi) hit |= 1u << i;
-          if (b[i] >= lo && b[i] <= hi) hit |= 16u << i;
+          if (a[i] >= lo && a[i] <= hi && !(nz && a[i] == 0)) hit |= 1u << i;
+          if (b[i] >= lo && b[i] <= hi && !(nz && b[i] == 0)) hit |= 16u << i;
         }
         hit &= in;
       }

@@ -8,7 +8,7 @@
                          the CIDs of its superchunk nodes, evicted least-recently-used by encoded bytes
   Variable.__getitem__   py-dcdf/dcdf/__init__.py:281-336 (lazy _Slice, scalar / cell / window dispatch)
   MMArray3.shape/get/cell/window   py-dcdf/src/lib.rs:497-538 (PyMMArray3F32), mmarray.rs:357-400
-  search with float bounds         mmarray.rs:407-417 is todo!() upstream; chunk.rs:213-228 takes fixed-point bounds
+  search with float bounds         mmarray.rs:407-417 is todo!() upstream; dcdf_superchunk_search_values on the device
 
 The store is any mapping CID (bytes) -> stored node bytes.  The slices' superchunk CIDs are kept in the reference's span
 tree (dcdf_b200/span.py: stored Span nodes, `Variable.cid` = the root span, dataset.rs:880-987), so a variable written here
@@ -21,7 +21,6 @@ import threading
 
 import numpy as np
 
-from . import _ffi
 from . import span as _span
 from .api import DcdfError, Superchunk
 
@@ -318,45 +317,17 @@ class Variable(MMArray3):
         return out
 
     def search(self, start, stop, top, bottom, left, right, lower, upper):
-        """Cells (instant, row, col) with lower <= value <= upper, bounds in the variable's own units.  The chunk-level
-        search (chunk.rs:213-228) takes fixed-point bounds; they are derived per slice from its fractional bits:
-        a stored value v is a multiple of 2^-bits, so lower <= v <= upper  <=>  2 ceil(lower 2^bits) + 1 <= fixed(v) <=
-        2 floor(upper 2^bits) + 1.  A subchunk that chose fewer bits than its slice would need its own conversion, which
-        the reference leaves as todo!() (mmarray.rs:407-417): such slices are answered from the decoded window."""
+        """Cells (instant, row, col) with lower <= value <= upper, bounds in the variable's own units; NaN cells never
+        match.  One value-range search on the device per span group (Superchunk.search_values_batch), which converts the
+        bounds with every subchunk's own fractional bits (the reference leaves float search as todo!(),
+        mmarray.rs:407-417)."""
         self._check(start, stop, top, bottom, left, right)
-        if lower > upper:
-            lower, upper = upper, lower
-        per = self.chunk_size * self.span_size
         hits = []
-        for sc, t0, a, b in self._groups(start, stop):
-            g = t0 // per
-            for s in range(a // self.chunk_size, (b - 1) // self.chunk_size + 1):
-                sa, sb = max(a, s * self.chunk_size), min(b, (s + 1) * self.chunk_size)
-                bits = self.slice_bits[g * self.span_size + s]
-                if self.dtype.kind == "f":
-                    kinds, _, _, cbits = sc.refs(s)
-                    uniform_bits = all(int(cb) == bits for k, cb in zip(kinds, cbits) if k == _ffi.REF_EXTERNAL) and sc.node_count() == 1
-                    if not uniform_bits:
-                        w = sc.window(sa, sb, top, bottom, left, right)
-                        idx = np.argwhere((w >= lower) & (w <= upper))
-                        idx[:, 0] += t0 + sa
-                        idx[:, 1] += top
-                        idx[:, 2] += left
-                        hits.append(idx.astype(np.int64))
-                        continue
-                    lo_f = 2 * int(np.ceil(np.float64(lower) * 2.0 ** bits)) + 1
-                    hi_f = 2 * int(np.floor(np.float64(upper) * 2.0 ** bits)) + 1
-                else:
-                    lo_f, hi_f = int(np.ceil(lower)), int(np.floor(upper))
-                ranges = [(lo_f, hi_f)]
-                if self.dtype.kind == "f" and lo_f <= 0 <= hi_f:
-                    ranges = [(lo_f, -1), (1, hi_f)]       # fixed 0 is NaN (fixed.rs:35-37), never a match
-                for a_f, b_f in ranges:
-                    if a_f > b_f:
-                        continue
-                    cells = sc.search(sa, sb, top, bottom, left, right, a_f, b_f)
-                    cells[:, 0] += t0
-                    hits.append(cells)
+        if stop > start:
+            for sc, t0, a, b in self._groups(start, stop):
+                cells = sc.search_values(a, b, top, bottom, left, right, lower, upper)
+                cells[:, 0] += t0
+                hits.append(cells)
         return np.concatenate(hits) if hits else np.zeros((0, 3), np.int64)
 
     def close(self):

@@ -232,6 +232,24 @@ int32_t dcdf_superchunk_window_batch(dcdf_ctx* ctx, const dcdf_superchunk* sc, u
 int32_t dcdf_superchunk_search_batch(dcdf_ctx* ctx, const dcdf_superchunk* sc, uint64_t n, const dcdf_cube* bounds,
                                      const int64_t* lower, const int64_t* upper, uint64_t* counts, int64_t* out_irc,
                                      uint64_t cap, uint64_t* n_found, int32_t mem);
+/* Value-range search in the array's own units (the decoded values dcdf_superchunk_window returns with the superchunk's
+ * encoding): a cell matches iff lower <= value <= upper.  NaN cells never match.  Other semantics as
+ * dcdf_superchunk_search_batch.
+ *  - value: exactly what the window decoder writes for the cell -- from_fixed in the encoding's float type with the
+ *    fractional bits of the cell's own subchunk; for an Elided slot, the table value of its node with the node's bits.
+ *    A cell matches iff lower <= (double)value <= upper.  Integer encodings compare the stored integer itself (0 is the
+ *    value 0 there, not NaN).
+ *  - bounds: reversed bounds are swapped (chunk.rs:214); -inf / +inf are allowed; a NaN bound returns DCDF_ERR_BAD_ARG.
+ *  - the hit set is exact, also where dcdf_superchunk_search_batch reproduces the reference's traversal (single-node
+ *    Logs, Logs over a single-node Snapshot, SURVEY App. B #15).  The bounds are converted on the device, per subchunk,
+ *    to the interval of codes whose value lies in [lower, upper] (from_fixed is monotone in the code).
+ *  - order: windows in call order; inside a window subchunks row-major, then instants ascending, as
+ *    dcdf_superchunk_search_batch; inside one (subchunk, instant) an order of the implementation's own, deterministic.
+ *    counts[n] are exact per window.  Two-call protocol as dcdf_superchunk_search_batch (out_irc == NULL: counts and
+ *    *n_found only). */
+int32_t dcdf_superchunk_search_values(dcdf_ctx* ctx, const dcdf_superchunk* sc, uint64_t n, const dcdf_cube* bounds,
+                                      const double* lower, const double* upper, uint64_t* counts, int64_t* out_irc,
+                                      uint64_t cap, uint64_t* n_found, int32_t mem);
 
 /* ------------------------------------------------------------------ storage side (SURVEY 8b / 8f1) */
 /* Content address of a stored node as the reference's in-memory store computes it (testing.rs:172-183):
