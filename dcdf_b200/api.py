@@ -4,6 +4,7 @@ Names and argument meaning follow the reference (paths relative to dcdf/src):
   Chunk.build / get / fill_cell / fill_window / iter_search / write_to / read_from   chunk.rs:42-278
   Superchunk.build / get / fill_cell / fill_window / search                          superchunk.rs:88-585
   Superchunk.search_values (float bounds; mmarray.rs:407-417 is todo!() upstream)
+  Superchunk.window_stats (per-instant count / min / max / sum / sum_sq of windows; no reference counterpart)
   MMArray3.{shape,get,cell,window,search}                                            mmarray.rs:135-536,
                                                                 py-dcdf/src/lib.rs:411-581 (PyMMArray3*)
   to_fixed / from_fixed / suggest_fraction                                           fixed.rs:31-159
@@ -170,6 +171,11 @@ class Context:
         out = np.empty(f.shape, dtype)
         self.check(self._lib.dcdf_from_fixed(self._h, _ptr(f), f.size, fractional_bits, _ptr(out), _ENC_OF_DTYPE[np.dtype(dtype).name], MEM_HOST))
         return out
+
+
+def stats_dtype(dtype):
+    """Record of Superchunk.window_stats_batch / Variable.window_stats for an array of `dtype`."""
+    return np.dtype([("count", np.uint64), ("min", dtype), ("max", dtype), ("sum", np.float64), ("sum_sq", np.float64)])
 
 
 def _out_array(shape, enc, raw):
@@ -458,6 +464,27 @@ class Superchunk(_Queryable):
         self.ctx.check(self.ctx._lib.dcdf_superchunk_window_batch(self.ctx._h, self._h, len(cubes), _ptr(cubes), _ptr(off), ptr,
                                                                   ENC_I64 if raw else self.encoding, mem))
         return out, off
+
+    def window_stats_batch(self, cubes):
+        """Per-instant statistics of n windows reduced on the device (dcdf_superchunk_window_stats) -> (records, off):
+        window i's records are records[off[i]:off[i + 1]], one per instant, ascending.  Fields: count (non-NaN cells),
+        min / max (the superchunk's dtype; NaN / 0 when count is 0), sum and sum_sq (float64) of the values the window
+        decoder writes."""
+        cubes = np.ascontiguousarray(cubes, dtype=np.int64).reshape(-1, 6)
+        off = np.zeros(len(cubes) + 1, np.uint64)
+        np.cumsum(np.abs(cubes[:, 1] - cubes[:, 0]).astype(np.uint64), out=off[1:])
+        dt = _DTYPE_OF_ENC[self.encoding]
+        n = int(off[-1])
+        count, vmin, vmax = np.empty(n, np.uint64), np.empty(n, dt), np.empty(n, dt)
+        total, total_sq = np.empty(n, np.float64), np.empty(n, np.float64)
+        self.ctx.check(self.ctx._lib.dcdf_superchunk_window_stats(self.ctx._h, self._h, len(cubes), _ptr(cubes), _ptr(off), _ptr(count),
+                                                                  _ptr(vmin), _ptr(vmax), _ptr(total), _ptr(total_sq), MEM_HOST))
+        records = np.empty(n, stats_dtype(dt))
+        records["count"], records["min"], records["max"], records["sum"], records["sum_sq"] = count, vmin, vmax, total, total_sq
+        return records, off
+
+    def window_stats(self, start, end, top, bottom, left, right):
+        return self.window_stats_batch([[start, end, top, bottom, left, right]])[0]
 
     def search_batch(self, cubes, lower, upper, want_cells=True):
         return self._search(self.ctx._lib.dcdf_superchunk_search_batch, np.int64, cubes, lower, upper, want_cells)

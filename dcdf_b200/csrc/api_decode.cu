@@ -488,6 +488,26 @@ void do_cell_batch(dcdf_ctx* ctx, MetaBlock* mb, uint64_t n, const int64_t* q, c
   tcollect(ctx, KT_CELL);
 }
 
+// Jobs of the tile window decoder (k_window_tiles4): one per (window, time slice, subchunk the window touches), window after
+// window, slices ascending, subchunks row-major; job_base[i] is window i's first, job_base[n] the count.
+u64 window_jobs(const MetaBlock* mb, const std::vector<CubeDev>& cubes, std::vector<u64>& job_base) {
+  const uint64_t n = cubes.size();
+  job_base.assign(n + 1, 0);
+  u64 n_jobs = 0;
+  const i64 cs = mb->Q.chunks_sidelen;
+  for (uint64_t i = 0; i < n; i++) {
+    const CubeDev& c = cubes[i];
+    job_base[i] = n_jobs;
+    if (c.end > c.start && c.bottom > c.top && c.right > c.left) {
+      const u64 nsub = (u64)((c.bottom - 1) / cs - c.top / cs + 1) * (u64)((c.right - 1) / cs - c.left / cs + 1);
+      const u64 nsl = (u64)((c.end - 1) / mb->Q.chunk_size - c.start / mb->Q.chunk_size + 1);
+      n_jobs += nsub * nsl;
+    }
+  }
+  job_base[n] = n_jobs;
+  return n_jobs;
+}
+
 void do_window_batch(dcdf_ctx* ctx, MetaBlock* mb, uint64_t n, const dcdf_cube* bounds, const uint64_t* out_off, void* out,
                      int32_t out_encoding, int32_t mem) {
   if (n == 0) return;
@@ -513,32 +533,22 @@ void do_window_batch(dcdf_ctx* ctx, MetaBlock* mb, uint64_t n, const dcdf_cube* 
   const bool tiles = mb->max_sidelen <= 64 && !ctx->opt.window_cells;
   if (tiles) {
     // one CTA per (window, slice, subchunk): per-thread walk with one block barrier per instant (decode_tile4.cuh)
-    std::vector<u64> job_base(n + 1);
-    u64 n_jobs = 0;
-    const i64 cs = mb->Q.chunks_sidelen;
-    for (uint64_t i = 0; i < n; i++) {
-      const CubeDev& c = cubes[i];
-      job_base[i] = n_jobs;
-      if (c.end > c.start && c.bottom > c.top && c.right > c.left) {
-        const u64 nsub = (u64)((c.bottom - 1) / cs - c.top / cs + 1) * (u64)((c.right - 1) / cs - c.left / cs + 1);
-        const u64 nsl = (u64)((c.end - 1) / mb->Q.chunk_size - c.start / mb->Q.chunk_size + 1);
-        n_jobs += nsub * nsl;
-      }
-    }
-    job_base[n] = n_jobs;
+    std::vector<u64> job_base;
+    const u64 n_jobs = window_jobs(mb, cubes, job_base);
     ctx->query_aux.reserve(sizeof(u64) * (n + 1));
     CK(cudaMemcpyAsync(ctx->query_aux.p, job_base.data(), sizeof(u64) * (n + 1), cudaMemcpyHostToDevice, ctx->stream));
     TileWindowParams TP;
     TP.Q = mb->Q; TP.cubes = d_c; TP.out_off = d_off; TP.job_base = ctx->query_aux.as<u64>();
     TP.n_queries = n; TP.n_jobs = n_jobs; TP.out = ot.dev; TP.raw = os.raw;
+    TP.part_base = nullptr; TP.part = nullptr;
     const bool narrow = mb->max_dac_levels <= 3 && !ctx->opt.window_wide;  // 32-bit expansion (4 CTAs / SM instead of 2)
-    CK(cudaFuncSetAttribute(k_window_tiles4<i64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Tile4Smem<i64>)));
-    CK(cudaFuncSetAttribute(k_window_tiles4<int32_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Tile4Smem<int32_t>)));
+    CK(cudaFuncSetAttribute(k_window_tiles4<i64, QuadOut>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Tile4Smem<i64>)));
+    CK(cudaFuncSetAttribute(k_window_tiles4<int32_t, QuadOut>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Tile4Smem<int32_t>)));
     tbegin(ctx, KT_WINDOW);
     if (n_jobs) {
       const unsigned grid = (unsigned)std::min<u64>(n_jobs, (u64)ctx->sm_count * 64);
-      if (narrow) k_window_tiles4<int32_t><<<grid, DT_THREADS, sizeof(Tile4Smem<int32_t>), ctx->stream>>>(TP);
-      else k_window_tiles4<i64><<<grid, DT_THREADS, sizeof(Tile4Smem<i64>), ctx->stream>>>(TP);
+      if (narrow) k_window_tiles4<int32_t, QuadOut><<<grid, DT_THREADS, sizeof(Tile4Smem<int32_t>), ctx->stream>>>(TP);
+      else k_window_tiles4<i64, QuadOut><<<grid, DT_THREADS, sizeof(Tile4Smem<i64>), ctx->stream>>>(TP);
       CK(cudaGetLastError());
       ctx->launches++;
     }
@@ -556,6 +566,100 @@ void do_window_batch(dcdf_ctx* ctx, MetaBlock* mb, uint64_t n, const dcdf_cube* 
   tend(ctx, KT_WINDOW);
   out_end(ctx, ot);
   tcollect(ctx, KT_WINDOW);
+}
+
+// Per-instant statistics of n windows (dcdf_superchunk_window_stats): k_window_tiles4<V, StatsOut<V>> writes one partial per
+// (window, subchunk, instant), k_window_stats_combine folds them into the records.  Superchunk subchunks are at most 64x64
+// (dcdf_superchunk_build refuses larger leaves); an opened superchunk with larger ones is refused here, there is no second
+// reduction path.
+void do_window_stats(dcdf_ctx* ctx, MetaBlock* mb, uint64_t n, const dcdf_cube* bounds, const uint64_t* out_off, uint64_t* count,
+                     void* vmin, void* vmax, double* sum, double* sum_sq, int32_t mem) {
+  if (n == 0) return;
+  if (!bounds || !out_off || !count || !vmin || !vmax || !sum || !sum_sq) api_fail(DCDF_ERR_BAD_ARG, "null window statistics argument");
+  if (mem != DCDF_MEM_HOST && mem != DCDF_MEM_DEVICE) api_fail(DCDF_ERR_BAD_ARG, "mem must be DCDF_MEM_HOST or DCDF_MEM_DEVICE");
+  if (mb->max_sidelen > 64) api_fail(DCDF_ERR_BAD_ARG, "window statistics need subchunks of at most 64x64");
+  std::vector<CubeDev> cubes(n);
+  std::vector<u64> part_base(n);
+  u64 n_part = 0;
+  const i64 cs = mb->Q.chunks_sidelen;
+  for (uint64_t i = 0; i < n; i++) {
+    const dcdf_cube c = order_cube(bounds[i]);
+    check_cube(c, mb->Q.shape);
+    cubes[i] = {c.start, c.end, c.top, c.bottom, c.left, c.right};
+    if (out_off[i + 1] < out_off[i] || (uint64_t)(c.end - c.start) != out_off[i + 1] - out_off[i])
+      api_fail(DCDF_ERR_BAD_ARG, "out_off does not match the windows' instants");
+    part_base[i] = n_part;
+    if (c.bottom > c.top && c.right > c.left)
+      n_part += (u64)((c.bottom - 1) / cs - c.top / cs + 1) * (u64)((c.right - 1) / cs - c.left / cs + 1) * (u64)(c.end - c.start);
+  }
+  const u64 rec0 = out_off[0], rec1 = out_off[n], n_rec = rec1 - rec0;
+  std::vector<u64> job_base;
+  const u64 n_jobs = window_jobs(mb, cubes, job_base);
+  cudaStream_t st = ctx->stream;
+  ctx->query_in.reserve(sizeof(CubeDev) * n + sizeof(u64) * (n + 1));
+  CubeDev* d_c = ctx->query_in.as<CubeDev>();
+  u64* d_off = reinterpret_cast<u64*>(d_c + n);
+  CK(cudaMemcpyAsync(d_c, cubes.data(), sizeof(CubeDev) * n, cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(d_off, out_off, sizeof(u64) * (n + 1), cudaMemcpyHostToDevice, st));
+  ctx->query_aux.reserve(sizeof(u64) * (2 * n + 1));
+  u64* d_jb = ctx->query_aux.as<u64>();
+  u64* d_pb = d_jb + n + 1;
+  CK(cudaMemcpyAsync(d_jb, job_base.data(), sizeof(u64) * (n + 1), cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(d_pb, part_base.data(), sizeof(u64) * n, cudaMemcpyHostToDevice, st));
+  ctx->query_aux2.reserve(sizeof(StatsPartial) * std::max<u64>(n_part, 1));
+  // outputs from record rec0 on: the caller's device arrays, or one staging block for the five host arrays
+  const size_t es = enc_size(mb->Q.encoding);
+  u64* o_count = count + rec0;
+  void* o_min = static_cast<u8*>(vmin) + es * rec0;
+  void* o_max = static_cast<u8*>(vmax) + es * rec0;
+  double* o_sum = sum + rec0;
+  double* o_sq = sum_sq + rec0;
+  if (mem == DCDF_MEM_HOST) {
+    const size_t a8 = (sizeof(u64) * n_rec + 15) & ~size_t(15), ae = (es * n_rec + 15) & ~size_t(15);
+    ctx->query_out.reserve(3 * a8 + 2 * ae);
+    u8* b = ctx->query_out.as<u8>();
+    o_count = reinterpret_cast<u64*>(b);
+    o_min = b + a8;
+    o_max = b + a8 + ae;
+    o_sum = reinterpret_cast<double*>(b + a8 + 2 * ae);
+    o_sq = reinterpret_cast<double*>(b + 2 * a8 + 2 * ae);
+  }
+  TileWindowParams TP;
+  TP.Q = mb->Q; TP.cubes = d_c; TP.out_off = d_off; TP.job_base = d_jb;
+  TP.n_queries = n; TP.n_jobs = n_jobs; TP.out = nullptr; TP.raw = 0;
+  TP.part_base = d_pb; TP.part = ctx->query_aux2.as<StatsPartial>();
+  StatsCombineParams CP;
+  CP.cubes = d_c; CP.out_off = d_off; CP.part_base = d_pb; CP.part = TP.part;
+  CP.n_queries = n; CP.rec0 = rec0; CP.rec1 = rec1; CP.cs = cs; CP.encoding = mb->Q.encoding;
+  CP.count = o_count; CP.vmin = o_min; CP.vmax = o_max; CP.sum = o_sum; CP.sum_sq = o_sq;
+  const bool narrow = mb->max_dac_levels <= 3 && !ctx->opt.window_wide;
+  const int smem32 = (int)(sizeof(Tile4Smem<int32_t>) + sizeof(StatsShared<int32_t>));
+  const int smem64 = (int)(sizeof(Tile4Smem<i64>) + sizeof(StatsShared<i64>));
+  if (narrow) CK(cudaFuncSetAttribute(k_window_tiles4<int32_t, StatsOut<int32_t>>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem32));
+  else CK(cudaFuncSetAttribute(k_window_tiles4<i64, StatsOut<i64>>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem64));
+  tbegin(ctx, KT_REDUCE);
+  if (n_jobs) {
+    const unsigned grid = (unsigned)std::min<u64>(n_jobs, (u64)ctx->sm_count * 64);
+    if (narrow) k_window_tiles4<int32_t, StatsOut<int32_t>><<<grid, DT_THREADS, smem32, st>>>(TP);
+    else k_window_tiles4<i64, StatsOut<i64>><<<grid, DT_THREADS, smem64, st>>>(TP);
+    CK(cudaGetLastError());
+    ctx->launches++;
+  }
+  if (n_rec) {
+    k_window_stats_combine<<<(unsigned)((n_rec + 255) / 256), 256, 0, st>>>(CP);
+    CK(cudaGetLastError());
+    ctx->launches++;
+  }
+  tend(ctx, KT_REDUCE);
+  if (mem == DCDF_MEM_HOST && n_rec) {
+    CK(cudaMemcpyAsync(count + rec0, o_count, sizeof(u64) * n_rec, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(static_cast<u8*>(vmin) + es * rec0, o_min, es * n_rec, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(static_cast<u8*>(vmax) + es * rec0, o_max, es * n_rec, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(sum + rec0, o_sum, sizeof(double) * n_rec, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(sum_sq + rec0, o_sq, sizeof(double) * n_rec, cudaMemcpyDeviceToHost, st));
+  }
+  CK(cudaStreamSynchronize(st));  // job_base / part_base stay alive until here
+  tcollect(ctx, KT_REDUCE);
 }
 
 // Fixed-point bounds (lower / upper), or, with strict, value bounds (vlower / vupper) that the kernels convert per subchunk
@@ -911,6 +1015,15 @@ int32_t dcdf_superchunk_window_batch(dcdf_ctx* ctx, const dcdf_superchunk* sc, u
   return guarded(ctx, [&] {
     if (!sc) api_fail(DCDF_ERR_BAD_ARG, "null superchunk");
     do_window_batch(ctx, super_meta(ctx, sc), n, bounds, out_off, out, out_encoding, mem);
+  });
+}
+
+int32_t dcdf_superchunk_window_stats(dcdf_ctx* ctx, const dcdf_superchunk* sc, uint64_t n, const dcdf_cube* bounds,
+                                     const uint64_t* out_off, uint64_t* count, void* vmin, void* vmax, double* sum, double* sum_sq,
+                                     int32_t mem) {
+  return guarded(ctx, [&] {
+    if (!sc) api_fail(DCDF_ERR_BAD_ARG, "null superchunk");
+    do_window_stats(ctx, super_meta(ctx, sc), n, bounds, out_off, count, vmin, vmax, sum, sum_sq, mem);
   });
 }
 

@@ -289,56 +289,51 @@ DCDF_DEVINL bool staged4(const u8* chunk, const InstDir& d, u32& delta) {
   return d.size + mis + 4u <= (u32)Tile4Smem<V>::BUF + 32u;
 }
 
-template <typename V>
+// One CTA per (window, time slice, subchunk) job.  OUT receives the cells: QuadOut writes the window, StatsOut<V> reduces
+// it per instant (dcdf_superchunk_window_stats); its hooks (begin / elided / instant_begin / instant_end / end) are all
+// that differs between the two.
+template <typename V, typename OUT>
 __global__ void __launch_bounds__(DT_THREADS, sizeof(V) == 4 ? 4 : 2) k_window_tiles4(const TileWindowParams P) {
   extern __shared__ __align__(16) unsigned char dt4_smem_raw[];
   Tile4Smem<V>& S = *reinterpret_cast<Tile4Smem<V>*>(dt4_smem_raw);
   const QuerySet& Q = P.Q;
-  const int tid = threadIdx.x;
   for (u64 ji = blockIdx.x; ji < P.n_jobs; ji += gridDim.x) {
     u64 lo_q = 0, hi_q = P.n_queries;
     while (hi_q - lo_q > 1) {
       const u64 mid = (lo_q + hi_q) >> 1;
       if (P.job_base[mid] <= ji) lo_q = mid; else hi_q = mid;
     }
-    const u64 q = lo_q;
-    const CubeDev c = P.cubes[q];
-    const u64 local = ji - P.job_base[q];
+    TileJob J;
+    J.q = lo_q;
+    J.c = P.cubes[J.q];
+    const CubeDev& c = J.c;
+    const u64 local = ji - P.job_base[J.q];
     const i64 cs = Q.chunks_sidelen;
     const i64 cr0 = c.top / cs, cc0 = c.left / cs;
     const i64 ncr = (c.bottom - 1) / cs - cr0 + 1, ncc = (c.right - 1) / cs - cc0 + 1;
     const u64 nsub = (u64)(ncr * ncc);
     const u32 s = (u32)(c.start / Q.chunk_size) + (u32)(local / nsub);
-    const u64 sub = local % nsub;
-    const i64 cr = cr0 + (i64)(sub / (u64)ncc), cc = cc0 + (i64)(sub % (u64)ncc);
+    J.sub = local % nsub;
+    const i64 cr = cr0 + (i64)(J.sub / (u64)ncc), cc = cc0 + (i64)(J.sub % (u64)ncc);
     const SliceMeta sm = Q.slices[s];
-    const i64 t_lo = max(c.start, sm.t0), t_hi = min(c.end, sm.t0 + (i64)sm.instants);
+    J.t_lo = max(c.start, sm.t0); J.t_hi = min(c.end, sm.t0 + (i64)sm.instants);
+    const i64 t_lo = J.t_lo, t_hi = J.t_hi;
     const i64 chunk_top = cr * cs, chunk_left = cc * cs;
+    J.chunk_top = chunk_top; J.chunk_left = chunk_left;
+    // a dense window output: element offset of the window's first cell and of tile cell (0, 0) inside an instant
     const i64 W_rows = c.bottom - c.top, W_cols = c.right - c.left;
-    const u64 obase = P.out_off[q];
+    const u64 obase = P.out_off[J.q];
+    const i64 tile_org = (chunk_top - c.top) * W_cols + (chunk_left - c.left);
+    J.top = (int)(max(chunk_top, c.top) - chunk_top); J.bottom = (int)(min(chunk_top + cs, c.bottom) - chunk_top);
+    J.left = (int)(max(chunk_left, c.left) - chunk_left); J.right = (int)(min(chunk_left + cs, c.right) - chunk_left);
     const u32 slot = (u32)(cr * Q.subsidelen + cc);
     const int32_t u = Q.slot_unit[sm.slot_base + slot];
     const UnitMeta m = u >= 0 ? Q.units[u] : UnitMeta{};
     const bool stored = u >= 0 && m.stored;
-    const i64 tile_org = (chunk_top - c.top) * W_cols + (chunk_left - c.left);  // element offset of tile cell (0, 0)
-    QuadOut O;
-    O.co.init(Q, P.out, P.raw, m.bits);
-    O.pitch = W_cols;
-    O.top = (int)(max(chunk_top, c.top) - chunk_top); O.bottom = (int)(min(chunk_top + cs, c.bottom) - chunk_top);
-    O.left = (int)(max(chunk_left, c.left) - chunk_left); O.right = (int)(min(chunk_left + cs, c.right) - chunk_left);
-    O.vec = O.co.kind == 2 && !(W_cols & 1) && !((obase + (u64)tile_org) & 1ull) && !((uintptr_t)P.out & 7u);
-    O.vec4 = O.co.kind == 2 && !(W_cols & 3) && !((obase + (u64)tile_org) & 3ull) && !((uintptr_t)P.out & 15u);
-    O.base = 0;
+    OUT O;
+    O.begin(P, J, m.bits, dt4_smem_raw + sizeof(Tile4Smem<V>));
     if (!stored) {
-      // Elided: one value per instant from the max table, parent's fractional bits (superchunk.rs:426-433)
-      const SlotDesc sdsc = Q.slot_desc[sm.slot_base + slot];
-      const int wr = O.bottom - O.top, wc = O.right - O.left;
-      for (i64 t = t_lo; t < t_hi; t++) {
-        const i64 v = Q.tbl_max[sdsc.tbl0 + (u64)(t - sm.t0) * sdsc.stride];
-        const u64 tb = obase + (u64)((t - c.start) * W_rows * W_cols + tile_org);
-        for (int i = tid; i < wr * wc; i += DT_THREADS)
-          emit(Q, P.out, tb + (u64)((i64)(O.top + i / wc) * W_cols + (O.left + i % wc)), v, sdsc.bits, P.raw);
-      }
+      O.elided(P, J, sm, Q.slot_desc[sm.slot_base + slot]);
       continue;
     }
     const u8* chunk = Q.blob + m.blob_off;
@@ -358,8 +353,8 @@ __global__ void __launch_bounds__(DT_THREADS, sizeof(V) == 4 ? 4 : 2) k_window_t
          // kernel holds ONE inlined copy of it
         u32 delta;
         const bool st = staged4<V>(chunk, S.dir[2], delta);
-        const QuadOut O2 = O;
-        instant4_global<V, Tile4Smem<V>, QuadOut>(st ? S.stage[1] + (int32_t)delta : chunk, &S.dir[2], true, false, L, &S, &O2);
+        const OUT O2 = O;
+        instant4_global<V, Tile4Smem<V>, OUT>(st ? S.stage[1] + (int32_t)delta : chunk, &S.dir[2], true, false, L, &S, &O2);
       }
       __syncthreads();
     }
@@ -379,19 +374,86 @@ __global__ void __launch_bounds__(DT_THREADS, sizeof(V) == 4 ? 4 : 2) k_window_t
         prefetch4<V, Tile4Smem<V>>(chunk, S.dir[slot1].off, S.dir[slot1].size, S, b ^ 1);
         if (i + 2 < n_t) prefetch_dir4<V, Tile4Smem<V>>(dir + ti + 2, S, slot2);
       }
-      O.base = tbase;
+      O.instant_begin(i, tbase);
       const InstDir& D = S.dir[rs];
       rs = slot1;
       const bool is_snap = D.snap == ti;
       u32 delta;
       if (staged4<V>(chunk, D, delta)) {
-        instant4<V, Tile4Smem<V>, QuadOut>(S.stage[b] + (int32_t)delta, D, is_snap, true, L, S, O);
+        instant4<V, Tile4Smem<V>, OUT>(S.stage[b] + (int32_t)delta, D, is_snap, true, L, S, O);
       } else {
-        const QuadOut O2 = O;  // only the copy has its address taken
-        instant4_global<V, Tile4Smem<V>, QuadOut>(chunk, &D, is_snap, true, L, &S, &O2);
+        const OUT O2 = O;  // only the copy has its address taken
+        instant4_global<V, Tile4Smem<V>, OUT>(chunk, &D, is_snap, true, L, &S, &O2);
       }
+      O.instant_end(i);
     }
+    O.end(n_t);
   }
+}
+
+// Window statistics, second pass: one thread per (window, instant) record folds the window's partials of that instant in
+// subchunk order (row-major) -- a fixed order, so a window's records do not depend on the batch around it.  min / max are
+// compared as values in the encoding's type (subchunks may have different fractional bits).
+struct StatsCombineParams {
+  const CubeDev* cubes;
+  const u64* out_off;    // [n + 1] record offsets
+  const u64* part_base;  // [n]
+  const StatsPartial* part;
+  u64 n_queries, rec0, rec1;  // records [rec0, rec1) = [out_off[0], out_off[n]); record g is written at index g - rec0
+  i64 cs;
+  int encoding;
+  u64* count;
+  void* vmin;
+  void* vmax;
+  double* sum;
+  double* sum_sq;
+};
+template <typename T>
+DCDF_DEVINL T stats_value(i64 code, int bits) {
+  if constexpr (std::is_integral<T>::value) return (T)code;
+  else return from_fixed_dev<T>(code, bits);
+}
+template <typename T>
+DCDF_DEVINL void stats_fold(const StatsCombineParams& P, u64 r, const StatsPartial* p, u64 nsub, u64 T_all) {
+  u64 n = 0;
+  T mn = 0, mx = 0;
+  double sum = 0.0, sq = 0.0;
+  for (u64 k = 0; k < nsub; k++) {
+    const StatsPartial x = p[k * T_all];
+    if (x.count) {
+      const T a = stats_value<T>(x.min, x.bits), b = stats_value<T>(x.max, x.bits);
+      mn = n == 0 || a < mn ? a : mn;
+      mx = n == 0 || b > mx ? b : mx;
+    }
+    n += x.count;
+    sum += x.sum;
+    sq += x.sum_sq;
+  }
+  if (n == 0) mn = mx = stats_value<T>(0, 0);  // NaN for floats (code 0), 0 for integers
+  P.count[r] = n;
+  static_cast<T*>(P.vmin)[r] = mn;
+  static_cast<T*>(P.vmax)[r] = mx;
+  P.sum[r] = sum;
+  P.sum_sq[r] = sq;
+}
+__global__ void k_window_stats_combine(const StatsCombineParams P) {
+  const u64 g = P.rec0 + (u64)blockIdx.x * blockDim.x + threadIdx.x;
+  if (g >= P.rec1) return;
+  u64 lo = 0, hi = P.n_queries;  // the window of record g: the last one whose records start at or before g
+  while (hi - lo > 1) {
+    const u64 mid = (lo + hi) >> 1;
+    if (P.out_off[mid] <= g) lo = mid; else hi = mid;
+  }
+  const CubeDev c = P.cubes[lo];
+  const u64 T_all = (u64)(c.end - c.start), t = g - P.out_off[lo];
+  const u64 nsub = c.bottom > c.top && c.right > c.left
+                       ? (u64)((c.bottom - 1) / P.cs - c.top / P.cs + 1) * (u64)((c.right - 1) / P.cs - c.left / P.cs + 1) : 0u;
+  const StatsPartial* p = P.part + P.part_base[lo] + t;
+  const u64 r = g - P.rec0;
+  if (P.encoding == 32) stats_fold<float>(P, r, p, nsub, T_all);
+  else if (P.encoding == 64) stats_fold<double>(P, r, p, nsub, T_all);
+  else if (P.encoding == 4) stats_fold<int32_t>(P, r, p, nsub, T_all);
+  else stats_fold<i64>(P, r, p, nsub, T_all);
 }
 
 // ---------------------------------------------------------------------------------------------------------------

@@ -3,6 +3,8 @@
 // staging, four-entry DAC / bitmap fetches for the children of one node (their BFS indices are consecutive:
 // 1 + 4 * rank(idx) .. + 3, snapshot.rs:177), the window-clipped quad writer.
 #pragma once
+#include <type_traits>
+
 #include "decode.cuh"
 
 namespace dcdf {
@@ -42,6 +44,17 @@ struct CellOut {
   }
 };
 
+// Window statistics (dcdf_superchunk_window_stats): the reduction of one (window, subchunk, instant).  min / max are codes
+// at `bits` (from_fixed is monotone in the code at fixed bits, so they are compared as codes inside a tile and as values
+// across tiles); sum / sum_sq are in the array's units.  count == 0: min / max are meaningless, the sums 0.
+struct StatsPartial {
+  u32 count;
+  int bits;
+  i64 min, max;
+  double sum, sum_sq;
+};
+static_assert(sizeof(StatsPartial) == 40, "StatsPartial is 40 bytes");
+
 struct TileWindowParams {
   QuerySet Q;
   const CubeDev* cubes;   // validated, ordered
@@ -50,6 +63,18 @@ struct TileWindowParams {
   u64 n_queries, n_jobs;
   void* out;
   int raw;
+  // window statistics: partial of (window q, subchunk sub, instant t) at part[part_base[q] + sub * (end - start) + t - start]
+  const u64* part_base;
+  StatsPartial* part;
+};
+
+// One job of k_window_tiles4: window q, one time slice [t_lo, t_hi), the subchunk `sub` (row-major among those the window
+// touches) whose tile starts at (chunk_top, chunk_left); the window clipped to the tile in tile coordinates.
+struct TileJob {
+  CubeDev c;
+  u64 q, sub;
+  i64 chunk_top, chunk_left, t_lo, t_hi;
+  int top, bottom, left, right;
 };
 
 constexpr u32 W3_NONE = 0xffffffffu;
@@ -188,6 +213,34 @@ struct QuadOut {
   i64 pitch;      // window columns
   int top, bottom, left, right;  // window clipped to the tile, tile coordinates
   bool vec, vec4; // f32 output whose row pairs / row quadruples are 8 / 16-byte aligned
+  // k_window_tiles4's hooks: a job starts (bits: the stored subchunk's), an Elided job, an instant starts (tbase: element
+  // index of tile cell (0, 0) at that instant in a dense window output) / ends, a job ends
+  DCDF_DEVINL void begin(const TileWindowParams& P, const TileJob& J, int bits, unsigned char*) {
+    const i64 W_cols = J.c.right - J.c.left;
+    const u64 obase = P.out_off[J.q];
+    const i64 tile_org = (J.chunk_top - J.c.top) * W_cols + (J.chunk_left - J.c.left);  // element offset of tile cell (0, 0)
+    co.init(P.Q, P.out, P.raw, bits);
+    pitch = W_cols;
+    top = J.top; bottom = J.bottom; left = J.left; right = J.right;
+    vec = co.kind == 2 && !(W_cols & 1) && !((obase + (u64)tile_org) & 1ull) && !((uintptr_t)P.out & 7u);
+    vec4 = co.kind == 2 && !(W_cols & 3) && !((obase + (u64)tile_org) & 3ull) && !((uintptr_t)P.out & 15u);
+    base = 0;  // set per instant
+  }
+  // Elided: one value per instant from the max table, parent's fractional bits (superchunk.rs:426-433)
+  DCDF_DEVINL void elided(const TileWindowParams& P, const TileJob& J, const SliceMeta& sm, const SlotDesc& sdsc) const {
+    const int wr = bottom - top, wc = right - left;
+    const i64 W_rows = J.c.bottom - J.c.top;
+    const u64 org = P.out_off[J.q] + (u64)((J.chunk_top - J.c.top) * pitch + (J.chunk_left - J.c.left));
+    for (i64 t = J.t_lo; t < J.t_hi; t++) {
+      const i64 v = P.Q.tbl_max[sdsc.tbl0 + (u64)(t - sm.t0) * sdsc.stride];
+      const u64 tb = org + (u64)((t - J.c.start) * W_rows * pitch);
+      for (int i = threadIdx.x; i < wr * wc; i += DT_THREADS)
+        emit(P.Q, P.out, tb + (u64)((i64)(top + i / wc) * pitch + (left + i % wc)), v, sdsc.bits, P.raw);
+    }
+  }
+  DCDF_DEVINL void instant_begin(u32, u64 tbase) { base = tbase; }
+  DCDF_DEVINL void instant_end(u32) {}
+  DCDF_DEVINL void end(u32) {}
   template <typename V>
   DCDF_DEVINL float cvt(V v) const {  // from_fixed (fixed.rs:81-86): 0 -> NaN, else (v - 1) * 2^-(bits+1), exact scaling
     const float f = (sizeof(V) == 4 ? __int2float_rn((int)v - 1) : __ll2float_rn((i64)v - 1)) * co.inv32;
@@ -349,6 +402,160 @@ struct CountOut {
     // that the strip's range is the quad's
     CountOut o = *this;
     o.put_pair(false, r0, c0, v, v);
+  }
+};
+
+// Window statistics through the tile decoder (k_window_tiles4<V, StatsOut<V>>): every thread folds the cells of its block
+// that lie inside the window into its own slot in shared memory (no atomics); after each instant the CTA reduces the slots
+// in a fixed order and thread 0 writes the (window, subchunk, instant) partial.  The sum is exact: the decoded value of a
+// code n is x * 2^-(bits+1) with x = float(n - 1) / double(n - 1) an integer (the code itself for integer encodings), and
+// x is summed as an integer (64 bits for the 32-bit expansion, 128 for the 64-bit one), converted to double once and
+// scaled.  sum_sq adds x * x in double and is scaled the same way.
+template <typename V>
+struct StatsSlot {
+  using Sum = typename std::conditional<sizeof(V) == 4, i64, __int128>::type;
+  Sum sum;
+  double sq;
+  V mn, mx;  // codes
+  u32 n;
+  DCDF_DEVINL void clear() {
+    sum = 0; sq = 0.0; n = 0;
+    mn = sizeof(V) == 4 ? (V)INT32_MAX : (V)INT64_MAX;
+    mx = sizeof(V) == 4 ? (V)INT32_MIN : (V)INT64_MIN;
+  }
+  DCDF_DEVINL void fold(const StatsSlot& o) { sum += o.sum; sq += o.sq; n += o.n; mn = min(mn, o.mn); mx = max(mx, o.mx); }
+};
+template <typename V>
+struct StatsShared {
+  StatsSlot<V> slot[DT_THREADS];
+  StatsSlot<V> warp[2][DT_WARPS];  // per-warp results of an instant, by instant parity (folded while the next one is decoded)
+};
+// An integer-valued float / double as the sum's type (exact: |x| <= 2^31 for the 32-bit expansion, <= 2^63 otherwise).
+template <typename S, typename F>
+DCDF_DEVINL S exact_int(F x) {
+  if (sizeof(S) == 8) return (S)(i64)x;
+  return fabs((double)x) < 0x1p62 ? (S)(i64)x : (S)x;
+}
+template <typename V>
+struct StatsOut {
+  using Sum = typename StatsSlot<V>::Sum;
+  static constexpr bool search_quirk = false;
+  static constexpr bool vec4 = false;
+  StatsShared<V>* C;
+  StatsPartial* rec;             // partial of the job's first instant; instant i at rec[i]
+  int top, bottom, left, right;  // window clipped to the tile, tile coordinates
+  int kind;                      // 0: integer encodings (the code is the value), 2: f32, 3: f64
+  int bits;
+  DCDF_DEVINL bool touches(int r0, int c0, int side) const { return r0 + side > top && r0 < bottom && c0 + side > left && c0 < right; }
+  DCDF_DEVINL bool inside(int r0, int c0, int side) const { return r0 >= top && r0 + side <= bottom && c0 >= left && c0 + side <= right; }
+  DCDF_DEVINL void add(StatsSlot<V>& s, V v) const {
+    if (kind != 0 && v == 0) return;  // NaN
+    s.n++;
+    s.mn = min(s.mn, v);
+    s.mx = max(s.mx, v);
+    if (kind == 2) {
+      const float x = sizeof(V) == 4 ? __int2float_rn((int)v - 1) : __ll2float_rn((i64)v - 1);
+      s.sum += exact_int<Sum>(x);
+      s.sq += (double)x * (double)x;
+    } else if (kind == 3) {
+      const double x = sizeof(V) == 4 ? __int2double_rn((int)v - 1) : __ll2double_rn((i64)v - 1);
+      s.sum += exact_int<Sum>(x);
+      s.sq += x * x;
+    } else {
+      s.sum += (Sum)v;
+      s.sq += (double)v * (double)v;
+    }
+  }
+  DCDF_DEVINL void put_pair(bool, int r0, int c0, const V (&a)[4], const V (&b)[4]) const {
+    // cells of this 2x4 strip inside the window: bits 0..3 = a, 4..7 = b (cell = 2 * (row & 1) + (col & 1))
+    const u32 rowm = ((r0 >= top && r0 < bottom) ? 0x33u : 0u) | ((r0 + 1 >= top && r0 + 1 < bottom) ? 0xccu : 0u);
+    const u32 colm = ((c0 >= left && c0 < right) ? 0x05u : 0u) | ((c0 + 1 >= left && c0 + 1 < right) ? 0x0au : 0u) |
+                     ((c0 + 2 >= left && c0 + 2 < right) ? 0x50u : 0u) | ((c0 + 3 >= left && c0 + 3 < right) ? 0xa0u : 0u);
+    const u32 in = rowm & colm;
+    if (!in) return;
+    StatsSlot<V>& slot = C->slot[threadIdx.x];
+    StatsSlot<V> s = slot;
+#pragma unroll
+    for (int i = 0; i < 4; i++) {
+      if ((in >> i) & 1u) add(s, a[i]);
+      if ((in >> (4 + i)) & 1u) add(s, b[i]);
+    }
+    slot = s;
+  }
+  DCDF_DEVINL void put(int r0, int c0, const V (&v)[4]) const {  // trees of side 2: one quad at (0, 0)
+    put_pair(false, r0, c0, v, v);  // the second quad lies outside every rectangle of a 2x2 tile (right <= 2)
+  }
+  // k_window_tiles4's hooks
+  DCDF_DEVINL void begin(const TileWindowParams& P, const TileJob& J, int bits_, unsigned char* smem) {
+    C = reinterpret_cast<StatsShared<V>*>(smem);
+    rec = P.part + P.part_base[J.q] + J.sub * (u64)(J.c.end - J.c.start) + (u64)(J.t_lo - J.c.start);
+    top = J.top; bottom = J.bottom; left = J.left; right = J.right;
+    kind = P.Q.encoding == 32 ? 2 : P.Q.encoding == 64 ? 3 : 0;
+    bits = bits_;
+    C->slot[threadIdx.x].clear();
+  }
+  DCDF_DEVINL double scale() const { return kind ? __longlong_as_double((long long)(1022 - bits) << 52) : 1.0; }  // 2^-(bits+1)
+  // Elided: one value per instant from the max table at its node's bits (superchunk.rs:426-433); nothing to decode
+  DCDF_DEVINL void elided(const TileWindowParams& P, const TileJob& J, const SliceMeta& sm, const SlotDesc& sdsc) {
+    bits = sdsc.bits;
+    const double sc = scale();
+    const i64 area = (i64)(bottom - top) * (i64)(right - left);
+    for (i64 t = J.t_lo + (i64)threadIdx.x; t < J.t_hi; t += DT_THREADS) {
+      const i64 v = P.Q.tbl_max[sdsc.tbl0 + (u64)(t - sm.t0) * sdsc.stride];
+      const bool nan = kind != 0 && v == 0;
+      const double x = kind == 2 ? (double)__ll2float_rn(v - 1) : kind == 3 ? __ll2double_rn(v - 1) : (double)v;
+      StatsPartial p;
+      p.count = nan ? 0u : (u32)area;
+      p.bits = bits;
+      p.min = v; p.max = v;
+      const __int128 xi = kind == 0 ? (__int128)v : exact_int<__int128>(x);
+      p.sum = nan ? 0.0 : (double)(xi * (__int128)area) * sc;
+      p.sum_sq = nan ? 0.0 : (double)area * (x * x) * sc * sc;
+      rec[t - J.t_lo] = p;
+    }
+  }
+  DCDF_DEVINL void instant_begin(u32 i, u64) const {
+    if (i > 0) flush(i - 1u);
+  }
+  // the CTA's reduction of instant i: warp shuffles in a fixed tree, then (flush) the warps in index order
+  DCDF_DEVINL void instant_end(u32 i) const {
+    StatsSlot<V>& slot = C->slot[threadIdx.x];
+    StatsSlot<V> s = slot;
+    slot.clear();
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      StatsSlot<V> x;
+      x.n = __shfl_down_sync(0xffffffffu, s.n, o);
+      x.mn = __shfl_down_sync(0xffffffffu, s.mn, o);
+      x.mx = __shfl_down_sync(0xffffffffu, s.mx, o);
+      x.sq = __shfl_down_sync(0xffffffffu, s.sq, o);
+      if (sizeof(V) == 4) {
+        x.sum = (Sum)__shfl_down_sync(0xffffffffu, (long long)s.sum, o);
+      } else {
+        const unsigned long long lo = __shfl_down_sync(0xffffffffu, (unsigned long long)s.sum, o);
+        const long long hi = __shfl_down_sync(0xffffffffu, (long long)(s.sum >> 64), o);
+        x.sum = (Sum)(((unsigned __int128)(u64)hi << 64) | lo);
+      }
+      s.fold(x);
+    }
+    if ((threadIdx.x & 31u) == 0) C->warp[i & 1u][threadIdx.x >> 5] = s;
+  }
+  DCDF_DEVINL void flush(u32 i) const {  // thread 0, after a barrier that follows instant i's instant_end
+    if (threadIdx.x != 0) return;
+    StatsSlot<V> s = C->warp[i & 1u][0];
+    for (int w = 1; w < DT_WARPS; w++) s.fold(C->warp[i & 1u][w]);
+    const double sc = scale();
+    StatsPartial p;
+    p.count = s.n;
+    p.bits = bits;
+    p.min = (i64)s.mn; p.max = (i64)s.mx;
+    p.sum = (double)s.sum * sc;
+    p.sum_sq = s.sq * sc * sc;
+    rec[i] = p;
+  }
+  DCDF_DEVINL void end(u32 n_t) const {
+    __syncthreads();
+    flush(n_t - 1u);
   }
 };
 

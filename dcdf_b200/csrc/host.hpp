@@ -95,7 +95,7 @@ inline void pool_free(void* p) {
   if (p) cudaFreeAsync(p, 0);  // callers have synchronized every stream that used p
 }
 
-enum { KT_ENCODE = 0, KT_STATS = 1, KT_GATHER = 2, KT_WINDOW = 3, KT_CELL = 4, KT_SEARCH = 5, KT_COUNT = 6 };
+enum { KT_ENCODE = 0, KT_STATS = 1, KT_GATHER = 2, KT_WINDOW = 3, KT_CELL = 4, KT_SEARCH = 5, KT_REDUCE = 6, KT_COUNT = 7 };
 
 }  // namespace dcdf
 
@@ -107,7 +107,7 @@ struct dcdf_ctx {
   cudaEvent_t fork_ev = nullptr, join_ev = nullptr;
   std::string last_error;
   uint64_t launches = 0;
-  float kernel_ms[dcdf::KT_COUNT] = {0, 0, 0, 0, 0, 0};
+  float kernel_ms[dcdf::KT_COUNT] = {0, 0, 0, 0, 0, 0, 0};
   cudaEvent_t ev[2 * dcdf::KT_COUNT] = {};
   int sm_count = 148;
   // dcdf_ctx_set_option (include/dcdf_cuda.h)

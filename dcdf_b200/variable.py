@@ -9,6 +9,7 @@
   Variable.__getitem__   py-dcdf/dcdf/__init__.py:281-336 (lazy _Slice, scalar / cell / window dispatch)
   MMArray3.shape/get/cell/window   py-dcdf/src/lib.rs:497-538 (PyMMArray3F32), mmarray.rs:357-400
   search with float bounds         mmarray.rs:407-417 is todo!() upstream; dcdf_superchunk_search_values on the device
+  window_stats                     per-instant count / min / max / sum / sum_sq of a window, dcdf_superchunk_window_stats
 
 The store is any mapping CID (bytes) -> stored node bytes.  The slices' superchunk CIDs are kept in the reference's span
 tree (dcdf_b200/span.py: stored Span nodes, `Variable.cid` = the root span, dataset.rs:880-987), so a variable written here
@@ -329,6 +330,21 @@ class Variable(MMArray3):
                 cells[:, 0] += t0
                 hits.append(cells)
         return np.concatenate(hits) if hits else np.zeros((0, 3), np.int64)
+
+    def window_stats(self, start, stop, top, bottom, left, right):
+        """Per-instant statistics of a window, reduced on the device from the encoded bytes (one
+        Superchunk.window_stats_batch call per span group): stop - start records in time order with fields count (non-NaN
+        cells), min, max (the variable's dtype; NaN for floats / 0 for integers when count is 0), sum and sum_sq (float64).
+        For example
+
+            r = v.window_stats(0, 365, 100, 200, 300, 400)
+            mean = r["sum"] / r["count"]
+            var = r["sum_sq"] / r["count"] - mean ** 2     # population variance
+        """
+        from .api import stats_dtype
+        self._check(start, stop, top, bottom, left, right)
+        parts = [sc.window_stats(a, b, top, bottom, left, right) for sc, _, a, b in self._groups(start, stop)] if stop > start else []
+        return np.concatenate(parts) if parts else np.empty(0, stats_dtype(self.dtype))
 
     def close(self):
         self.cache.close()

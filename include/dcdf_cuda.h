@@ -111,7 +111,7 @@ const char* dcdf_last_error(const dcdf_ctx* ctx);
 uint64_t dcdf_ctx_launch_count(const dcdf_ctx* ctx);
 /* CUDA-event time (ms) of the dominant kernel(s) of the last build / query call, measured on the
  * context's stream.  which: 0 = encode kernel, 1 = stats kernel, 2 = gather, 3 = window decode,
- * 4 = cell decode, 5 = search. */
+ * 4 = cell decode, 5 = search, 6 = window statistics (both of its kernels). */
 int32_t dcdf_ctx_last_kernel_ms(const dcdf_ctx* ctx, int32_t which, float* ms);
 
 /* ------------------------------------------------------------------ a1 / a2 / a3 / a21 */
@@ -226,6 +226,27 @@ int32_t dcdf_superchunk_window(dcdf_ctx* ctx, const dcdf_superchunk* sc, const d
 /* Batched windows: n cubes, out_off[n+1] element offsets into `out`. */
 int32_t dcdf_superchunk_window_batch(dcdf_ctx* ctx, const dcdf_superchunk* sc, uint64_t n, const dcdf_cube* bounds,
                                      const uint64_t* out_off, void* out, int32_t out_encoding, int32_t mem);
+/* Per-instant statistics of n windows, reduced on the device from the encoded bytes (the reference has no counterpart:
+ * there a window is decoded and reduced by the caller).  One record per (window, instant): window i has end - start
+ * records, instants ascending, from record out_off[i] on (out_off[n+1] host array, the convention of
+ * dcdf_superchunk_window_batch counted in records).  Record r is count[r], vmin / vmax[r], sum[r], sum_sq[r].
+ *  - value of a cell: exactly what dcdf_superchunk_window writes for it in the superchunk's encoding -- from_fixed with
+ *    its subchunk's own fractional bits; for an Elided slot at any nesting level the node's table value at the node's
+ *    bits; the stored integer for i32 / i64.  NaN cells (code 0 of a float encoding) are skipped.
+ *  - count (uint64): the number of non-NaN cells of the window at that instant, exact.
+ *  - vmin / vmax: in the superchunk's encoding (float / double / int32_t / int64_t arrays), compared by value across
+ *    subchunks, exact for i64.  count == 0: NaN for float encodings, 0 for integer ones.
+ *  - sum / sum_sq (double): sum of the values and of their squares; 0 when count == 0.  Per (window, subchunk, instant)
+ *    the values are summed exactly as integers and scaled once; partials are added in subchunk order (row-major), so
+ *    the error is a few 2^-53 * sum|v| per subchunk the window touches.
+ *  - determinism: a window's records are bitwise identical across calls, alone or inside any batch, with or without the
+ *    context option "window_wide", for a built superchunk and the same one reopened with dcdf_superchunk_open.
+ *  - reversed bounds are swapped (Cube::new); a zero-area window gives records with count 0; out-of-range windows
+ *    return DCDF_ERR_OUT_OF_BOUNDS; out_off that does not match end - start, NULL pointers, or subchunks larger than
+ *    64x64 (only possible for an opened superchunk) return DCDF_ERR_BAD_ARG.  `mem` says where all five outputs live. */
+int32_t dcdf_superchunk_window_stats(dcdf_ctx* ctx, const dcdf_superchunk* sc, uint64_t n, const dcdf_cube* bounds,
+                                     const uint64_t* out_off, uint64_t* count, void* vmin, void* vmax,
+                                     double* sum, double* sum_sq, int32_t mem);
 /* Batched value-range search over n windows (same fixed-point [lower, upper] semantics as
  * dcdf_chunk_search).  counts[n] (host) receives matches per window; out_irc (may be NULL) receives the
  * triplets window after window.  Order inside a window: subchunks row-major, then chunk order. */
