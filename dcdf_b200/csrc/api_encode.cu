@@ -177,15 +177,28 @@ void launch_encode_v5(dcdf_ctx* ctx, const EncParams& P, u32 grid) {
   CK(cudaGetLastError());
   ctx->launches++;
 }
+// Clipped fast-path tiles with at most 32 rows or columns in the raster (list 7): one warp per tile, twelve tiles per
+// CTA (384 threads, like the six two-warp tiles of k_encode_v5).  ptxas (sm_100a): 168 registers, 352 / 604 bytes of
+// spill stores / loads; E5SmemEdge is 18,720 bytes, so twelve tiles take 224,640 of the 232,448 bytes an SM offers.
+void launch_encode_v5_edge(dcdf_ctx* ctx, const EncParams& P, u32 grid) {
+  constexpr int G = 12;
+  const u32 stage_limit = std::min<u32>(ctx->opt.stage_limit, (u32)E5_POOL_EDGE);
+  const size_t smem = sizeof(E5SmemEdge) * G;
+  CK(cudaFuncSetAttribute(k_encode_v5_edge<G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  k_encode_v5_edge<G><<<(grid + G - 1) / G, 32 * G, smem, ctx->aux_stream>>>(P, stage_limit, ctx->opt.fast_sync_mask);
+  CK(cudaGetLastError());
+  ctx->launches++;
+}
 // list = wide * 2 + clipped  (narrow kernels are compiled for two resident CTAs per SM); 4 = clipped 64-side trees,
-// 5 = fast path
+// 5 = fast path, 6 = clipped fast path, 7 = clipped fast path with half the tree outside the raster
 template <typename InT>
 void launch_encode(dcdf_ctx* ctx, const EncParams& P, u32 grid, int list) {
   if (grid == 0) return;
   if (list >= 5) {
     if (sizeof(InT) == 4) {  // k_finalize_tree only fills these lists for f32 input
       if (list == 5) launch_encode_v5<true>(ctx, P, grid);
-      else launch_encode_v5<false>(ctx, P, grid);
+      else if (list == 6) launch_encode_v5<false>(ctx, P, grid);
+      else launch_encode_v5_edge(ctx, P, grid);
     }
     return;
   }
@@ -260,7 +273,7 @@ void run_encode(dcdf_ctx* ctx, EncodeJob& job, EncodeOut& out, bool want_pieces)
   ctx->istats.reserve(sizeof(InstStats) * (size_t)n_units * job.t_max);
   ctx->slices.reserve(sizeof(SliceDesc) * n_slices + 2 * sizeof(u64) * n_tables);
   ctx->sstate.reserve(sizeof(SliceState) * n_slices);
-  ctx->order.reserve(sizeof(u32) * (7 * (size_t)n_units + 8));
+  ctx->order.reserve(sizeof(u32) * (8 * (size_t)n_units + 8));
   ctx->pieces.reserve(sizeof(Piece) * (n_pieces + 2 * (size_t)n_tables));
   ctx->results.reserve(sizeof(UnitResult) * n_units);
   ctx->stored.reserve(n_units);
@@ -276,7 +289,7 @@ void run_encode(dcdf_ctx* ctx, EncodeJob& job, EncodeOut& out, bool want_pieces)
   out.tbl_min = d_tbl_min;
   out.tbl_total = tbl_total;
 
-  // small: [0] err (u32) | [8] arena_head (u64) | [16] order counts (5 x u32)
+  // small: [0] err (u32) | [8] arena_head (u64) | [16] order counts (8 x u32)
   u32* d_err = ctx->small.as<u32>();
   unsigned long long* d_head = reinterpret_cast<unsigned long long*>(ctx->small.as<u8>() + 8);
   u32* d_counts = reinterpret_cast<u32*>(ctx->small.as<u8>() + 16);
@@ -445,7 +458,7 @@ void run_encode(dcdf_ctx* ctx, EncodeJob& job, EncodeOut& out, bool want_pieces)
     time_begin(ctx, KT_ENCODE);
     CK(cudaEventRecord(ctx->fork_ev, st));  // clipped-tile lists run on the auxiliary stream beside the full-tile lists
     CK(cudaStreamWaitEvent(ctx->aux_stream, ctx->fork_ev, 0));
-    for (int list = 6; list >= 0; list--) {  // the fast-path lists (most units of a typical raster) go first
+    for (int list = 7; list >= 0; list--) {  // the fast-path lists (most units of a typical raster) go first
       EP.order = FP.order + (size_t)list * n_units;
       EP.order_count = d_counts + list;
       switch (job.encoding) {
@@ -910,10 +923,11 @@ int32_t dcdf_ctx_get_stat(const dcdf_ctx* ctx, const char* name, int64_t* value)
   if (!ctx || !name || !value) return DCDF_ERR_BAD_ARG;
   const std::string n(name);
   const uint32_t* c = ctx->last_list_counts;
-  if (n == "encode_units_fast") *value = (int64_t)c[5] + c[6];
+  if (n == "encode_units_fast") *value = (int64_t)c[5] + c[6] + c[7];
+  else if (n == "encode_units_edge") *value = (int64_t)c[7];
   else if (n == "encode_units_general") *value = (int64_t)c[0] + c[1] + c[2] + c[3] + c[4];
   else if (n == "encode_units_wide") *value = (int64_t)c[2] + c[3];
-  else if (n == "encode_units_clipped") *value = (int64_t)c[1] + c[3] + c[4] + c[6];
+  else if (n == "encode_units_clipped") *value = (int64_t)c[1] + c[3] + c[4] + c[6] + c[7];
   else return DCDF_ERR_BAD_ARG;
   return DCDF_OK;
 }

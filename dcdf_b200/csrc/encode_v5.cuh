@@ -31,22 +31,29 @@ namespace dcdf {
 
 constexpr int E5_THREADS = 64;
 constexpr int E5_POOL = 9 * 1024;
+// Edge tiles (list 7): the raster covers at most the top or the left half of the tree, so one warp holds every
+// level-3 node with cells; its structures are at most about half as large
+constexpr int E5_POOL_EDGE = 5 * 1024;
 
-struct E5Smem {
-  __align__(16) u8 pool[E5_POOL + 16];  // emission image (+ room for the alignment shift)
-  int4 cell[16][E5_THREADS];            // cells of the block's snapshot: [quad q][thread]
-  int2 l4s[4][E5_THREADS];              // (max, min) of the snapshot's level-4 nodes
-  int2 l4t[4][E5_THREADS];              // ... of the instant being encoded
-  u32 leaf[16][E5_THREADS];             // Log payload: low bytes of the four leaf codes of quad q
-  u32 qx[4][E5_THREADS];                // Log payload: low bytes of the four quad max codes of level-4 node a
-  u32 qn[4][E5_THREADS];                // ... and of the four quad min codes
-  int4 rec1[4];                         // level-1 nodes: tmax, tmin, first-cell diff, equal
-  int2 ent1[4];                         // level-1 log entries
-  u32 wt[2][2][4];                      // [warp][0 = snapshot, 1 = log][STRUCT, a1, b1, c1]
+// TT threads per tile (one per level-3 node that can hold cells), POOL bytes of emission image
+template <int TT, int POOL>
+struct E5SmemT {
+  __align__(16) u8 pool[POOL + 16];  // emission image (+ room for the alignment shift)
+  int4 cell[16][TT];                 // cells of the block's snapshot: [quad q][thread]
+  int2 l4s[4][TT];                   // (max, min) of the snapshot's level-4 nodes
+  int2 l4t[4][TT];                   // ... of the instant being encoded
+  u32 leaf[16][TT];                  // Log payload: low bytes of the four leaf codes of quad q
+  u32 qx[4][TT];                     // Log payload: low bytes of the four quad max codes of level-4 node a
+  u32 qn[4][TT];                     // ... and of the four quad min codes
+  int4 rec1[4];                      // level-1 nodes: tmax, tmin, first-cell diff, equal
+  int2 ent1[4];                      // level-1 log entries
+  u32 wt[2][2][4];                   // [warp][0 = snapshot, 1 = log][STRUCT, a1, b1, c1]
   u32 bm_off[12], bm_len[12];
   u32 n_bm;
   unsigned long long piece_off;
 };
+using E5Smem = E5SmemT<E5_THREADS, E5_POOL>;
+using E5SmemEdge = E5SmemT<32, E5_POOL_EDGE>;
 
 struct E5Cand {
   u32 in5, in4;        // internal flags: quad q = bit 15-q, level-4 node a = bit 3-a
@@ -78,7 +85,8 @@ struct E5Tot {
 };
 // Block totals of one candidate and the entry counts of its two DACs (snapshot.rs:71-79, log.rs:77-86): below the
 // level-1 nodes nothing is longer than two bytes, so DAC levels 2 and 3 only hold bytes of the root / level-1 entries.
-DCDF_DEVINL void e5_totals(E5Tot& T, const E5Smem& S, int cand, bool in0, u32 in1m, const u32 (&topx)[4], const u32 (&topn)[4]) {
+template <class Smem>
+DCDF_DEVINL void e5_totals(E5Tot& T, const Smem& S, int cand, bool in0, u32 in1m, const u32 (&topx)[4], const u32 (&topn)[4]) {
 #pragma unroll
   for (int i = 0; i < 4; i++) T.tot[i] = in0 ? S.wt[0][cand][i] + S.wt[1][cand][i] : 0u;
   T.I0 = in0 ? 1u : 0u;
@@ -236,7 +244,8 @@ DCDF_DEVINL void e5_store_word(u8* p, u32 w) {
 // quads, then the four quad max entries, then the min entries of the internal quads -- the order in which their second
 // bytes sit in DAC level 1 (dac.rs:109-121).  Log: cells of the instant come from a second (L2-resident) read of the
 // node, the snapshot's from shared memory.  Snapshot: the emission pass has just stored the cells in shared memory.
-template <bool FULL>
+// scell: the node's quad 0 in E5SmemT::cell, whose quads lie TT apart
+template <bool FULL, int TT = E5_THREADS>
 __device__ __noinline__ void e5_long_node(bool as_snapshot, const float* pn, i64 sr, float scale2, const int4* scell, int2 n4, u32 in5a,
                                           u8* xb1, u8* nb1, u32* pos /* lx1, rx1, rn1 */, int rl, int cl, int vec) {
   int4 q[4];
@@ -249,7 +258,7 @@ __device__ __noinline__ void e5_long_node(bool as_snapshot, const float* pn, i64
   u32 zx[4], zn[4];
 #pragma unroll
   for (int b = 0; b < 4; b++) {
-    const int4 s = scell[b * E5_THREADS];
+    const int4 s = scell[b * TT];
     const int4 t = as_snapshot ? s : q[b];
     int qmax, qmin, sqmax, sqmin;
     e4_qmm<FULL>(t, qmax, qmin);
@@ -303,28 +312,46 @@ struct E5Bulk {
   unsigned long long pad_;
 };
 
-// barrier over the 64 threads of one tile (named barrier 1 + tile slot; barrier 0 stays the CTA-wide one)
-DCDF_DEVINL void e5_tile_sync(int slot) { asm volatile("bar.sync %0, 64;" ::"r"(slot + 1) : "memory"); }
+// barrier over the threads of one tile: named barrier 1 + tile slot for a two-warp tile (barrier 0 stays the CTA-wide
+// one), the warp itself for a one-warp tile
+template <int NW>
+DCDF_DEVINL void e5_tile_sync(int slot) {
+  if (NW == 1) __syncwarp();
+  else asm volatile("bar.sync %0, 64;" ::"r"(slot + 1) : "memory");
+}
 
-// G tiles per CTA, one per 64-thread group.  The tiles are independent (own shared-memory slab, own named barrier);
-// what they share is the instruction stream: one CTA-wide barrier per instant keeps all 2G warps of the SM inside the
+// G tiles per CTA, one per group of NW warps.  The tiles are independent (own shared-memory slab, own named barrier);
+// what they share is the instruction stream: one CTA-wide barrier per instant keeps all NW * G warps of the SM inside the
 // same stretch of code, so instruction-cache lines fetched for one warp are hits for the others (with unsynchronised
 // CTAs the kernel spent a quarter of its issue slots waiting for instruction fetches).
-template <int G, bool FULL, bool BULK>
+// NW = 2: thread t of a tile is level-3 node t.  NW = 1 (edge tiles, FULL == false only): the unit has at most 32 rows or
+// at most 32 columns in the raster, so the level-3 nodes of the other half of the tree (rows 32-63: nodes 32-63;
+// columns 32-63: nodes 16-31 and 48-63) hold no cell.  Lane l takes node l (top half) or node l, l + 16 (left half):
+// each group of 16 lanes is still one level-1 node.  The missing half is two all-None level-1 nodes; what the NW = 2
+// kernel computes for such a node is a constant: no internal node below it (all its counters are 0), record
+// (None, INT32_MAX, diff 0, equal) and Log entries (0, 0), set once below.
+template <int G, bool FULL, bool BULK, int NW = 2>
 DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sync_mask);
 template <int G, bool FULL, bool BULK = false>
 __global__ void __launch_bounds__(E5_THREADS * G, 1) k_encode_v5(const EncParams P, const u32 stage_limit, const int sync_mask) {
   e5_body<G, FULL, BULK>(P, stage_limit, sync_mask);
 }
-template <int G, bool FULL, bool BULK>
+template <int G>
+__global__ void __launch_bounds__(32 * G, 1) k_encode_v5_edge(const EncParams P, const u32 stage_limit, const int sync_mask) {
+  e5_body<G, false, false, 1>(P, stage_limit, sync_mask);
+}
+template <int G, bool FULL, bool BULK, int NW>
 DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sync_mask) {
+  static_assert(NW == 2 || (NW == 1 && !FULL && !BULK), "one-warp tiles are clipped edge tiles");
+  constexpr int TT = 32 * NW;  // threads per tile
+  using Smem = std::conditional_t<NW == 2, E5Smem, E5SmemEdge>;
   // every row of four cells is 16-byte aligned -> 128-bit loads; BULK (host checked the alignment): loads from the staged tile
   const int vec = BULK ? 2 : (((P.stride_r | P.stride_t) & 3) == 0 && (((uintptr_t)P.data) & 15) == 0) ? 1 : 0;
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  const int slot = threadIdx.x / E5_THREADS;
-  constexpr size_t kSlab = sizeof(E5Smem) + (BULK ? sizeof(E5Bulk) : 0);
-  E5Smem& S = *reinterpret_cast<E5Smem*>(smem_raw + (size_t)slot * kSlab);
-  E5Bulk& SB = *reinterpret_cast<E5Bulk*>(smem_raw + (size_t)slot * kSlab + sizeof(E5Smem));  // only touched when BULK
+  const int slot = threadIdx.x / TT;
+  constexpr size_t kSlab = sizeof(Smem) + (BULK ? sizeof(E5Bulk) : 0);
+  Smem& S = *reinterpret_cast<Smem*>(smem_raw + (size_t)slot * kSlab);
+  E5Bulk& SB = *reinterpret_cast<E5Bulk*>(smem_raw + (size_t)slot * kSlab + sizeof(Smem));  // only touched when BULK
 
   const u32 n_order = *P.order_count;
   if (blockIdx.x * (u32)G >= n_order) return;
@@ -339,12 +366,14 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
     const u32 oi = blockIdx.x * (u32)G + (u32)g;
     if (oi < n_order) max_instants = max(max_instants, P.units[P.order[oi]].instants);
   }
-  const int tid = threadIdx.x % E5_THREADS, lane = tid & 31, warp = tid >> 5;
+  const int tid = threadIdx.x % TT, lane = tid & 31, warp = tid >> 5;
+  // the thread's level-3 node (NW = 1: the top half of the tree when the unit has at most 32 rows, else the left half)
+  const int node = NW == 2 ? tid : unit.rows <= 32 ? lane : lane < 16 ? lane : lane + 16;
   const float scale2 = (float)((i64)2 << unit.bits);
   const i64 sr = BULK ? 64 : P.stride_r;
   // the thread's 8x8 block
   const float* const base = BULK ? SB.raw + (8 * (int)morton_row(tid)) * 64 + 8 * (int)morton_col(tid)
-                                 : static_cast<const float*>(P.data) + unit.base + (i64)(8 * (int)morton_row(tid)) * sr + 8 * (int)morton_col(tid);
+                                 : static_cast<const float*>(P.data) + unit.base + (i64)(8 * (int)morton_row(node)) * sr + 8 * (int)morton_col(node);
   // BULK: thread r fetches row r of the tile (256 bytes) of one instant
   const float* const my_row = static_cast<const float*>(P.data) + unit.base + (i64)tid * P.stride_r;
   auto fetch_instant = [&](int t) {
@@ -356,23 +385,34 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
       e5_mbar_init(&SB.mbar, 1u);
       asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-    e5_tile_sync(slot);
+    e5_tile_sync<NW>(slot);
     if (unit.instants > 0) fetch_instant(0);
   }
   const bool owner2 = (lane & 3) == 0;
-  const int k1 = tid >> 4;  // own level-1 node
+  const int k1 = node >> 4;  // own level-1 node
   // rows / columns of the raster left from the origin of the thread's level-4 node a (clipped tiles)
-  const int rl8 = unit.rows - 8 * (int)morton_row(tid), cl8 = unit.cols - 8 * (int)morton_col(tid);
+  const int rl8 = unit.rows - 8 * (int)morton_row(node), cl8 = unit.cols - 8 * (int)morton_col(node);
 #define E5_RL(a) (rl8 - 4 * ((a) >> 1))
 #define E5_CL(a) (cl8 - 4 * ((a) & 1))
 
   {  // the emission image starts out all zero; every copy-out re-zeroes what it used
     uint4* z = reinterpret_cast<uint4*>(S.pool);
-    for (int i = tid; i < (E5_POOL + 16) / 16; i += E5_THREADS) z[i] = make_uint4(0, 0, 0, 0);
+    for (int i = tid; i < (int)(sizeof(S.pool) / 16); i += TT) z[i] = make_uint4(0, 0, 0, 0);
   }
   if (!FULL) {  // cells outside the raster are None in the snapshot image from the start
     for (int q = 0; q < 16; q++) S.cell[q][tid] = make_int4(E4_NONE, E4_NONE, E4_NONE, E4_NONE);
     for (int a = 0; a < 4; a++) S.l4s[a][tid] = make_int2(E4_NONE, INT32_MAX);
+  }
+  if (NW == 1 && lane == 0) {  // the two level-1 nodes without threads (see above); never written again
+    const u32 missing1 = unit.rows <= 32 ? 0xcu : 0xau;  // bit k: level-1 node k
+    for (int k = 0; k < 4; k++) {
+      if ((missing1 >> k) & 1u) {
+        S.rec1[k] = make_int4(E4_NONE, INT32_MAX, 0, 1);
+        S.ent1[k] = make_int2(0, 0);
+      }
+    }
+    for (int c = 0; c < 2; c++)
+      for (int i = 0; i < 4; i++) S.wt[1][c][i] = 0u;
   }
 
   u32 err = 0;
@@ -561,7 +601,7 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
       e5_count(C, owner2, ws);  // pass 0: structure only (the masks are still empty) -> the lower bound
 
       // ---------------- per-warp totals and the four level-1 records go through shared memory
-      if (pass == 1 && !forced) e5_tile_sync(slot);  // the other warp may still be reading the totals of pass 0
+      if (pass == 1 && !forced) e5_tile_sync<NW>(slot);  // the other warp may still be reading the totals of pass 0
 #pragma unroll
       for (int i = 0; i < 4; i++) {
         const u32 rs = __reduce_add_sync(0xffffffffu, ws[i]);
@@ -575,7 +615,7 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
         S.rec1[k1] = make_int4(t1max, t1min, diff1, eq1 ? 1 : 0);
         if (pass == 0) S.ent1[k1] = make_int2(e5_dx<FULL>(t1max, s1max), e5_dn(t1min, s1min));
       }
-      e5_tile_sync(slot);  // B1
+      e5_tile_sync<NW>(slot);  // B1
 
       // ---------------- root (every thread, redundantly)
       int n1dif[4];
@@ -646,12 +686,15 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
     const bool in0 = as_snapshot ? s_in0 : l_in0;
     const u32 in1m = as_snapshot ? s_in1 : l_in1;
     const int cand = as_snapshot ? 0 : 1;
-    // this warp's share of the root / level-1 entries: warp 0 the max DAC, warp 1 the min DAC (lane j = entry j)
-    E5Top top;
-    {
-      const bool mn = warp == 1;
+    // this warp's share of the root / level-1 entries: warp 0 the max DAC, warp 1 the min DAC (lane j = entry j); the
+    // warp of a one-warp tile takes both (top[0] max, top[1] min)
+    constexpr int NTOP = 3 - NW;
+    E5Top top[NTOP];
+#pragma unroll
+    for (int r = 0; r < NTOP; r++) {
+      const bool mn = NW == 2 ? warp == 1 : r == 1;
       const bool valid = mn ? (in0 && (lane == 0 || (lane < 5 && ((in1m >> (4 - lane)) & 1u)))) : (lane == 0 || (in0 && lane < 5));
-      e5_top(top, valid, mn ? e5_lane5(lane, e0n, e1n) : e5_lane5(lane, e0x, e1x), lane);
+      e5_top(top[r], valid, mn ? e5_lane5(lane, e0n, e1n) : e5_lane5(lane, e0x, e1x), lane);
     }
     const bool staged = my_size <= stage_limit;
     // The piece's place in the arena: the atomic's round trip is long, so a staged structure only looks at the answer
@@ -678,7 +721,7 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
     if (end != my_size) err |= EF_BAD_FORMAT;
     // the image starts `shift` bytes into the pool so that entry 1 of the max DAC's level 0 is 4-byte aligned
     const u32 shift = staged ? ((4u - ((DX.bytes[0] + 1u) & 3u)) & 3u) : 0u;
-    if (!staged) e5_tile_sync(slot);
+    if (!staged) e5_tile_sync<NW>(slot);
     u64 piece_off = 0;
     bool fits = true;
     if (!staged) {
@@ -687,9 +730,9 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
       if (!fits) err |= EF_ARENA_FULL;
       if (fits) {
         uint4* z = reinterpret_cast<uint4*>(P.arena + piece_off);
-        for (u32 i = tid; i < (my_size + 15u) / 16u; i += E5_THREADS) z[i] = make_uint4(0, 0, 0, 0);
+        for (u32 i = tid; i < (my_size + 15u) / 16u; i += TT) z[i] = make_uint4(0, 0, 0, 0);
       }
-      e5_tile_sync(slot);
+      e5_tile_sync<NW>(slot);
     }
     const bool emit = staged || fits;
 
@@ -791,7 +834,7 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
         if (!as_snapshot) e5_or_bits(eq_words, (Pn4 - Mn4) + 4u * R3 - R4, accE, nE);
       }
       if (x3) {  // own level-3 node
-        const u32 pos = Pn3 + 4u * R2p + (u32)(tid & 3);
+        const u32 pos = Pn3 + 4u * R2p + (u32)(node & 3);
         if (W.in3) {
           e5_or_bit(nm_words, pos);
           if ((W.mu >> 9) & 1u) e5_or_bit(nw0, Mn3 + R3);
@@ -801,7 +844,7 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
         if ((W.mu >> 8) & 1u) e5_or_bit(xw0, pos);
       }
       if (x2 && owner2) {  // level-2 node of the group
-        const u32 pos = Pn2 + 4u * R1 + (u32)((tid >> 2) & 3);
+        const u32 pos = Pn2 + 4u * R1 + (u32)((node >> 2) & 3);
         if (W.in2) {
           e5_or_bit(nm_words, pos);
           if ((W.mu >> 11) & 1u) e5_or_bit(nw0, Mn2 + R2own);
@@ -812,15 +855,17 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
       }
       // root and level-1 nodes.  Continuation bits of their DAC entries: warp 0 takes the max DAC, warp 1 the min DAC,
       // one lane per entry (at most five); nodemap and `equal` bits of these nodes: one thread.
-      {
-        u8* const tw0 = warp == 0 ? xw0 : nw0;
-        u8* const tw1 = warp == 0 ? e4_words_of(out, DX.hdr[1], T.cmax[1]) : e4_words_of(out, DN.hdr[1], T.cmin[1]);
-        u8* const tw2 = warp == 0 ? e4_words_of(out, DX.hdr[2], T.cmax[2]) : e4_words_of(out, DN.hdr[2], T.cmin[2]);
-        if (top.len > 1) e5_or_bit(tw0, top.pos[0]);
-        if (top.len > 2) e5_or_bit(tw1, top.pos[1]);
-        if (top.len > 3) e5_or_bit(tw2, top.pos[2]);
+#pragma unroll
+      for (int r = 0; r < NTOP; r++) {
+        const bool mx = NW == 2 ? warp == 0 : r == 0;
+        u8* const tw0 = mx ? xw0 : nw0;
+        u8* const tw1 = mx ? e4_words_of(out, DX.hdr[1], T.cmax[1]) : e4_words_of(out, DN.hdr[1], T.cmin[1]);
+        u8* const tw2 = mx ? e4_words_of(out, DX.hdr[2], T.cmax[2]) : e4_words_of(out, DN.hdr[2], T.cmin[2]);
+        if (top[r].len > 1) e5_or_bit(tw0, top[r].pos[0]);
+        if (top[r].len > 2) e5_or_bit(tw1, top[r].pos[1]);
+        if (top[r].len > 3) e5_or_bit(tw2, top[r].pos[2]);
       }
-      if (tid == E5_THREADS - 1) {
+      if (tid == TT - 1) {
         if (in0) {
           e5_or_bits(nm_words, 0, 0x10u | in1m, 5);
           if (!as_snapshot) {
@@ -836,7 +881,7 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
         }
       }
     }
-    e5_tile_sync(slot);  // B2a: all word-wide ORs done before the first byte store
+    e5_tile_sync<NW>(slot);  // B2a: all word-wide ORs done before the first byte store
 
     // ================= phase B: DAC bytes =================
     {
@@ -892,7 +937,7 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
         const u32 ml16 = (u32)(W.ml >> (48 - 16 * a)) & 0xffffu;
         const u32 lq = ((W.mq >> (12 - 4 * a)) & 0xfu) | (((W.mq >> (28 - 4 * a)) & 0xfu) & in5a);
         if ((ml16 & (e4_expand4(in5a) & 0xffffu)) | lq)
-          e5_long_node<FULL>(as_snapshot, e5_node_ptr(pt, sr, a), sr, scale2, &S.cell[4 * a][tid], n4, in5a, xb1, nb1, pos, E5_RL(a), E5_CL(a), vec);
+          e5_long_node<FULL, TT>(as_snapshot, e5_node_ptr(pt, sr, a), sr, scale2, &S.cell[4 * a][tid], n4, in5a, xb1, nb1, pos, E5_RL(a), E5_CL(a), vec);
       }
     }
     if (emit) {
@@ -924,7 +969,7 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
       }
       if (x3) {
         const u32 zx = zigzag32(as_snapshot ? e5_dx<FULL>(t2max, t3max) : e5_dx<FULL>(t3max, s3max));
-        xb0[Pn3 + 4u * R2p + (u32)(tid & 3)] = (u8)zx;
+        xb0[Pn3 + 4u * R2p + (u32)(node & 3)] = (u8)zx;
         if (zx > 0xffu) e5_hi(xb1, zx, bx3 + e4_f3(pre[1]));
         if (W.in3) {
           const u32 zn = zigzag32(as_snapshot ? e5_dn(t3min, t2min) : e5_dn(t3min, s3min));
@@ -934,7 +979,7 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
       }
       if (x2 && owner2) {
         const u32 zx = zigzag32(as_snapshot ? e5_dx<FULL>(t1max, t2max) : e5_dx<FULL>(t2max, s2max));
-        xb0[Pn2 + 4u * R1 + (u32)((tid >> 2) & 3)] = (u8)zx;
+        xb0[Pn2 + 4u * R1 + (u32)((node >> 2) & 3)] = (u8)zx;
         if (zx > 0xffu) e5_hi(xb1, zx, bx2 + e4_f2(pre[1]));
         if (W.in2) {
           const u32 zn = zigzag32(as_snapshot ? e5_dn(t2min, t1min) : e5_dn(t2min, s2min));
@@ -942,17 +987,19 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
           if (zn > 0xffu) e5_hi(nb1, zn, bn2 + e4_f2(pre[3]));
         }
       }
-      {  // root and level-1 entries (any length): the same lanes as in phase A
-        u8* const tb0 = warp == 0 ? xb0 : nb0;
-        u8* const tb1 = warp == 0 ? xb1 : nb1;
-        u8* const tb2 = out + (warp == 0 ? DX.bytes[2] : DN.bytes[2]);
-        u8* const tb3 = out + (warp == 0 ? DX.bytes[3] : DN.bytes[3]);
-        if (top.len > 0) tb0[top.pos[0]] = (u8)top.z;
-        if (top.len > 1) tb1[top.pos[1]] = (u8)(top.z >> 8);
-        if (top.len > 2) tb2[top.pos[2]] = (u8)(top.z >> 16);
-        if (top.len > 3) tb3[top.pos[3]] = (u8)(top.z >> 24);
+#pragma unroll
+      for (int r = 0; r < NTOP; r++) {  // root and level-1 entries (any length): the same lanes as in phase A
+        const bool mx = NW == 2 ? warp == 0 : r == 0;
+        u8* const tb0 = mx ? xb0 : nb0;
+        u8* const tb1 = mx ? xb1 : nb1;
+        u8* const tb2 = out + (mx ? DX.bytes[2] : DN.bytes[2]);
+        u8* const tb3 = out + (mx ? DX.bytes[3] : DN.bytes[3]);
+        if (top[r].len > 0) tb0[top[r].pos[0]] = (u8)top[r].z;
+        if (top[r].len > 1) tb1[top[r].pos[1]] = (u8)(top[r].z >> 8);
+        if (top[r].len > 2) tb2[top[r].pos[2]] = (u8)(top[r].z >> 16);
+        if (top[r].len > 3) tb3[top[r].pos[3]] = (u8)(top[r].z >> 24);
       }
-      if (warp == 1 && lane >= 16) {  // structure header (snapshot.rs:48-52 / log.rs:53-58): k, shape, sidelen; DAC level counts
+      if ((NW == 1 || warp == 1) && lane >= 16) {  // structure header (snapshot.rs:48-52 / log.rs:53-58): k, shape, sidelen; DAC level counts
         const u32 i = lane - 16u;
         if (i < 13u) {
           const u32 word = i < 5u ? (u32)unit.rows : i < 9u ? (u32)unit.cols : 64u;
@@ -964,7 +1011,7 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
         }
       }
     }
-    e5_tile_sync(slot);  // B2
+    e5_tile_sync<NW>(slot);  // B2
     // BULK: nobody reads the staged tile any more -> the next instant's rows start coming in behind the rank directories
     if (BULK && inst + 1 < unit.instants) fetch_instant(inst + 1);
 
@@ -974,7 +1021,7 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
       const u32 n_fix = as_snapshot ? 1u : 2u;
       const u32 n_bm = n_fix + (u32)DX.levels + (u32)DN.levels;
 #pragma unroll 1
-      for (u32 i = warp; i < n_bm; i += 2) {
+      for (u32 i = warp; i < n_bm; i += NW) {
         u32 hdr, len;
         if (i == 0) { hdr = nm_hdr; len = nm_len; }
         else if (i < n_fix) { hdr = eq_hdr; len = eq_len; }
@@ -1010,7 +1057,7 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
       }
     }
     if (decltype(in_shared)::value && tid == 0) publish_piece();
-    e5_tile_sync(slot);  // B3
+    e5_tile_sync<NW>(slot);  // B3
 
     // ================= copy-out (re-aligning by `shift` bytes) and re-zero the image =================
     if constexpr (decltype(in_shared)::value) {
@@ -1022,7 +1069,7 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
       const u32 sh = 8u * shift;
       const u32 n16 = (my_size + 15u) / 16u;
 #pragma unroll 1
-      for (u32 i = tid; i < n16; i += E5_THREADS) {
+      for (u32 i = tid; i < n16; i += TT) {
         const uint4 v = *reinterpret_cast<const uint4*>(src + 4u * i);
         const u32 nx = src[4u * i + 4u];
         uint4 o;
@@ -1030,9 +1077,9 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
         o.z = __funnelshift_r(v.z, v.w, sh); o.w = __funnelshift_r(v.w, nx, sh);
         if (fits) dst[i] = o;
       }
-      e5_tile_sync(slot);  // every word has been read (a chunk's last word belongs to the next one's first)
+      e5_tile_sync<NW>(slot);  // every word has been read (a chunk's last word belongs to the next one's first)
 #pragma unroll 1
-      for (u32 i = tid; i < n16 + 1u; i += E5_THREADS) *reinterpret_cast<uint4*>(src + 4u * i) = make_uint4(0, 0, 0, 0);
+      for (u32 i = tid; i < n16 + 1u; i += TT) *reinterpret_cast<uint4*>(src + 4u * i) = make_uint4(0, 0, 0, 0);
     }
 
     };

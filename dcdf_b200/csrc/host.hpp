@@ -125,7 +125,7 @@ struct dcdf_ctx {
     int search_no_cache = 0;             // the search's writing pass recomputes instead of reading cached findings
     int trace = 0;                       // host-side phase times of the encode pipeline on stderr (adds stream syncs)
   } opt;
-  uint32_t last_list_counts[7] = {0, 0, 0, 0, 0, 0, 0};  // units per encoder work list of the last build (dcdf_ctx_get_stat)
+  uint32_t last_list_counts[8] = {0, 0, 0, 0, 0, 0, 0, 0};  // units per encoder work list of the last build (dcdf_ctx_get_stat)
   // scratch
   dcdf::DevBuf input_copy, units, ustats, istats, slices, sstate, tbl_scratch, order, pieces, results, stored, chunk_off,
       arena, small, exact, query_in, query_out, query_aux, query_aux2, search_cache, tree_buf;

@@ -1022,6 +1022,8 @@ __global__ void __launch_bounds__(256) k_finalize_tree(const TreeParams P, u32 n
           u32 list = (narrow ? 0u : 2u) + (full ? 0u : 1u);
           if (narrow && !full && unit.lo == 0) list = 4u;  // clipped, but still a 64-side tree: k_encode_v4<.., false>
           if (fast) list = full ? 5u : 6u;                  // k_encode_v5<.., true / false>
+          // ... at most 32 rows or columns in the raster: half of the tree holds no cell -> one warp per tile
+          if (fast && !full && min(unit.rows, unit.cols) <= 32) list = 7u;  // k_encode_v5_edge
           P.order[(size_t)list * P.order_pitch + atomicAdd(&P.order_counts[list], 1u)] = u;
         }
       }

@@ -102,7 +102,8 @@ int32_t dcdf_ctx_set_stream(dcdf_ctx* ctx, void* cuda_stream);
  *   "trace" 0|1             host-side phase times of the encode pipeline on stderr
  * Unknown names return DCDF_ERR_BAD_ARG. */
 int32_t dcdf_ctx_set_option(dcdf_ctx* ctx, const char* name, int64_t value);
-/* Counters of the last build call: "encode_units_fast" (units encoded by the fast-path kernel), "encode_units_general",
+/* Counters of the last build call: "encode_units_fast" (units encoded by the fast-path kernels), "encode_units_edge" (the
+ * part of those with at most 32 rows or columns in the raster, one warp per tile), "encode_units_general",
  * "encode_units_wide" (64-bit values), "encode_units_clipped". */
 int32_t dcdf_ctx_get_stat(const dcdf_ctx* ctx, const char* name, int64_t* value);
 int32_t dcdf_ctx_synchronize(dcdf_ctx* ctx);
