@@ -80,13 +80,11 @@ DCDF_DEVINL void e5_count(const E5Cand& C, bool owner2, u32* w /* [4] */) {
 
 struct E5Tot {
   u32 tot[4];
-  u32 cmax[4], cmin[4];
   u32 I0, I1, nm_len, n_int;
 };
-// Block totals of one candidate and the entry counts of its two DACs (snapshot.rs:71-79, log.rs:77-86): below the
-// level-1 nodes nothing is longer than two bytes, so DAC levels 2 and 3 only hold bytes of the root / level-1 entries.
+// Block totals of one candidate (snapshot.rs:71-79, log.rs:77-86)
 template <class Smem>
-DCDF_DEVINL void e5_totals(E5Tot& T, const Smem& S, int cand, bool in0, u32 in1m, const u32 (&topx)[4], const u32 (&topn)[4]) {
+DCDF_DEVINL void e5_totals(E5Tot& T, const Smem& S, int cand, bool in0, u32 in1m) {
 #pragma unroll
   for (int i = 0; i < 4; i++) T.tot[i] = in0 ? S.wt[0][cand][i] + S.wt[1][cand][i] : 0u;
   T.I0 = in0 ? 1u : 0u;
@@ -94,36 +92,41 @@ DCDF_DEVINL void e5_totals(E5Tot& T, const Smem& S, int cand, bool in0, u32 in1m
   const u32 upper = T.I0 + T.I1 + e4_f2(T.tot[0]) + e4_f3(T.tot[0]) + e4_f4(T.tot[0]);
   T.n_int = upper + e4_f5(T.tot[0]);
   T.nm_len = 1u + 4u * upper;
-  T.cmax[0] = 1u + 4u * T.n_int;
-  T.cmin[0] = T.n_int;
-#pragma unroll
-  for (int j = 1; j < 4; j++) {
-    T.cmax[j] = topx[j] + (j == 1 ? e4_fsum(T.tot[1]) + T.tot[2] : 0u);
-    T.cmin[j] = topn[j] + (j == 1 ? e4_fsum(T.tot[3]) : 0u);
-  }
 }
 
-// The root's and the level-1 nodes' entries of one DAC, one per lane: lane 0 = root, lane 1 + k = level-1 node k.  They
-// are the first entries of the DAC in BFS order, hence the first ones of every DAC level they reach: entry -> zigzag
-// code, byte length, position on each level, and the number of top entries per level (dac.rs:109-121).
+// The root's and the level-1 nodes' entries of a DAC are held one per lane: lane 0 = root, lane 1 + k = level-1 node k.
+// They are the first entries of the DAC in BFS order, hence the first ones of every DAC level they reach (dac.rs:109-121).
+// Byte length of such an entry (0: the entry does not exist)
+DCDF_DEVINL int e5_len(bool valid, int e) {
+  return valid ? 1 + (e4_longer<1>(e) ? 1 : 0) + (e4_longer<2>(e) ? 1 : 0) + (e4_longer<3>(e) ? 1 : 0) : 0;
+}
+// ... as nibbles 1..3 (nibble j set when the entry reaches DAC level j): a warp sum then counts the top entries per level
+DCDF_DEVINL u32 e5_nib(int len) { return 0x1110u & ((1u << (4 * len)) - 1u); }
+// an entry of the winner: zigzag code, length, position of its bytes on DAC levels 0 and 1 (levels 2 and 3: e5_top_long)
 struct E5Top {
   u32 z;
-  int len;       // 0: the entry does not exist
-  u32 pos[4];    // position of the entry's byte j on DAC level j
-  u32 n[4];      // top entries that reach level j
+  int len;
+  u32 pos0, pos1;
 };
-DCDF_DEVINL void e5_top(E5Top& t, bool valid, int e, u32 lane) {
-  t.z = zigzag32(e);
-  t.len = valid ? 1 + (e4_longer<1>(e) ? 1 : 0) + (e4_longer<2>(e) ? 1 : 0) + (e4_longer<3>(e) ? 1 : 0) : 0;
-  const u32 lt = (1u << lane) - 1u;
-#pragma unroll
-  for (int j = 0; j < 4; j++) {
-    const u32 m = __ballot_sync(0xffffffffu, t.len > j);
-    t.pos[j] = (u32)__popc(m & lt);
-    t.n[j] = (u32)__popc(m);
-  }
+
+// The stream items of a candidate, one per lane, in stream order (snapshot.rs:48-58 / log.rs:53-64, dac.rs:37-44):
+// lane 0 = nodemap bitmap, 1 = `equal` bitmap (Logs only), 2 + j = level j of the max DAC, 6 + j = level j of the min
+// DAC; the DAC's level-count byte goes with its level 0.  ntop: top entries per DAC level (e5_nib, min DAC << 16).
+// cnt = the item's bits or entries; returns its size in bytes.  Below the level-1 nodes nothing is longer than two bytes,
+// so DAC levels 2 and 3 only hold bytes of the root / level-1 entries.
+DCDF_DEVINL u32 e5_item(u32& cnt, const E5Tot& T, bool as_log, u32 ntop, int lane) {
+  const int j = (lane - 2) & 7, lev = j & 3;
+  const bool mn = j >= 4;
+  u32 c = (ntop >> (4 * j)) & 0xfu;
+  if (lev == 0) c = mn ? T.n_int : 1u + 4u * T.n_int;
+  else if (lev == 1) c += mn ? e4_fsum(T.tot[3]) : e4_fsum(T.tot[1]) + T.tot[2];
+  if (lane == 0) c = T.nm_len;
+  if (lane == 1) c = T.nm_len - T.n_int;
+  cnt = lane < 10 ? c : 0u;
+  if (lane < 2) return (lane == 0 || as_log) ? bitmap_size(c) : 0u;
+  return lane >= 10 ? 0u : (c ? bitmap_size(c) + c : 0u) + (lev == 0 ? 1u : 0u);
 }
-DCDF_DEVINL int e5_lane5(u32 lane, int v0, const int (&v)[4]) { return lane == 0 ? v0 : lane == 1 ? v[0] : lane == 2 ? v[1] : lane == 3 ? v[2] : v[3]; }
+
 // second byte of a two-byte code (DAC level 1): rare, out of line; returns the next position
 __device__ __noinline__ u32 e5_hi(u8* b1, u32 z, u32 r1) {
   b1[r1] = (u8)(z >> 8);
@@ -149,6 +152,24 @@ DCDF_DEVINL void e5_or_bit(u8* bytes, u32 bitpos) {
   const uintptr_t A = (uintptr_t)bytes;
   const u32 g = bitpos + 8u * (u32)(A & 3u);
   e4_red_or(reinterpret_cast<u32*>(A & ~(uintptr_t)3) + (g >> 5), e4_bswap(0x80000000u >> (g & 31u)));
+}
+// Bytes 3 and 4 of the top entries (rare: the root of a Snapshot, or a jump of 2^15 or more): continuation bits on DAC
+// levels 1 and 2 (phase A) or the bytes on levels 2 and 3 (phase B).  l0: lane of the DAC's level-0 item.  Warp-wide.
+__device__ __noinline__ void e5_top_long(bool bytes, u8* out, const E5Top& t, int l0, u32 hdr, u32 cnt, u32 at) {
+  const u32 lt = (1u << (threadIdx.x & 31u)) - 1u;
+  const u32 p2 = (u32)__popc(__ballot_sync(0xffffffffu, t.len > 2) & lt);
+  if (!bytes) {
+    u8* const w1 = e4_words_of(out, __shfl_sync(0xffffffffu, hdr, l0 + 1), __shfl_sync(0xffffffffu, cnt, l0 + 1));
+    u8* const w2 = e4_words_of(out, __shfl_sync(0xffffffffu, hdr, l0 + 2), __shfl_sync(0xffffffffu, cnt, l0 + 2));
+    if (t.len > 2) e5_or_bit(w1, t.pos1);
+    if (t.len > 3) e5_or_bit(w2, p2);
+  } else {
+    const u32 p3 = (u32)__popc(__ballot_sync(0xffffffffu, t.len > 3) & lt);
+    u8* const b2 = out + __shfl_sync(0xffffffffu, at, l0 + 2);
+    u8* const b3 = out + __shfl_sync(0xffffffffu, at, l0 + 3);
+    if (t.len > 2) b2[p2] = (u8)(t.z >> 16);
+    if (t.len > 3) b3[p3] = (u8)(t.z >> 24);
+  }
 }
 // One level-4 node (4x4 cells at pn, row stride sr) as four quads (x, y = upper row; z, w = lower row).
 // Clipped tiles (FULL == false): rl / cl = rows / columns of the node that lie inside the raster (may be <= 0); cells
@@ -389,6 +410,7 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
     if (unit.instants > 0) fetch_instant(0);
   }
   const bool owner2 = (lane & 3) == 0;
+  const bool is1 = (u32)(lane - 1) < 4u;  // lane 1 + k holds level-1 node k at the top of the tree
   const int k1 = node >> 4;  // own level-1 node
   // rows / columns of the raster left from the origin of the thread's level-4 node a (clipped tiles)
   const int rl8 = unit.rows - 8 * (int)morton_row(node), cl8 = unit.cols - 8 * (int)morton_col(node);
@@ -442,13 +464,14 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
     bool eq3 = false, u3 = false;
     int t2max = 0, t2min = 0, t1max = 0, t1min = 0, t0max = 0, t0min = 0;
     bool u2 = false, eq2 = false, u0 = false, eq0 = false;
-    int n1max[4], n1min[4];
-    u32 n1flags = 0;             // bit k: level-1 node k is `equal`
+    // lanes 1..4: level-1 node lane - 1 (record, flags, Log entries)
+    int n1max = 0, n1min = 0, l_e1max = 0, l_e1min = 0;
+    bool n1un = false, n1eq = false;
     u32 l_in1 = 0, s_in1 = 0;    // level-1 internal flags, node k = bit 3-k
     bool l_in0 = false, s_in0 = false;
-    int l_e1max[4], l_e1min[4];
     u32 wl[4] = {0, 0, 0, 0}, ws[4] = {0, 0, 0, 0};
     E5Tot T;
+    u32 ntop = 0, item_cnt = 0, item_size = 0;  // the winner's top-entry counts and this lane's stream item (e5_item)
     bool as_snapshot = forced;
     u32 my_size = 0, log_size = 0;
 
@@ -617,49 +640,42 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
       }
       e5_tile_sync<NW>(slot);  // B1
 
-      // ---------------- root (every thread, redundantly)
-      int n1dif[4];
-      n1flags = 0;
-#pragma unroll
-      for (int k = 0; k < 4; k++) {
-        const int4 r = S.rec1[k];
-        n1max[k] = r.x; n1min[k] = r.y; n1dif[k] = r.z;
-        if (r.w != 0) n1flags |= 1u << k;
+      // ---------------- root from the level-1 records, one per lane (lane 1 + k: node k; the others hold neutral values)
+      {
+        const int4 r = S.rec1[(lane - 1) & 3];
+        n1max = is1 ? r.x : INT32_MIN; n1min = is1 ? r.y : INT32_MAX;
+        n1un = e4_unif<FULL>(r.x, r.y);
+        n1eq = r.w != 0;
+        t0max = __reduce_max_sync(0xffffffffu, n1max);
+        t0min = __reduce_min_sync(0xffffffffu, n1min);
+        const int dif0 = shfl(r.z, 1);
+        eq0 = __ballot_sync(0xffffffffu, is1 && n1eq && r.z == dif0) == 0x1eu;
+        // bit 1 + k of a ballot -> bit 3 - k
+        s_in1 = __brev(__ballot_sync(0xffffffffu, is1 && !n1un)) >> 27;
+        l_in1 = __brev(__ballot_sync(0xffffffffu, is1 && !n1un && !n1eq)) >> 27;
+        if (pass == 0) { const int2 e = S.ent1[(lane - 1) & 3]; l_e1max = e.x; l_e1min = e.y; }
       }
-      t0max = max(max(n1max[0], n1max[1]), max(n1max[2], n1max[3]));
-      t0min = min(min(n1min[0], n1min[1]), min(n1min[2], n1min[3]));
       u0 = t0max == t0min;
-      eq0 = n1flags == 0xfu && n1dif[1] == n1dif[0] && n1dif[2] == n1dif[0] && n1dif[3] == n1dif[0];
-      l_in1 = 0; s_in1 = 0;
-#pragma unroll
-      for (int k = 0; k < 4; k++) {
-        const bool un = e4_unif<FULL>(n1max[k], n1min[k]);
-        if (!un) s_in1 |= 1u << (3 - k);
-        if (!un && !((n1flags >> k) & 1u)) l_in1 |= 1u << (3 - k);
-      }
       l_in0 = !u0 && !eq0; s_in0 = !u0;
-      if (pass == 0) {
-#pragma unroll
-        for (int k = 0; k < 4; k++) { const int2 e = S.ent1[k]; l_e1max[k] = e.x; l_e1min[k] = e.y; }
-      }
 
-      // ---------------- exact size of this pass's candidate (snapshot.rs:84-93, log.rs:92-98)
+      // ---------------- exact size of this pass's candidate (snapshot.rs:84-93, log.rs:92-98): one stream item per lane
       const bool as_log = pass == 0;
-      int c_e1max[4], c_e1min[4];
-#pragma unroll
-      for (int k = 0; k < 4; k++) { c_e1max[k] = as_log ? l_e1max[k] : e5_dx<FULL>(t0max, n1max[k]); c_e1min[k] = as_log ? l_e1min[k] : e5_dn(n1min[k], t0min); }
       E5Tot Tc;
+      u32 c_ntop, c_cnt;
       {
         const bool c_in0 = as_log ? l_in0 : s_in0;
-        const u32 c_in1 = as_log ? l_in1 : s_in1;
-        E5Top tx, tn;
-        e5_top(tx, lane == 0 || (c_in0 && lane < 5), e5_lane5(lane, as_log ? t0max - s0max : t0max, c_e1max), lane);
-        e5_top(tn, c_in0 && (lane == 0 || (lane < 5 && ((c_in1 >> (4 - lane)) & 1u))), e5_lane5(lane, as_log ? t0min - s0min : t0min, c_e1min), lane);
-        e5_totals(Tc, S, as_log ? 1 : 0, c_in0, c_in1, tx.n, tn.n);
+        const bool c_int1 = !n1un && !(as_log && n1eq);  // own level-1 node internal
+        const int ex = lane == 0 ? (as_log ? t0max - s0max : t0max) : as_log ? l_e1max : e5_dx<FULL>(t0max, n1max);
+        const int en = lane == 0 ? (as_log ? t0min - s0min : t0min) : as_log ? l_e1min : e5_dn(n1min, t0min);
+        const int lx = e5_len(lane == 0 || (c_in0 && is1), ex), ln = e5_len(c_in0 && (lane == 0 || (is1 && c_int1)), en);
+        c_ntop = __reduce_add_sync(0xffffffffu, e5_nib(lx) | (e5_nib(ln) << 16));
+        e5_totals(Tc, S, as_log ? 1 : 0, c_in0, as_log ? l_in1 : s_in1);
       }
-      const u32 size = 13u + bitmap_size(Tc.nm_len) + (as_log ? bitmap_size(Tc.nm_len - Tc.n_int) : 0u) + e4_dac_size(Tc.cmax) + e4_dac_size(Tc.cmin);
+      const u32 c_size = e5_item(c_cnt, Tc, as_log, c_ntop, lane);
+      const u32 size = 13u + __reduce_add_sync(0xffffffffu, c_size);
       if (as_log) {
         T = Tc;
+        ntop = c_ntop; item_cnt = c_cnt; item_size = c_size;
         log_size = size; my_size = size;
         // lower bound of the Snapshot: every entry takes at least one byte
         const u32 st = s_in0 ? S.wt[0][0][0] + S.wt[1][0][0] : 0u;
@@ -669,7 +685,7 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
         if (!(snap_lb <= log_size)) break;  // the Log wins without looking closer
       } else {
         as_snapshot = forced || size <= log_size;  // ties go to the snapshot (chunk.rs:62)
-        if (as_snapshot) { T = Tc; my_size = size; }
+        if (as_snapshot) { T = Tc; ntop = c_ntop; item_cnt = c_cnt; item_size = c_size; my_size = size; }
       }
     }
 
@@ -678,9 +694,7 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
     W.in5 = as_snapshot ? C.in5 : L.in5; W.in4 = as_snapshot ? C.in4 : L.in4;
     W.in3 = as_snapshot ? C.in3 : L.in3; W.in2 = as_snapshot ? C.in2 : L.in2; W.in1 = as_snapshot ? C.in1 : L.in1;
     W.ml = as_snapshot ? C.ml : L.ml; W.mq = as_snapshot ? C.mq : L.mq; W.mu = as_snapshot ? C.mu : L.mu;
-    int e1x[4], e1n[4];
-#pragma unroll
-    for (int k = 0; k < 4; k++) { e1x[k] = as_snapshot ? e5_dx<FULL>(t0max, n1max[k]) : l_e1max[k]; e1n[k] = as_snapshot ? e5_dn(n1min[k], t0min) : l_e1min[k]; }
+    const int e1x = as_snapshot ? e5_dx<FULL>(t0max, n1max) : l_e1max, e1n = as_snapshot ? e5_dn(n1min, t0min) : l_e1min;
     const int e0x = as_snapshot ? t0max : t0max - s0max, e0n = as_snapshot ? t0min : t0min - s0min;
     const u32 nm_len = T.nm_len, n_int = T.n_int, I0 = T.I0, I1 = T.I1;
     const bool in0 = as_snapshot ? s_in0 : l_in0;
@@ -690,11 +704,16 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
     // warp of a one-warp tile takes both (top[0] max, top[1] min)
     constexpr int NTOP = 3 - NW;
     E5Top top[NTOP];
+    const u32 lt = (1u << lane) - 1u;
 #pragma unroll
     for (int r = 0; r < NTOP; r++) {
       const bool mn = NW == 2 ? warp == 1 : r == 1;
-      const bool valid = mn ? (in0 && (lane == 0 || (lane < 5 && ((in1m >> (4 - lane)) & 1u)))) : (lane == 0 || (in0 && lane < 5));
-      e5_top(top[r], valid, mn ? e5_lane5(lane, e0n, e1n) : e5_lane5(lane, e0x, e1x), lane);
+      const bool valid = mn ? (in0 && (lane == 0 || (is1 && !n1un && !(!as_snapshot && n1eq)))) : (lane == 0 || (in0 && is1));
+      const int e = lane == 0 ? (mn ? e0n : e0x) : (mn ? e1n : e1x);
+      top[r].z = zigzag32(e);
+      top[r].len = e5_len(valid, e);
+      top[r].pos0 = (u32)__popc(__ballot_sync(0xffffffffu, top[r].len > 0) & lt);
+      top[r].pos1 = (u32)__popc(__ballot_sync(0xffffffffu, top[r].len > 1) & lt);
     }
     const bool staged = my_size <= stage_limit;
     // The piece's place in the arena: the atomic's round trip is long, so a staged structure only looks at the answer
@@ -711,16 +730,19 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
       my_off = atomicAdd(P.arena_head, (unsigned long long)need);
       if (!staged) publish_piece();
     }
-    // stream layout (snapshot.rs:48-58 / log.rs:53-64)
+    // stream layout (snapshot.rs:48-58 / log.rs:53-64, dac.rs:37-44): where each lane's item (e5_item) starts; a DAC
+    // level's bitmap header sits at item_hdr, its bytes at item_at
+    const u32 item_hdr = 13u + e4_warp_excl(item_size, lane) + ((lane == 2 || lane == 6) ? 1u : 0u);
+    const u32 item_at = item_hdr + (item_cnt ? bitmap_size(item_cnt) : 0u);
     const u32 eq_len = nm_len - n_int;
     const u32 nm_hdr = 13u;
     const u32 eq_hdr = nm_hdr + bitmap_size(nm_len);
-    E4Dac DX, DN;
-    u32 end = e4_lay_dac(DX, as_snapshot ? eq_hdr : eq_hdr + bitmap_size(eq_len), T.cmax);
-    end = e4_lay_dac(DN, end, T.cmin);
-    if (end != my_size) err |= EF_BAD_FORMAT;
+    const u32 x_hdr0 = shfl(item_hdr, 2), x_at0 = shfl(item_at, 2), x_at1 = shfl(item_at, 3);
+    const u32 n_hdr0 = shfl(item_hdr, 6), n_at0 = shfl(item_at, 6), n_at1 = shfl(item_at, 7);
+    const u32 lv = __ballot_sync(0xffffffffu, item_cnt != 0u);
+    const u32 x_levels = (u32)__popc(lv & 0x3cu), n_levels = (u32)__popc(lv & 0x3c0u);
     // the image starts `shift` bytes into the pool so that entry 1 of the max DAC's level 0 is 4-byte aligned
-    const u32 shift = staged ? ((4u - ((DX.bytes[0] + 1u) & 3u)) & 3u) : 0u;
+    const u32 shift = staged ? ((4u - ((x_at0 + 1u) & 3u)) & 3u) : 0u;
     if (!staged) e5_tile_sync<NW>(slot);
     u64 piece_off = 0;
     bool fits = true;
@@ -743,12 +765,12 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
     u8* const out = decltype(in_shared)::value ? S.pool + shift : P.arena + piece_off;
     u8* const nm_words = e4_words_of(out, nm_hdr, nm_len);
     u8* const eq_words = e4_words_of(out, eq_hdr, eq_len);
-    u8* const xw0 = e4_words_of(out, DX.hdr[0], T.cmax[0]);  // continuation bits of DAC level 0
-    u8* const nw0 = e4_words_of(out, DN.hdr[0], T.cmin[0]);
-    u8* const xb0 = out + DX.bytes[0];
-    u8* const xb1 = out + DX.bytes[1];
-    u8* const nb0 = out + DN.bytes[0];
-    u8* const nb1 = out + DN.bytes[1];
+    u8* const xw0 = e4_words_of(out, x_hdr0, 1u + 4u * n_int);  // continuation bits of DAC level 0
+    u8* const nw0 = e4_words_of(out, n_hdr0, n_int);
+    u8* const xb0 = out + x_at0;
+    u8* const xb1 = out + x_at1;
+    u8* const nb0 = out + n_at0;
+    u8* const nb1 = out + n_at1;
 
     // block-wide positions
     const u32 T0 = T.tot[0];
@@ -774,8 +796,8 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
     const u32 R3 = e4_f3(pre[0]), R4 = e4_f4(pre[0]), R5 = e4_f5(pre[0]);
     // positions of this thread's second bytes (DAC level 1) per tree level: entries longer than one byte before them
     const u32 tx = T.tot[1], tn = T.tot[3];
-    const u32 bx2 = T.cmax[1] - e4_fsum(tx) - T.tot[2], bx3 = bx2 + e4_f2(tx), bx4 = bx3 + e4_f3(tx), bx5 = bx4 + e4_f4(tx), bx6 = bx5 + e4_f5(tx);
-    const u32 bn2 = T.cmin[1] - e4_fsum(tn), bn3 = bn2 + e4_f2(tn), bn4 = bn3 + e4_f3(tn), bn5 = bn4 + e4_f4(tn);
+    const u32 bx2 = (ntop >> 4) & 0xfu, bx3 = bx2 + e4_f2(tx), bx4 = bx3 + e4_f3(tx), bx5 = bx4 + e4_f4(tx), bx6 = bx5 + e4_f5(tx);
+    const u32 bn2 = (ntop >> 20) & 0xfu, bn3 = bn2 + e4_f2(tn), bn4 = bn3 + e4_f3(tn), bn5 = bn4 + e4_f4(tn);
     // log "equal" flags of nodes that are neither uniform nor internal
     const u32 eqb5 = ~u5 & eq5 & 0xffffu, eqb4 = ~u4 & eq4 & 0xfu;
     const bool eqb3 = !u3 && eq3, eqb2 = !u2 && eq2;
@@ -853,31 +875,21 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
         }
         if ((W.mu >> 10) & 1u) e5_or_bit(xw0, pos);
       }
-      // root and level-1 nodes.  Continuation bits of their DAC entries: warp 0 takes the max DAC, warp 1 the min DAC,
-      // one lane per entry (at most five); nodemap and `equal` bits of these nodes: one thread.
+      // root and level-1 nodes, lane 0 = root, lane 1 + k = node k.  Continuation bits of their DAC entries: warp 0
+      // takes the max DAC, warp 1 the min DAC
 #pragma unroll
       for (int r = 0; r < NTOP; r++) {
         const bool mx = NW == 2 ? warp == 0 : r == 0;
-        u8* const tw0 = mx ? xw0 : nw0;
-        u8* const tw1 = mx ? e4_words_of(out, DX.hdr[1], T.cmax[1]) : e4_words_of(out, DN.hdr[1], T.cmin[1]);
-        u8* const tw2 = mx ? e4_words_of(out, DX.hdr[2], T.cmax[2]) : e4_words_of(out, DN.hdr[2], T.cmin[2]);
-        if (top[r].len > 1) e5_or_bit(tw0, top[r].pos[0]);
-        if (top[r].len > 2) e5_or_bit(tw1, top[r].pos[1]);
-        if (top[r].len > 3) e5_or_bit(tw2, top[r].pos[2]);
+        if (top[r].len > 1) e5_or_bit(mx ? xw0 : nw0, top[r].pos0);
+        if (__any_sync(0xffffffffu, top[r].len > 2)) e5_top_long(false, out, top[r], mx ? 2 : 6, item_hdr, item_cnt, item_at);
       }
-      if (tid == TT - 1) {
-        if (in0) {
-          e5_or_bits(nm_words, 0, 0x10u | in1m, 5);
-          if (!as_snapshot) {
-            u32 accE = 0; int nE = 0;
-#pragma unroll
-            for (int k = 0; k < 4; k++) {
-              if (!((in1m >> (3 - k)) & 1u)) { accE = (accE << 1) | ((!e4_unif<FULL>(n1max[k], n1min[k]) && ((n1flags >> k) & 1u)) ? 1u : 0u); nE++; }
-            }
-            e5_or_bits(eq_words, 0, accE, nE);
-          }
-        } else if (!as_snapshot && !u0 && eq0) {
-          e5_or_bit(eq_words, 0);
+      // ... their nodemap and `equal` bits; a level-1 node's `equal` bit comes after those of the non-internal ones before it
+      if (warp == NW - 1) {
+        if (lane == 0) {
+          if (in0) e5_or_bits(nm_words, 0, 0x10u | in1m, 5);
+          else if (!as_snapshot && !u0 && eq0) e5_or_bit(eq_words, 0);
+        } else if (is1 && in0 && !as_snapshot && !n1un && n1eq) {
+          e5_or_bit(eq_words, (u32)(lane - 1 - __popc(in1m >> (5 - lane))));
         }
       }
     }
@@ -990,14 +1002,9 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
 #pragma unroll
       for (int r = 0; r < NTOP; r++) {  // root and level-1 entries (any length): the same lanes as in phase A
         const bool mx = NW == 2 ? warp == 0 : r == 0;
-        u8* const tb0 = mx ? xb0 : nb0;
-        u8* const tb1 = mx ? xb1 : nb1;
-        u8* const tb2 = out + (mx ? DX.bytes[2] : DN.bytes[2]);
-        u8* const tb3 = out + (mx ? DX.bytes[3] : DN.bytes[3]);
-        if (top[r].len > 0) tb0[top[r].pos[0]] = (u8)top[r].z;
-        if (top[r].len > 1) tb1[top[r].pos[1]] = (u8)(top[r].z >> 8);
-        if (top[r].len > 2) tb2[top[r].pos[2]] = (u8)(top[r].z >> 16);
-        if (top[r].len > 3) tb3[top[r].pos[3]] = (u8)(top[r].z >> 24);
+        if (top[r].len > 0) (mx ? xb0 : nb0)[top[r].pos0] = (u8)top[r].z;
+        if (top[r].len > 1) (mx ? xb1 : nb1)[top[r].pos1] = (u8)(top[r].z >> 8);
+        if (__any_sync(0xffffffffu, top[r].len > 2)) e5_top_long(true, out, top[r], mx ? 2 : 6, item_hdr, item_cnt, item_at);
       }
       if ((NW == 1 || warp == 1) && lane >= 16) {  // structure header (snapshot.rs:48-52 / log.rs:53-58): k, shape, sidelen; DAC level counts
         const u32 i = lane - 16u;
@@ -1005,9 +1012,9 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
           const u32 word = i < 5u ? (u32)unit.rows : i < 9u ? (u32)unit.cols : 64u;
           out[i] = i == 0 ? (u8)2 : (u8)(word >> (8u * ((12u - i) & 3u)));
         } else if (i == 13u) {
-          out[DX.hdr[0] - 1] = (u8)DX.levels;
+          out[x_hdr0 - 1] = (u8)x_levels;
         } else if (i == 14u) {
-          out[DN.hdr[0] - 1] = (u8)DN.levels;
+          out[n_hdr0 - 1] = (u8)n_levels;
         }
       }
     }
@@ -1019,21 +1026,12 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
       // ================= bitmap headers and rank directories: index[b] = ones in bits [0, 128(b+1))  (bitmap.rs:97-104)
       // bitmaps in stream order: nodemap, equal (Logs), the levels of the max DAC, the levels of the min DAC
       const u32 n_fix = as_snapshot ? 1u : 2u;
-      const u32 n_bm = n_fix + (u32)DX.levels + (u32)DN.levels;
+      const u32 n_bm = n_fix + x_levels + n_levels;
 #pragma unroll 1
       for (u32 i = warp; i < n_bm; i += NW) {
-        u32 hdr, len;
-        if (i == 0) { hdr = nm_hdr; len = nm_len; }
-        else if (i < n_fix) { hdr = eq_hdr; len = eq_len; }
-        else if (i < n_fix + (u32)DX.levels) {
-          const u32 j = i - n_fix;
-          hdr = j == 0 ? DX.hdr[0] : j == 1 ? DX.hdr[1] : j == 2 ? DX.hdr[2] : DX.hdr[3];
-          len = j == 0 ? T.cmax[0] : j == 1 ? T.cmax[1] : j == 2 ? T.cmax[2] : T.cmax[3];
-        } else {
-          const u32 j = i - n_fix - (u32)DX.levels;
-          hdr = j == 0 ? DN.hdr[0] : j == 1 ? DN.hdr[1] : j == 2 ? DN.hdr[2] : DN.hdr[3];
-          len = j == 0 ? T.cmin[0] : j == 1 ? T.cmin[1] : j == 2 ? T.cmin[2] : T.cmin[3];
-        }
+        // the lane that holds bitmap i: nodemap, `equal`, then the max DAC's levels from lane 2, the min DAC's from lane 6
+        const int src = (int)(i < n_fix ? i : i < n_fix + x_levels ? 2u + (i - n_fix) : 6u + (i - n_fix - x_levels));
+        const u32 hdr = shfl(item_hdr, src), len = shfl(item_cnt, src);
         if (lane == 0) {
           store_be32(out + hdr, len);
           store_be32(out + hdr + 4, 4u);  // k = 4 (bitmap.rs:69)
