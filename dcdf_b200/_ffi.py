@@ -17,7 +17,7 @@ ERR_NAMES = {0: "OK", 1: "NONFINITE", 2: "PRECISION_LOSS", 3: "OVERFLOW", 4: "BA
 ENC_I32, ENC_I64, ENC_F32, ENC_F64 = 4, 8, 32, 64
 MEM_HOST, MEM_DEVICE = 0, 1
 REF_ELIDED, REF_LOCAL, REF_EXTERNAL = 0, 1, 2
-KT_ENCODE, KT_STATS, KT_GATHER, KT_WINDOW, KT_CELL, KT_SEARCH, KT_REDUCE = range(7)
+KT_ENCODE, KT_STATS, KT_GATHER, KT_WINDOW, KT_CELL, KT_SEARCH, KT_REDUCE, KT_TIME_STATS = range(8)
 
 
 class Array3(C.Structure):
@@ -111,6 +111,7 @@ def _declare(lib):
         "dcdf_superchunk_window": (i32, [vp, vp, _P(Cube), vp, i32, i32]),
         "dcdf_superchunk_window_batch": (i32, [vp, vp, u64, vp, vp, vp, i32, i32]),
         "dcdf_superchunk_window_stats": (i32, [vp, vp, u64, vp, vp, vp, vp, vp, vp, vp, i32]),
+        "dcdf_superchunk_time_stats": (i32, [vp, vp, u64, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32]),
         "dcdf_superchunk_search_batch": (i32, [vp, vp, u64, vp, vp, vp, vp, vp, u64, _P(u64), i32]),
         "dcdf_superchunk_search_values": (i32, [vp, vp, u64, vp, vp, vp, vp, vp, u64, _P(u64), i32]),
         "dcdf_superchunk_save": (i32, [vp, vp, u32, _P(vp)]),

@@ -5,6 +5,7 @@ Names and argument meaning follow the reference (paths relative to dcdf/src):
   Superchunk.build / get / fill_cell / fill_window / search                          superchunk.rs:88-585
   Superchunk.search_values (float bounds; mmarray.rs:407-417 is todo!() upstream)
   Superchunk.window_stats (per-instant count / min / max / sum / sum_sq of windows; no reference counterpart)
+  Superchunk.time_stats (per-cell count / n_band / min / max / sum / sum_sq over time; no reference counterpart)
   MMArray3.{shape,get,cell,window,search}                                            mmarray.rs:135-536,
                                                                 py-dcdf/src/lib.rs:411-581 (PyMMArray3*)
   to_fixed / from_fixed / suggest_fraction                                           fixed.rs:31-159
@@ -176,6 +177,15 @@ class Context:
 def stats_dtype(dtype):
     """Record of Superchunk.window_stats_batch / Variable.window_stats for an array of `dtype`."""
     return np.dtype([("count", np.uint64), ("min", dtype), ("max", dtype), ("sum", np.float64), ("sum_sq", np.float64)])
+
+
+def time_stats_dtype(dtype):
+    """Record of Superchunk.time_stats_batch / Variable.time_stats for an array of `dtype`."""
+    return np.dtype([("count", np.uint64), ("n_band", np.uint64), ("min", dtype), ("max", dtype), ("sum", np.float64),
+                     ("sum_sq", np.float64)])
+
+
+_TIME_FIELDS = ("count", "n_band", "min", "max", "sum", "sum_sq")
 
 
 def _out_array(shape, enc, raw):
@@ -485,6 +495,38 @@ class Superchunk(_Queryable):
 
     def window_stats(self, start, end, top, bottom, left, right):
         return self.window_stats_batch([[start, end, top, bottom, left, right]])[0]
+
+    def _time_stats_into(self, cubes, lower, upper, cols, off, accumulate):
+        """dcdf_superchunk_time_stats into the column arrays `cols` (one per field of time_stats_dtype)."""
+        band = lower is not None or upper is not None
+        lo = hi = None
+        if band:
+            lo = np.ascontiguousarray(np.broadcast_to(np.asarray(-np.inf if lower is None else lower, np.float64), len(cubes)))
+            hi = np.ascontiguousarray(np.broadcast_to(np.asarray(np.inf if upper is None else upper, np.float64), len(cubes)))
+        p = lambda a: None if a is None else _ptr(a)
+        self.ctx.check(self.ctx._lib.dcdf_superchunk_time_stats(self.ctx._h, self._h, len(cubes), _ptr(cubes), _ptr(off), p(lo), p(hi),
+                                                                *[p(cols[f]) for f in _TIME_FIELDS], int(accumulate), MEM_HOST))
+
+    def time_stats_batch(self, cubes, lower=None, upper=None):
+        """Per-cell statistics over time of n windows reduced on the device (dcdf_superchunk_time_stats) -> (records, off):
+        window i's records are records[off[i]:off[i + 1]], one per cell, row-major.  Fields: count (non-NaN instants),
+        n_band (instants with lower <= value <= upper; bounds are scalars or one per window, a missing one is infinite;
+        without bounds n_band equals count), min / max (the superchunk's dtype; NaN / 0 when count is 0), sum and sum_sq
+        (float64, summed per time slice in time order, then over the slices)."""
+        cubes = np.ascontiguousarray(cubes, dtype=np.int64).reshape(-1, 6)
+        off = np.zeros(len(cubes) + 1, np.uint64)
+        np.cumsum((np.abs(cubes[:, 3] - cubes[:, 2]) * np.abs(cubes[:, 5] - cubes[:, 4])).astype(np.uint64), out=off[1:])
+        records = np.empty(int(off[-1]), time_stats_dtype(_DTYPE_OF_ENC[self.encoding]))
+        cols = {f: np.empty(len(records), records.dtype[f]) for f in _TIME_FIELDS}
+        self._time_stats_into(cubes, lower, upper, cols, off, False)
+        for f in _TIME_FIELDS:
+            records[f] = cols[f]
+        return records, off
+
+    def time_stats(self, start, end, top, bottom, left, right, lower=None, upper=None):
+        """Single-window time_stats_batch: records shaped (rows, cols)."""
+        rec, _ = self.time_stats_batch([[start, end, top, bottom, left, right]], lower, upper)
+        return rec.reshape(abs(bottom - top), abs(right - left))
 
     def search_batch(self, cubes, lower, upper, want_cells=True):
         return self._search(self.ctx._lib.dcdf_superchunk_search_batch, np.int64, cubes, lower, upper, want_cells)

@@ -662,6 +662,178 @@ void do_window_stats(dcdf_ctx* ctx, MetaBlock* mb, uint64_t n, const dcdf_cube* 
   tcollect(ctx, KT_REDUCE);
 }
 
+// Per-cell statistics over time of n windows (dcdf_superchunk_time_stats).  The slices the windows touch are cut into
+// groups whose partials (one TimePartial per (window, slice, cell)) fit the "time_stats_scratch" budget, at least one
+// slice per group.  Per group, every window is clipped to the group's instants, k_window_tiles4<V, TimeStatsOut<V>> runs
+// the group's jobs and k_time_stats_combine continues the records with the group's pieces in slice order; so the records
+// do not depend on the grouping.  Subchunks larger than 64x64 are refused as in do_window_stats.
+void do_time_stats(dcdf_ctx* ctx, MetaBlock* mb, uint64_t n, const dcdf_cube* bounds, const uint64_t* out_off, const double* lower,
+                   const double* upper, uint64_t* count, uint64_t* n_band, void* vmin, void* vmax, double* sum, double* sum_sq,
+                   int32_t accumulate, int32_t mem) {
+  ctx->last_time_groups = 0;
+  ctx->last_time_scratch = 0;
+  if (n == 0) return;
+  if (!bounds || !out_off || !count || !vmin || !vmax || !sum || !sum_sq) api_fail(DCDF_ERR_BAD_ARG, "null time statistics argument");
+  if (!lower != !upper) api_fail(DCDF_ERR_BAD_ARG, "lower and upper must both be given or both be NULL");
+  const bool band = lower != nullptr;
+  if (band && !n_band) api_fail(DCDF_ERR_BAD_ARG, "a band needs n_band");
+  if (mem != DCDF_MEM_HOST && mem != DCDF_MEM_DEVICE) api_fail(DCDF_ERR_BAD_ARG, "mem must be DCDF_MEM_HOST or DCDF_MEM_DEVICE");
+  if (mb->max_sidelen > 64) api_fail(DCDF_ERR_BAD_ARG, "time statistics need subchunks of at most 64x64");
+  std::vector<CubeDev> cubes(n);
+  std::vector<double> bnd(band ? 2 * n : 0);
+  const i64 csz = mb->Q.chunk_size, T = mb->Q.shape[0];
+  const i64 n_sl = (T + csz - 1) / csz;
+  std::vector<u64> cost(n_sl + 1, 0);  // cells of the windows that cover each slice (a difference array first)
+  for (uint64_t i = 0; i < n; i++) {
+    const dcdf_cube c = order_cube(bounds[i]);
+    check_cube(c, mb->Q.shape);
+    cubes[i] = {c.start, c.end, c.top, c.bottom, c.left, c.right};
+    const u64 area = (u64)((c.bottom - c.top) * (c.right - c.left));
+    if (out_off[i + 1] < out_off[i] || area != out_off[i + 1] - out_off[i]) api_fail(DCDF_ERR_BAD_ARG, "out_off does not match the windows' areas");
+    if (band) {
+      double lo = lower[i], hi = upper[i];
+      if (std::isnan(lo) || std::isnan(hi)) api_fail(DCDF_ERR_BAD_ARG, "NaN band bound in window %llu", (unsigned long long)i);
+      if (lo > hi) std::swap(lo, hi);
+      bnd[2 * i] = lo; bnd[2 * i + 1] = hi;
+    }
+    if (area && c.end > c.start) {
+      cost[c.start / csz] += area;
+      cost[(c.end - 1) / csz + 1] -= area;
+    }
+  }
+  for (i64 s = 1; s <= n_sl; s++) cost[s] += cost[s - 1];
+  // groups of slices [g_lo, g_hi): greedy in slice order under the budget; slices no window covers are skipped
+  const u64 budget = ctx->opt.time_stats_scratch;
+  std::vector<std::pair<i64, i64>> groups;
+  u64 g_bytes = 0, max_bytes = 0;
+  for (i64 s = 0; s < n_sl; s++) {
+    const u64 b = cost[s] * sizeof(TimePartial);
+    if (!b) continue;
+    if (groups.empty() || g_bytes + b > budget) {
+      groups.push_back({s, s + 1});
+      g_bytes = 0;
+    }
+    groups.back().second = s + 1;
+    g_bytes += b;
+    max_bytes = std::max(max_bytes, g_bytes);
+  }
+  const u64 rec0 = out_off[0], rec1 = out_off[n], n_rec = rec1 - rec0;
+  const bool no_slices = groups.empty();
+  if (no_slices) {
+    if (accumulate || !n_rec) return;  // nothing to continue / no records
+    groups.push_back({0, 0});          // zero-instant windows: the combine writes empty records
+  }
+  const size_t n_g = groups.size();
+  // every group's clipped windows, job and partial offsets, uploaded before the timed kernels
+  std::vector<CubeDev> gcubes(n_g * n);
+  std::vector<u64> job_base(n_g * (n + 1)), part_base(n_g * n), n_jobs(n_g);
+  for (size_t g = 0; g < n_g; g++) {
+    const i64 t_lo = groups[g].first * csz, t_hi = std::min(groups[g].second * csz, T);
+    CubeDev* gc = gcubes.data() + g * n;
+    u64 np = 0;
+    for (uint64_t i = 0; i < n; i++) {
+      gc[i] = cubes[i];
+      gc[i].start = std::min(std::max(cubes[i].start, t_lo), t_hi);
+      gc[i].end = std::max(std::min(cubes[i].end, t_hi), gc[i].start);
+      part_base[g * n + i] = np;
+      if (gc[i].end > gc[i].start)
+        np += (u64)((gc[i].bottom - gc[i].top) * (gc[i].right - gc[i].left)) * (u64)((gc[i].end - 1) / csz - gc[i].start / csz + 1);
+    }
+    std::vector<u64> jb;
+    n_jobs[g] = window_jobs(mb, std::vector<CubeDev>(gc, gc + n), jb);
+    std::copy(jb.begin(), jb.end(), job_base.begin() + g * (n + 1));
+  }
+  cudaStream_t st = ctx->stream;
+  const size_t b_cubes = sizeof(CubeDev) * n_g * n, b_off = sizeof(u64) * (n + 1);
+  ctx->query_in.reserve(b_cubes + b_off);
+  CubeDev* d_c = ctx->query_in.as<CubeDev>();
+  u64* d_off = reinterpret_cast<u64*>(d_c + n_g * n);
+  CK(cudaMemcpyAsync(d_c, gcubes.data(), b_cubes, cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(d_off, out_off, b_off, cudaMemcpyHostToDevice, st));
+  ctx->query_aux.reserve(sizeof(u64) * (job_base.size() + part_base.size()) + sizeof(double) * bnd.size());
+  u64* d_jb = ctx->query_aux.as<u64>();
+  u64* d_pb = d_jb + job_base.size();
+  double* d_band = reinterpret_cast<double*>(d_pb + part_base.size());
+  CK(cudaMemcpyAsync(d_jb, job_base.data(), sizeof(u64) * job_base.size(), cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(d_pb, part_base.data(), sizeof(u64) * part_base.size(), cudaMemcpyHostToDevice, st));
+  if (band) CK(cudaMemcpyAsync(d_band, bnd.data(), sizeof(double) * bnd.size(), cudaMemcpyHostToDevice, st));
+  ctx->query_aux2.reserve(std::max<u64>(max_bytes, 16));
+  // outputs from record rec0 on: the caller's device arrays, or one staging block for the six host arrays (loaded with
+  // the records to continue under accumulate)
+  const size_t es = enc_size(mb->Q.encoding);
+  u64* o_count = count + rec0;
+  u64* o_band = n_band ? n_band + rec0 : nullptr;
+  void* o_min = static_cast<u8*>(vmin) + es * rec0;
+  void* o_max = static_cast<u8*>(vmax) + es * rec0;
+  double* o_sum = sum + rec0;
+  double* o_sq = sum_sq + rec0;
+  if (mem == DCDF_MEM_HOST) {
+    const size_t a8 = (sizeof(u64) * n_rec + 15) & ~size_t(15), ae = (es * n_rec + 15) & ~size_t(15);
+    ctx->query_out.reserve(4 * a8 + 2 * ae);
+    u8* b = ctx->query_out.as<u8>();
+    u64* s_count = reinterpret_cast<u64*>(b);
+    u64* s_band = reinterpret_cast<u64*>(b + a8);
+    void* s_min = b + 2 * a8;
+    void* s_max = b + 2 * a8 + ae;
+    double* s_sum = reinterpret_cast<double*>(b + 2 * a8 + 2 * ae);
+    double* s_sq = reinterpret_cast<double*>(b + 3 * a8 + 2 * ae);
+    if (accumulate && n_rec) {
+      CK(cudaMemcpyAsync(s_count, o_count, sizeof(u64) * n_rec, cudaMemcpyHostToDevice, st));
+      if (o_band) CK(cudaMemcpyAsync(s_band, o_band, sizeof(u64) * n_rec, cudaMemcpyHostToDevice, st));
+      CK(cudaMemcpyAsync(s_min, o_min, es * n_rec, cudaMemcpyHostToDevice, st));
+      CK(cudaMemcpyAsync(s_max, o_max, es * n_rec, cudaMemcpyHostToDevice, st));
+      CK(cudaMemcpyAsync(s_sum, o_sum, sizeof(double) * n_rec, cudaMemcpyHostToDevice, st));
+      CK(cudaMemcpyAsync(s_sq, o_sq, sizeof(double) * n_rec, cudaMemcpyHostToDevice, st));
+    }
+    o_count = s_count; o_band = o_band ? s_band : nullptr; o_min = s_min; o_max = s_max; o_sum = s_sum; o_sq = s_sq;
+  }
+  TileWindowParams TP;
+  TP.Q = mb->Q; TP.out_off = d_off; TP.n_queries = n; TP.out = nullptr; TP.raw = 0;
+  TP.part = nullptr; TP.tpart = ctx->query_aux2.as<TimePartial>(); TP.band = band ? d_band : nullptr;
+  TimeCombineParams CP;
+  CP.out_off = d_off; CP.part = TP.tpart; CP.n_queries = n; CP.rec0 = rec0; CP.rec1 = rec1; CP.chunk_size = csz;
+  CP.encoding = mb->Q.encoding;
+  CP.count = o_count; CP.n_band = o_band; CP.vmin = o_min; CP.vmax = o_max; CP.sum = o_sum; CP.sum_sq = o_sq;
+  const bool narrow = mb->max_dac_levels <= 3 && !ctx->opt.window_wide;
+  const int smem32 = (int)(sizeof(Tile4Smem<int32_t>) + sizeof(TimeStatsShared<int32_t>));
+  const int smem64 = (int)(sizeof(Tile4Smem<i64>) + sizeof(TimeStatsShared<i64>));
+  if (narrow) CK(cudaFuncSetAttribute(k_window_tiles4<int32_t, TimeStatsOut<int32_t>>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem32));
+  else CK(cudaFuncSetAttribute(k_window_tiles4<i64, TimeStatsOut<i64>>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem64));
+  tbegin(ctx, KT_TIME_STATS);
+  for (size_t g = 0; g < n_g; g++) {
+    TP.cubes = CP.cubes = d_c + g * n;
+    TP.job_base = d_jb + g * (n + 1);
+    TP.part_base = CP.part_base = d_pb + g * n;
+    TP.n_jobs = n_jobs[g];
+    if (n_jobs[g]) {
+      const unsigned grid = (unsigned)std::min<u64>(n_jobs[g], (u64)ctx->sm_count * 64);
+      if (narrow) k_window_tiles4<int32_t, TimeStatsOut<int32_t>><<<grid, DT_THREADS, smem32, st>>>(TP);
+      else k_window_tiles4<i64, TimeStatsOut<i64>><<<grid, DT_THREADS, smem64, st>>>(TP);
+      CK(cudaGetLastError());
+      ctx->launches++;
+    }
+    if (n_rec) {
+      CP.init = g == 0 && !accumulate;
+      k_time_stats_combine<<<(unsigned)((n_rec + 255) / 256), 256, 0, st>>>(CP);
+      CK(cudaGetLastError());
+      ctx->launches++;
+    }
+  }
+  tend(ctx, KT_TIME_STATS);
+  if (mem == DCDF_MEM_HOST && n_rec) {
+    CK(cudaMemcpyAsync(count + rec0, o_count, sizeof(u64) * n_rec, cudaMemcpyDeviceToHost, st));
+    if (o_band) CK(cudaMemcpyAsync(n_band + rec0, o_band, sizeof(u64) * n_rec, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(static_cast<u8*>(vmin) + es * rec0, o_min, es * n_rec, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(static_cast<u8*>(vmax) + es * rec0, o_max, es * n_rec, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(sum + rec0, o_sum, sizeof(double) * n_rec, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(sum_sq + rec0, o_sq, sizeof(double) * n_rec, cudaMemcpyDeviceToHost, st));
+  }
+  CK(cudaStreamSynchronize(st));
+  tcollect(ctx, KT_TIME_STATS);
+  ctx->last_time_groups = no_slices ? 0 : n_g;
+  ctx->last_time_scratch = max_bytes;
+}
+
 // Fixed-point bounds (lower / upper), or, with strict, value bounds (vlower / vupper) that the kernels convert per subchunk
 // with its own fractional bits, with the exact hit set (the strict kernels: k_search_tiles4 / k_count_tiles4 / k_search
 // with ST = true).
@@ -1024,6 +1196,16 @@ int32_t dcdf_superchunk_window_stats(dcdf_ctx* ctx, const dcdf_superchunk* sc, u
   return guarded(ctx, [&] {
     if (!sc) api_fail(DCDF_ERR_BAD_ARG, "null superchunk");
     do_window_stats(ctx, super_meta(ctx, sc), n, bounds, out_off, count, vmin, vmax, sum, sum_sq, mem);
+  });
+}
+
+int32_t dcdf_superchunk_time_stats(dcdf_ctx* ctx, const dcdf_superchunk* sc, uint64_t n, const dcdf_cube* bounds,
+                                   const uint64_t* out_off, const double* lower, const double* upper, uint64_t* count,
+                                   uint64_t* n_band, void* vmin, void* vmax, double* sum, double* sum_sq, int32_t accumulate,
+                                   int32_t mem) {
+  return guarded(ctx, [&] {
+    if (!sc) api_fail(DCDF_ERR_BAD_ARG, "null superchunk");
+    do_time_stats(ctx, super_meta(ctx, sc), n, bounds, out_off, lower, upper, count, n_band, vmin, vmax, sum, sum_sq, accumulate, mem);
   });
 }
 

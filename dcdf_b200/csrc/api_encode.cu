@@ -912,6 +912,7 @@ int32_t dcdf_ctx_set_option(dcdf_ctx* ctx, const char* name, int64_t value) {
   else if (n == "search_dfs") ctx->opt.search_dfs = value != 0;
   else if (n == "search_no_cache") ctx->opt.search_no_cache = value != 0;
   else if (n == "trace") ctx->opt.trace = value != 0;
+  else if (n == "time_stats_scratch") ctx->opt.time_stats_scratch = value <= 0 ? 1ull << 30 : (uint64_t)value;
   else {
     ctx->last_error = "unknown option " + n;
     return DCDF_ERR_BAD_ARG;
@@ -928,6 +929,8 @@ int32_t dcdf_ctx_get_stat(const dcdf_ctx* ctx, const char* name, int64_t* value)
   else if (n == "encode_units_general") *value = (int64_t)c[0] + c[1] + c[2] + c[3] + c[4];
   else if (n == "encode_units_wide") *value = (int64_t)c[2] + c[3];
   else if (n == "encode_units_clipped") *value = (int64_t)c[1] + c[3] + c[4] + c[6] + c[7];
+  else if (n == "time_stats_groups") *value = (int64_t)ctx->last_time_groups;
+  else if (n == "time_stats_scratch_bytes") *value = (int64_t)ctx->last_time_scratch;
   else return DCDF_ERR_BAD_ARG;
   return DCDF_OK;
 }

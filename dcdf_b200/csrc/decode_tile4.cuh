@@ -289,11 +289,16 @@ DCDF_DEVINL bool staged4(const u8* chunk, const InstDir& d, u32& delta) {
   return d.size + mis + 4u <= (u32)Tile4Smem<V>::BUF + 32u;
 }
 
-// One CTA per (window, time slice, subchunk) job.  OUT receives the cells: QuadOut writes the window, StatsOut<V> reduces
-// it per instant (dcdf_superchunk_window_stats); its hooks (begin / elided / instant_begin / instant_end / end) are all
-// that differs between the two.
+// CTAs per SM k_window_tiles4 is built for: TimeStatsOut's accumulators take most of an SM's shared memory, so it gets one
+// CTA and the registers of the whole SM.
 template <typename V, typename OUT>
-__global__ void __launch_bounds__(DT_THREADS, sizeof(V) == 4 ? 4 : 2) k_window_tiles4(const TileWindowParams P) {
+constexpr int tiles4_min_blocks() { return std::is_same<OUT, TimeStatsOut<V>>::value ? 1 : sizeof(V) == 4 ? 4 : 2; }
+
+// One CTA per (window, time slice, subchunk) job.  OUT receives the cells: QuadOut writes the window, StatsOut<V> reduces
+// it per instant (dcdf_superchunk_window_stats), TimeStatsOut<V> per cell over the job's instants
+// (dcdf_superchunk_time_stats); their hooks (begin / elided / instant_begin / instant_end / end) are all that differs.
+template <typename V, typename OUT>
+__global__ void __launch_bounds__(DT_THREADS, (tiles4_min_blocks<V, OUT>())) k_window_tiles4(const TileWindowParams P) {
   extern __shared__ __align__(16) unsigned char dt4_smem_raw[];
   Tile4Smem<V>& S = *reinterpret_cast<Tile4Smem<V>*>(dt4_smem_raw);
   const QuerySet& Q = P.Q;
@@ -454,6 +459,81 @@ __global__ void k_window_stats_combine(const StatsCombineParams P) {
   else if (P.encoding == 64) stats_fold<double>(P, r, p, nsub, T_all);
   else if (P.encoding == 4) stats_fold<int32_t>(P, r, p, nsub, T_all);
   else stats_fold<i64>(P, r, p, nsub, T_all);
+}
+
+// Time statistics, second pass: one thread per (window, cell) record folds the record's partials of this scratch group in
+// slice order into the outputs -- starting from empty records (init) or continuing the ones there.  A fixed order, so a
+// record does not depend on the batch around it nor on how the slices were grouped.
+struct TimeCombineParams {
+  const CubeDev* cubes;   // the windows with their instants clipped to the group
+  const u64* out_off;     // [n + 1] record offsets
+  const u64* part_base;   // [n]
+  const TimePartial* part;
+  u64 n_queries, rec0, rec1;  // records [rec0, rec1) = [out_off[0], out_off[n]); record g is written at index g - rec0
+  i64 chunk_size;
+  int encoding, init;
+  u64* count;
+  u64* n_band;            // may be nullptr
+  void* vmin;
+  void* vmax;
+  double* sum;
+  double* sum_sq;
+};
+template <typename T>
+DCDF_DEVINL T time_value(TimeVal v) {
+  if constexpr (std::is_integral<T>::value) return (T)v.i;
+  else return (T)v.f;
+}
+template <typename T>
+DCDF_DEVINL void time_fold(const TimeCombineParams& P, u64 r, const TimePartial* p, u64 nsl, u64 area) {
+  u64 n = 0, nb = 0;
+  T mn = 0, mx = 0;
+  double sum = 0.0, sq = 0.0;
+  if (!P.init) {
+    n = P.count[r];
+    nb = P.n_band ? P.n_band[r] : 0u;
+    mn = static_cast<const T*>(P.vmin)[r];
+    mx = static_cast<const T*>(P.vmax)[r];
+    sum = P.sum[r];
+    sq = P.sum_sq[r];
+  }
+  for (u64 k = 0; k < nsl; k++) {
+    const TimePartial x = p[k * area];
+    if (x.count) {
+      const T a = time_value<T>(x.min), b = time_value<T>(x.max);
+      mn = n == 0 || a < mn ? a : mn;
+      mx = n == 0 || b > mx ? b : mx;
+    }
+    n += x.count;
+    nb += x.n_band;
+    sum = __dadd_rn(sum, x.sum);
+    sq = __dadd_rn(sq, x.sum_sq);
+  }
+  if (n == 0) mn = mx = stats_value<T>(0, 0);  // NaN for floats (code 0), 0 for integers
+  P.count[r] = n;
+  if (P.n_band) P.n_band[r] = nb;
+  static_cast<T*>(P.vmin)[r] = mn;
+  static_cast<T*>(P.vmax)[r] = mx;
+  P.sum[r] = sum;
+  P.sum_sq[r] = sq;
+}
+__global__ void k_time_stats_combine(const TimeCombineParams P) {
+  const u64 g = P.rec0 + (u64)blockIdx.x * blockDim.x + threadIdx.x;
+  if (g >= P.rec1) return;
+  u64 lo = 0, hi = P.n_queries;  // the window of record g: the last one whose records start at or before g
+  while (hi - lo > 1) {
+    const u64 mid = (lo + hi) >> 1;
+    if (P.out_off[mid] <= g) lo = mid; else hi = mid;
+  }
+  const CubeDev c = P.cubes[lo];
+  const u64 area = (u64)((c.bottom - c.top) * (c.right - c.left));
+  const u64 nsl = c.end > c.start ? (u64)((c.end - 1) / P.chunk_size - c.start / P.chunk_size + 1) : 0u;
+  const TimePartial* p = P.part + P.part_base[lo] + (g - P.out_off[lo]);
+  const u64 r = g - P.rec0;
+  if (P.encoding == 32) time_fold<float>(P, r, p, nsl, area);
+  else if (P.encoding == 64) time_fold<double>(P, r, p, nsl, area);
+  else if (P.encoding == 4) time_fold<int32_t>(P, r, p, nsl, area);
+  else time_fold<i64>(P, r, p, nsl, area);
 }
 
 // ---------------------------------------------------------------------------------------------------------------

@@ -55,6 +55,21 @@ struct StatsPartial {
 };
 static_assert(sizeof(StatsPartial) == 40, "StatsPartial is 40 bytes");
 
+// Per-cell statistics over time (dcdf_superchunk_time_stats): the reduction of one cell over one piece -- the window's
+// instants inside one time slice.  min / max are values of the encoding (f for f32 / f64, i for i32 / i64; subchunk bits
+// differ per slice, so codes could not be compared later); sum / sum_sq are ((0 + v_0) + v_1) + ... in double, in time
+// order.  count == 0: min / max are meaningless, the sums 0.
+union TimeVal {
+  i64 i;
+  double f;
+};
+struct TimePartial {
+  u32 count, n_band;
+  TimeVal min, max;
+  double sum, sum_sq;
+};
+static_assert(sizeof(TimePartial) == 40, "TimePartial is 40 bytes");
+
 struct TileWindowParams {
   QuerySet Q;
   const CubeDev* cubes;   // validated, ordered
@@ -66,6 +81,10 @@ struct TileWindowParams {
   // window statistics: partial of (window q, subchunk sub, instant t) at part[part_base[q] + sub * (end - start) + t - start]
   const u64* part_base;
   StatsPartial* part;
+  // time statistics: partial of (window q, k-th slice of the window, cell) at tpart[part_base[q] + k * area + cell], cells
+  // row-major; band[2q], band[2q + 1]: the window's ordered band (nullptr: no band)
+  TimePartial* tpart;
+  const double* band;
 };
 
 // One job of k_window_tiles4: window q, one time slice [t_lo, t_hi), the subchunk `sub` (row-major among those the window
@@ -556,6 +575,159 @@ struct StatsOut {
   DCDF_DEVINL void end(u32 n_t) const {
     __syncthreads();
     flush(n_t - 1u);
+  }
+};
+
+// Per-cell statistics over time through the tile decoder (k_window_tiles4<V, TimeStatsOut<V>>).  A thread owns its 4x4
+// block for the whole job, so it folds every instant of its cells into their accumulators in shared memory with no
+// barrier and no atomics; after the last instant the CTA writes one TimePartial per cell of the clipped rectangle,
+// row-major (coalesced).  Cell k = 4 * quad + cell of block p sits at index k * DT_THREADS + p (a warp's accesses are
+// consecutive).  The counters are 16 bits wide: every TS_SPAN instants each thread adds its cells' counters to their
+// partials in global memory and restarts them, so a slice may hold any number of instants.
+constexpr int TS_CELLS = 16 * DT_THREADS;
+constexpr u32 TS_SPAN = 0xffffu;
+template <typename V>
+struct TimeStatsShared {
+  double sum[TS_CELLS], sq[TS_CELLS];
+  V mn[TS_CELLS], mx[TS_CELLS];  // codes at the subchunk's bits
+  uint16_t n[TS_CELLS], nb[TS_CELLS];
+};
+DCDF_DEVINL u32 ts_index(int r, int c) {  // accumulator of tile cell (r, c)
+  const u32 k = 4u * (2u * (((u32)r >> 1) & 1u) + (((u32)c >> 1) & 1u)) + 2u * ((u32)r & 1u) + ((u32)c & 1u);
+  return k * DT_THREADS + morton_encode((u32)r >> 2, (u32)c >> 2);
+}
+// The value the window decoder writes for an i64 code, as a double (NaN: code 0 of a float encoding, tested apart).
+DCDF_DEVINL double ts_value(i64 v, int kind, int bits) {
+  return kind == 2 ? (double)from_fixed_dev<float>(v, bits) : kind == 3 ? from_fixed_dev<double>(v, bits) : __ll2double_rn(v);
+}
+template <typename V>
+struct TimeStatsOut {
+  static constexpr bool search_quirk = false;
+  static constexpr bool vec4 = false;
+  TimeStatsShared<V>* C;
+  TimePartial* rec;              // partial of tile cell (top, left); cell (r, c) at rec[(r - top) * pitch + c - left]
+  u32 pitch;                     // window columns
+  int top, bottom, left, right;  // window clipped to the tile, tile coordinates
+  int kind;                      // 0: integer encodings (the code is the value), 2: f32, 3: f64
+  int bits;
+  double lo, hi;                 // band (-inf, inf without one)
+  DCDF_DEVINL bool touches(int r0, int c0, int side) const { return r0 + side > top && r0 < bottom && c0 + side > left && c0 < right; }
+  DCDF_DEVINL bool inside(int r0, int c0, int side) const { return r0 >= top && r0 + side <= bottom && c0 >= left && c0 + side <= right; }
+  // the value QuadOut writes for the code (its cvt / CellOut::put), as a double
+  DCDF_DEVINL double value(V v) const {
+    if (kind == 2) return (double)((sizeof(V) == 4 ? __int2float_rn((int)v - 1) : __ll2float_rn((i64)v - 1)) * __int_as_float((126 - bits) << 23));
+    if (kind == 3) return (sizeof(V) == 4 ? __int2double_rn((int)v - 1) : __ll2double_rn((i64)v - 1)) * __longlong_as_double((long long)(1022 - bits) << 52);
+    return sizeof(V) == 4 ? (double)(int)v : __ll2double_rn((i64)v);
+  }
+  DCDF_DEVINL void add(u32 idx, V v) const {
+    if (kind != 0 && v == 0) return;  // NaN
+    const double x = value(v);
+    TimeStatsShared<V>& S = *C;
+    S.n[idx] = (uint16_t)(S.n[idx] + 1u);
+    if (x >= lo && x <= hi) S.nb[idx] = (uint16_t)(S.nb[idx] + 1u);
+    S.mn[idx] = min(S.mn[idx], v);
+    S.mx[idx] = max(S.mx[idx], v);
+    S.sum[idx] = __dadd_rn(S.sum[idx], x);
+    S.sq[idx] = __dadd_rn(S.sq[idx], __dmul_rn(x, x));
+  }
+  DCDF_DEVINL void put_pair(bool, int r0, int c0, const V (&a)[4], const V (&b)[4]) const {
+    // cells of this 2x4 strip inside the window: bits 0..3 = a, 4..7 = b (cell = 2 * (row & 1) + (col & 1))
+    const u32 rowm = ((r0 >= top && r0 < bottom) ? 0x33u : 0u) | ((r0 + 1 >= top && r0 + 1 < bottom) ? 0xccu : 0u);
+    const u32 colm = ((c0 >= left && c0 < right) ? 0x05u : 0u) | ((c0 + 1 >= left && c0 + 1 < right) ? 0x0au : 0u) |
+                     ((c0 + 2 >= left && c0 + 2 < right) ? 0x50u : 0u) | ((c0 + 3 >= left && c0 + 3 < right) ? 0xa0u : 0u);
+    const u32 in = rowm & colm;
+    if (!in) return;
+    const u32 ka = (4u * 2u * (((u32)r0 >> 1) & 1u)) * DT_THREADS + threadIdx.x;  // quad a: 2 * (row / 2 & 1), c0 % 4 == 0
+#pragma unroll
+    for (int i = 0; i < 4; i++) {
+      if ((in >> i) & 1u) add(ka + (u32)i * DT_THREADS, a[i]);
+      if ((in >> (4 + i)) & 1u) add(ka + (u32)(4 + i) * DT_THREADS, b[i]);
+    }
+  }
+  DCDF_DEVINL void put(int r0, int c0, const V (&v)[4]) const {  // trees of side 2: one quad at (0, 0)
+    put_pair(false, r0, c0, v, v);  // the second quad lies outside every rectangle of a 2x2 tile (right <= 2)
+  }
+  // k_window_tiles4's hooks
+  DCDF_DEVINL void begin(const TileWindowParams& P, const TileJob& J, int bits_, unsigned char* smem) {
+    C = reinterpret_cast<TimeStatsShared<V>*>(smem);
+    const i64 W_cols = J.c.right - J.c.left, area = (J.c.bottom - J.c.top) * W_cols;
+    const u64 k = (u64)(J.t_lo / P.Q.chunk_size - J.c.start / P.Q.chunk_size);
+    top = J.top; bottom = J.bottom; left = J.left; right = J.right;
+    pitch = (u32)W_cols;
+    rec = P.tpart + P.part_base[J.q] + k * (u64)area + (u64)((J.chunk_top + top - J.c.top) * W_cols + (J.chunk_left + left - J.c.left));
+    kind = P.Q.encoding == 32 ? 2 : P.Q.encoding == 64 ? 3 : 0;
+    bits = bits_;
+    lo = P.band ? P.band[2 * J.q] : -INFINITY;
+    hi = P.band ? P.band[2 * J.q + 1] : INFINITY;
+  }
+  DCDF_DEVINL TimeVal to_val(i64 code, int b) const {
+    TimeVal r;
+    if (kind) r.f = ts_value(code, kind, b); else r.i = code;
+    return r;
+  }
+  // Elided: every cell holds the node's table value at the node's bits (superchunk.rs:426-433); one partial, computed by
+  // every thread, written to each cell of the rectangle
+  DCDF_DEVINL void elided(const TileWindowParams& P, const TileJob& J, const SliceMeta& sm, const SlotDesc& sdsc) const {
+    TimePartial x;
+    x.count = 0; x.n_band = 0;
+    i64 mn = INT64_MAX, mx = INT64_MIN;
+    double s = 0.0, q = 0.0;
+    for (i64 t = J.t_lo; t < J.t_hi; t++) {
+      const i64 v = P.Q.tbl_max[sdsc.tbl0 + (u64)(t - sm.t0) * sdsc.stride];
+      if (kind != 0 && v == 0) continue;
+      const double f = ts_value(v, kind, sdsc.bits);
+      x.count++;
+      if (f >= lo && f <= hi) x.n_band++;
+      mn = min(mn, v); mx = max(mx, v);
+      s = __dadd_rn(s, f);
+      q = __dadd_rn(q, __dmul_rn(f, f));
+    }
+    x.min = to_val(mn, sdsc.bits); x.max = to_val(mx, sdsc.bits);
+    x.sum = s; x.sum_sq = q;
+    const int wc = right - left;
+    for (int i = threadIdx.x; i < (bottom - top) * wc; i += DT_THREADS) rec[(u64)(i / wc) * pitch + (u32)(i % wc)] = x;
+  }
+  // instant 0: the thread's own accumulators start (the previous job's end read them before a barrier this one passed)
+  DCDF_DEVINL void instant_begin(u32 i, u64) const {
+    if (i % TS_SPAN == 0) {
+      const u32 p = threadIdx.x;
+      const int R0 = 4 * (int)morton_row(p), C0 = 4 * (int)morton_col(p);
+      TimeStatsShared<V>& S = *C;
+#pragma unroll 1
+      for (u32 k = 0; k < 16u; k++) {
+        const u32 idx = k * DT_THREADS + p;
+        if (i > 0) {  // counters of the last TS_SPAN instants to the cell's partial
+          const int r = R0 + 2 * (int)(k >> 3) + (int)((k >> 1) & 1u), c = C0 + 2 * (int)((k >> 2) & 1u) + (int)(k & 1u);
+          if (r >= top && r < bottom && c >= left && c < right) {
+            TimePartial& g = rec[(u64)(r - top) * pitch + (u32)(c - left)];
+            g.count = (i == TS_SPAN ? 0u : g.count) + S.n[idx];
+            g.n_band = (i == TS_SPAN ? 0u : g.n_band) + S.nb[idx];
+          }
+        } else {
+          S.sum[idx] = 0.0; S.sq[idx] = 0.0;
+          S.mn[idx] = sizeof(V) == 4 ? (V)INT32_MAX : (V)INT64_MAX;
+          S.mx[idx] = sizeof(V) == 4 ? (V)INT32_MIN : (V)INT64_MIN;
+        }
+        S.n[idx] = 0; S.nb[idx] = 0;
+      }
+    }
+  }
+  DCDF_DEVINL void instant_end(u32) const {}
+  DCDF_DEVINL void end(u32 n_t) const {
+    __syncthreads();  // every block's accumulators are final (and the counters spilled by their owners are visible)
+    const TimeStatsShared<V>& S = *C;
+    const int wc = right - left;
+    for (int i = threadIdx.x; i < (bottom - top) * wc; i += DT_THREADS) {
+      const int r = top + i / wc, c = left + i % wc;
+      const u32 idx = ts_index(r, c);
+      TimePartial& g = rec[(u64)(r - top) * pitch + (u32)(c - left)];
+      TimePartial x;
+      x.count = (n_t > TS_SPAN ? g.count : 0u) + S.n[idx];
+      x.n_band = (n_t > TS_SPAN ? g.n_band : 0u) + S.nb[idx];
+      x.min = to_val((i64)S.mn[idx], bits); x.max = to_val((i64)S.mx[idx], bits);
+      x.sum = S.sum[idx]; x.sum_sq = S.sq[idx];
+      g = x;
+    }
   }
 };
 

@@ -95,7 +95,7 @@ inline void pool_free(void* p) {
   if (p) cudaFreeAsync(p, 0);  // callers have synchronized every stream that used p
 }
 
-enum { KT_ENCODE = 0, KT_STATS = 1, KT_GATHER = 2, KT_WINDOW = 3, KT_CELL = 4, KT_SEARCH = 5, KT_REDUCE = 6, KT_COUNT = 7 };
+enum { KT_ENCODE = 0, KT_STATS = 1, KT_GATHER = 2, KT_WINDOW = 3, KT_CELL = 4, KT_SEARCH = 5, KT_REDUCE = 6, KT_TIME_STATS = 7, KT_COUNT = 8 };
 
 }  // namespace dcdf
 
@@ -107,7 +107,7 @@ struct dcdf_ctx {
   cudaEvent_t fork_ev = nullptr, join_ev = nullptr;
   std::string last_error;
   uint64_t launches = 0;
-  float kernel_ms[dcdf::KT_COUNT] = {0, 0, 0, 0, 0, 0, 0};
+  float kernel_ms[dcdf::KT_COUNT] = {0, 0, 0, 0, 0, 0, 0, 0};
   cudaEvent_t ev[2 * dcdf::KT_COUNT] = {};
   int sm_count = 148;
   // dcdf_ctx_set_option (include/dcdf_cuda.h)
@@ -124,8 +124,10 @@ struct dcdf_ctx {
     int search_dfs = 0;                  // depth-first search kernel instead of the tile search
     int search_no_cache = 0;             // the search's writing pass recomputes instead of reading cached findings
     int trace = 0;                       // host-side phase times of the encode pipeline on stderr (adds stream syncs)
+    uint64_t time_stats_scratch = 1ull << 30;  // time statistics: partials per group of slices, in bytes (at least one slice per group)
   } opt;
   uint32_t last_list_counts[8] = {0, 0, 0, 0, 0, 0, 0, 0};  // units per encoder work list of the last build (dcdf_ctx_get_stat)
+  uint64_t last_time_groups = 0, last_time_scratch = 0;     // slice groups / partial bytes of the largest group, last time statistics call
   // scratch
   dcdf::DevBuf input_copy, units, ustats, istats, slices, sstate, tbl_scratch, order, pieces, results, stored, chunk_off,
       arena, small, exact, query_in, query_out, query_aux, query_aux2, search_cache, tree_buf;

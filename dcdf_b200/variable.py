@@ -10,6 +10,7 @@
   MMArray3.shape/get/cell/window   py-dcdf/src/lib.rs:497-538 (PyMMArray3F32), mmarray.rs:357-400
   search with float bounds         mmarray.rs:407-417 is todo!() upstream; dcdf_superchunk_search_values on the device
   window_stats                     per-instant count / min / max / sum / sum_sq of a window, dcdf_superchunk_window_stats
+  time_stats                       per-cell count / n_band / min / max / sum / sum_sq over time, dcdf_superchunk_time_stats
 
 The store is any mapping CID (bytes) -> stored node bytes.  The slices' superchunk CIDs are kept in the reference's span
 tree (dcdf_b200/span.py: stored Span nodes, `Variable.cid` = the root span, dataset.rs:880-987), so a variable written here
@@ -345,6 +346,37 @@ class Variable(MMArray3):
         self._check(start, stop, top, bottom, left, right)
         parts = [sc.window_stats(a, b, top, bottom, left, right) for sc, _, a, b in self._groups(start, stop)] if stop > start else []
         return np.concatenate(parts) if parts else np.empty(0, stats_dtype(self.dtype))
+
+    def time_stats(self, start, stop, top, bottom, left, right, lower=None, upper=None):
+        """Per-cell statistics over instants [start, stop) of a window, reduced on the device from the encoded bytes (one
+        dcdf_superchunk_time_stats call per span group, each continuing the records of the one before): records shaped
+        (rows, cols) with fields count (non-NaN instants), n_band (instants with lower <= value <= upper; equals count
+        without bounds), min, max (the variable's dtype; NaN for floats / 0 for integers when count is 0), sum and sum_sq
+        (float64).  For example, a climatology and the days above a threshold:
+
+            r = v.time_stats(0, 365, 100, 200, 300, 400, lower=30.0)
+            mean = r["sum"] / r["count"]
+            var = r["sum_sq"] / r["count"] - mean ** 2     # population variance
+            hot_days = r["n_band"]
+        """
+        from .api import _TIME_FIELDS, time_stats_dtype
+        self._check(start, stop, top, bottom, left, right)
+        rows, cols_ = bottom - top, right - left
+        rec = np.empty((rows, cols_), time_stats_dtype(self.dtype))
+        cols = {f: np.empty(rows * cols_, rec.dtype[f]) for f in _TIME_FIELDS}
+        cube = np.array([[start, start, top, bottom, left, right]], np.int64)
+        off = np.array([0, rows * cols_], np.uint64)
+        if stop > start and rec.size:
+            for k, (sc, _, a, b) in enumerate(self._groups(start, stop)):    # a group's handle may not outlive the next load
+                cube[0, 0], cube[0, 1] = a, b
+                sc._time_stats_into(cube, lower, upper, cols, off, k > 0)
+        else:                                        # zero instants: empty records
+            cols["count"][:] = cols["n_band"][:] = 0
+            cols["min"][:] = cols["max"][:] = np.nan if np.issubdtype(self.dtype, np.floating) else 0
+            cols["sum"][:] = cols["sum_sq"][:] = 0.0
+        for f in _TIME_FIELDS:
+            rec[f] = cols[f].reshape(rows, cols_)
+        return rec
 
     def close(self):
         self.cache.close()

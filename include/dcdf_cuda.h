@@ -100,11 +100,15 @@ int32_t dcdf_ctx_set_stream(dcdf_ctx* ctx, void* cuda_stream);
  *   "search_dfs" 0|1        depth-first search kernel instead of the tile search
  *   "search_no_cache" 0|1   search's writing pass recomputes instead of reading the counting pass's findings
  *   "trace" 0|1             host-side phase times of the encode pipeline on stderr
+ *   "time_stats_scratch" n  dcdf_superchunk_time_stats: bytes of partials per group of time slices (default 1 GiB,
+ *                           <= 0 restores it; a group holds at least one slice); results do not depend on it
  * Unknown names return DCDF_ERR_BAD_ARG. */
 int32_t dcdf_ctx_set_option(dcdf_ctx* ctx, const char* name, int64_t value);
 /* Counters of the last build call: "encode_units_fast" (units encoded by the fast-path kernels), "encode_units_edge" (the
  * part of those with at most 32 rows or columns in the raster, one warp per tile), "encode_units_general",
- * "encode_units_wide" (64-bit values), "encode_units_clipped". */
+ * "encode_units_wide" (64-bit values), "encode_units_clipped".  Of the last dcdf_superchunk_time_stats call:
+ * "time_stats_groups" (groups of time slices, each one pass of its two kernels) and "time_stats_scratch_bytes" (partial
+ * bytes of the largest group). */
 int32_t dcdf_ctx_get_stat(const dcdf_ctx* ctx, const char* name, int64_t* value);
 int32_t dcdf_ctx_synchronize(dcdf_ctx* ctx);
 const char* dcdf_last_error(const dcdf_ctx* ctx);
@@ -112,7 +116,8 @@ const char* dcdf_last_error(const dcdf_ctx* ctx);
 uint64_t dcdf_ctx_launch_count(const dcdf_ctx* ctx);
 /* CUDA-event time (ms) of the dominant kernel(s) of the last build / query call, measured on the
  * context's stream.  which: 0 = encode kernel, 1 = stats kernel, 2 = gather, 3 = window decode,
- * 4 = cell decode, 5 = search, 6 = window statistics (both of its kernels). */
+ * 4 = cell decode, 5 = search, 6 = window statistics (both of its kernels), 7 = time statistics (all kernels of
+ * the call, every group of slices). */
 int32_t dcdf_ctx_last_kernel_ms(const dcdf_ctx* ctx, int32_t which, float* ms);
 
 /* ------------------------------------------------------------------ a1 / a2 / a3 / a21 */
@@ -248,6 +253,35 @@ int32_t dcdf_superchunk_window_batch(dcdf_ctx* ctx, const dcdf_superchunk* sc, u
 int32_t dcdf_superchunk_window_stats(dcdf_ctx* ctx, const dcdf_superchunk* sc, uint64_t n, const dcdf_cube* bounds,
                                      const uint64_t* out_off, uint64_t* count, void* vmin, void* vmax,
                                      double* sum, double* sum_sq, int32_t mem);
+/* Per-cell statistics over time of n windows, reduced on the device from the encoded bytes (no reference counterpart).
+ * One record per (window, cell): window i has (bottom - top) * (right - left) records, row-major, from record out_off[i]
+ * on (out_off[n+1] host array, the convention of dcdf_superchunk_window_batch counted in records).  Record r is
+ * count[r], n_band[r], vmin / vmax[r], sum[r], sum_sq[r].
+ *  - value of a cell at an instant: as for dcdf_superchunk_window_stats, exactly what dcdf_superchunk_window writes.
+ *    NaN values are skipped.
+ *  - count (uint64): the number of non-NaN instants, exact.
+ *  - n_band (uint64): the number of instants with lower[i] <= (double)v <= upper[i]; NaN never counts.  Reversed bounds
+ *    are swapped, +-inf is allowed, a NaN bound returns DCDF_ERR_BAD_ARG.  lower and upper both NULL: no band, n_band
+ *    may be NULL (when given, it receives count).
+ *  - vmin / vmax: in the superchunk's encoding, compared by value.  count == 0: NaN for float encodings, 0 for integer ones.
+ *  - sum / sum_sq (double), in a fixed order.  A piece is the window's instants inside one time slice.  Per piece,
+ *    s_p = ((0 + v_0) + v_1) + ... in double, in time order, v the value converted to double (exact for f32 / f64 / i32,
+ *    round-to-nearest for i64); sum_sq adds v * v rounded once.  The record's sum is ((0 + s_0) + s_1) + ... over the
+ *    pieces in time order.
+ *  - accumulate != 0: the outputs hold records of an earlier call for the same window shapes, and this call continues
+ *    them as if its pieces followed the earlier ones: counts add, min / max fold by value, each piece is added to the
+ *    running sums in order.  (A Variable's span groups end on slice boundaries, so a series of calls over consecutive
+ *    instants equals one call.)
+ *  - determinism: a window's records are bitwise identical alone or inside any batch, with or without "window_wide",
+ *    for a built superchunk and the same one reopened, and for any "time_stats_scratch".
+ *  - a zero-instant window gives records with count 0 (unchanged under accumulate); a zero-area window has no records.
+ *    Out-of-range windows return DCDF_ERR_OUT_OF_BOUNDS; out_off that does not match the areas, NULL outputs, a NaN
+ *    bound, or subchunks larger than 64x64 (only possible for an opened superchunk) return DCDF_ERR_BAD_ARG.  `mem`
+ *    says where all six outputs live. */
+int32_t dcdf_superchunk_time_stats(dcdf_ctx* ctx, const dcdf_superchunk* sc, uint64_t n, const dcdf_cube* bounds,
+                                   const uint64_t* out_off, const double* lower, const double* upper,
+                                   uint64_t* count, uint64_t* n_band, void* vmin, void* vmax,
+                                   double* sum, double* sum_sq, int32_t accumulate, int32_t mem);
 /* Batched value-range search over n windows (same fixed-point [lower, upper] semantics as
  * dcdf_chunk_search).  counts[n] (host) receives matches per window; out_irc (may be NULL) receives the
  * triplets window after window.  Order inside a window: subchunks row-major, then chunk order. */
