@@ -5,7 +5,7 @@
 // add, and the kernel can be small:
 //   * same mapping as encode_v4.cuh (one 64-thread CTA per unit, thread t = level-3 node t in Morton order, 8x8 cells),
 //     same masks / packed counters / BFS layout arithmetic, same bytes;
-//   * ONE fused pass per Log instant: a thread reads its four level-4 nodes (4x4 cells each, four 128-bit loads)
+//   * ONE fused pass per instant: a thread reads its four level-4 nodes (4x4 cells each, four 128-bit loads)
 //     straight from global memory, converts, and while the cells are in registers computes the differences to the
 //     block's snapshot, the equal / uniform flags, the length classes AND the low bytes of every zigzag code, which
 //     go to a 6 KB payload in shared memory.  The instant itself is never stored: emission copies payload words to
@@ -13,9 +13,11 @@
 //     pyramid, second zigzag -- is gone);
 //   * entries longer than one byte (rare below the root) are re-derived at emission time from a second, L2-resident
 //     read of just that level-4 node;
-//   * a Snapshot is needed for one instant in several (first of a block): its exact size (only when the Log does not
-//     already beat the one-byte-per-entry lower bound) and its emission each take their own pass over the tile from
-//     L2; the emission pass also rewrites the snapshot image the following Logs refer to;
+//   * the same pass sizes the Snapshot candidate exactly, so the Log / Snapshot decision needs no second pass: a
+//     Snapshot's level-6 and level-5 entries all lie within their level-4 node's range, so one test per node proves
+//     them one byte long (nodes with a range above 127, and nodes the raster's edge cuts through, are re-read from L2);
+//   * a Snapshot (one instant in several, the first of a block among them) takes a pass over the tile from L2 for its
+//     emission, which also rewrites the snapshot image the following Logs refer to;
 //   * the emission image is placed so that byte 1 of the max DAC's level 0 is 4-byte aligned: every sibling group
 //     (BFS positions 1 + 4k .. 4 + 4k) is then one aligned 32-bit store; the copy to the arena re-aligns with funnel
 //     shifts.
@@ -304,6 +306,34 @@ __device__ __noinline__ void e5_long_node(bool as_snapshot, const float* pn, i64
   pos[0] = lx1; pos[1] = rx1; pos[2] = rn1;
 }
 
+// Snapshot entries of one level-4 node that take two bytes (snapshot.rs:122-147: quad max - cell, node max - quad max,
+// quad min - node min), cell by cell from a second (L2-resident) read of the node: leaves (bits 15..0, cell m of the node
+// = bit 15 - m), quad max entries (bits 19..16, quad b = bit 19 - b), quad min entries (bits 23..20).  Rare: only for
+// nodes whose range does not prove every entry short, and for nodes the raster's edge cuts through
+template <bool FULL>
+__device__ __noinline__ u32 e5_snap_long(const float* pn, i64 sr, float scale2, int rl, int cl, int vec) {
+  uint4 raw[4];
+  int4 q[4];
+  e5_load_node<FULL>(pn, sr, raw, rl, cl, vec);
+  e5_quads<FULL>(raw, scale2, q, rl, cl);
+  int qmax[4], qmin[4];
+#pragma unroll
+  for (int b = 0; b < 4; b++) e4_qmm<FULL>(q[b], qmax[b], qmin[b]);
+  const int amax = max(max(qmax[0], qmax[1]), max(qmax[2], qmax[3])), amin = min(min(qmin[0], qmin[1]), min(qmin[2], qmin[3]));
+  u32 m = 0;
+#pragma unroll
+  for (int b = 0; b < 4; b++) {
+    const int4 t = q[b];
+    if (e4_longer<1>(e5_dx<FULL>(qmax[b], t.x))) m |= 1u << (15 - 4 * b);
+    if (e4_longer<1>(e5_dx<FULL>(qmax[b], t.y))) m |= 1u << (14 - 4 * b);
+    if (e4_longer<1>(e5_dx<FULL>(qmax[b], t.z))) m |= 1u << (13 - 4 * b);
+    if (e4_longer<1>(e5_dx<FULL>(qmax[b], t.w))) m |= 1u << (12 - 4 * b);
+    if (e4_longer<1>(e5_dx<FULL>(amax, qmax[b]))) m |= 1u << (19 - b);
+    if (e4_longer<1>(e5_dn(qmin[b], amin))) m |= 1u << (23 - b);
+  }
+  return m;
+}
+
 // mbarrier + bulk copy (the TMA unit's 1-D form) for the BULK variant of the kernel
 DCDF_DEVINL u32 e5_smem_u32(const void* p) { return (u32)__cvta_generic_to_shared(p); }
 DCDF_DEVINL void e5_mbar_init(unsigned long long* b, u32 count) {
@@ -473,196 +503,163 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
     E5Tot T;
     u32 ntop = 0, item_cnt = 0, item_size = 0;  // the winner's top-entry counts and this lane's stream item (e5_item)
     bool as_snapshot = forced;
-    u32 my_size = 0, log_size = 0;
+    u32 my_size = 0;
 
-    // Pass 0: the fused Log pass and the Log's exact size against a lower bound of the Snapshot's.  Pass 1 (first
-    // instant of a block, the 254-log cap, or a Log that does not beat the bound): the Snapshot's exact size.
-#pragma unroll 1
-    for (int pass = forced ? 1 : 0; pass < 2; pass++) {
-      t3max = INT32_MIN; t3min = INT32_MAX;
-      u5 = 0; u4 = 0;
+    // ONE fused pass decides: the Log's differences, flags, length classes and payload, the Snapshot's entry masks, then
+    // the exact sizes of both candidates.  A forced Snapshot (first instant of a block, the 254-log cap) runs the Log part
+    // too, against a snapshot image that may be stale or not set yet, and ignores it.
+    t3max = INT32_MIN; t3min = INT32_MAX;
+    {
+      // ---------------- load, convert, differences, flags, length classes, payload
       uint4 raw[4];
       e5_load_node<FULL>(e5_node_ptr(pt, sr, 0), sr, raw, E5_RL(0), E5_CL(0), vec);
-      if (pass == 0) {
-        // ---------------- load, convert, differences, flags, length classes, payload
-        eq3 = true;
+      eq3 = true;
 #pragma unroll 1
-        for (int a = 0; a < 4; a++) {
-          int4 q[4];
-          e5_quads<FULL>(raw, scale2, q, E5_RL(a), E5_CL(a));
-          if (a < 3) e5_load_node<FULL>(e5_node_ptr(pt, sr, a + 1), sr, raw, E5_RL(a + 1), E5_CL(a + 1), vec);
-          const int2 s4 = S.l4s[a][tid];
-          int amax = INT32_MIN, amin = INT32_MAX, dfirst = 0;
-          bool aeq = true;
-          u32 leaf16 = 0, u5n = 0, e5n = 0, qx = 0, qn = 0;
-          u32 exw = 0, enw = 0;          // low bytes of the four quad max / min entries
-          u32 ovx = 0, ovn = 0, ovm = 0; // exact low bytes of the zigzag codes of entries outside -128..127
+      for (int a = 0; a < 4; a++) {
+        int4 q[4];
+        e5_quads<FULL>(raw, scale2, q, E5_RL(a), E5_CL(a));
+        if (a < 3) e5_load_node<FULL>(e5_node_ptr(pt, sr, a + 1), sr, raw, E5_RL(a + 1), E5_CL(a + 1), vec);
+        const int2 s4 = S.l4s[a][tid];
+        int amax = INT32_MIN, amin = INT32_MAX, dfirst = 0;
+        bool aeq = true;
+        u32 leaf16 = 0, u5n = 0, e5n = 0, qx = 0, qn = 0;
+        u32 exw = 0, enw = 0;          // low bytes of the four quad max / min entries
+        u32 ovx = 0, ovn = 0, ovm = 0; // exact low bytes of the zigzag codes of entries outside -128..127
 #pragma unroll
-          for (int b = 0; b < 4; b++) {
-            const int4 t = q[b], sq = S.cell[4 * a + b][tid];
-            int qmax, qmin, sqmax, sqmin;
-            e4_qmm<FULL>(t, qmax, qmin);
-            e4_qmm<FULL>(sq, sqmax, sqmin);
-            const int d0 = e4_sub(t.x, sq.x), d1 = e4_sub(t.y, sq.y), d2 = e4_sub(t.z, sq.z), d3 = e4_sub(t.w, sq.w);  // None - None = 0 (log.rs:751)
-            const int ex = e5_dx<FULL>(qmax, sqmax), en = e5_dn(qmin, sqmin);
-            const bool e5 = (((d1 ^ d0) | (d2 ^ d0) | (d3 ^ d0)) == 0);  // all four leaf diffs equal (log.rs:780-806)
-            if (e4_unif<FULL>(qmax, qmin)) u5n |= 1u << (3 - b);
-            if (e5) e5n |= 1u << (3 - b);
-            u32 leafw = e5_zz4(e5_low4(d0, d1, d2, d3));
-            exw = __byte_perm(exw, (u32)ex, b == 0 ? 0x3214 : b == 1 ? 0x3240 : b == 2 ? 0x3410 : 0x4210);
-            enw = __byte_perm(enw, (u32)en, b == 0 ? 0x3214 : b == 1 ? 0x3240 : b == 2 ? 0x3410 : 0x4210);
-            // one test for "some entry of this quad needs two bytes" (zigzag code above 255  <=>  value outside -128..127)
-            if ((((u32)d0 + 128u) | ((u32)d1 + 128u) | ((u32)d2 + 128u) | ((u32)d3 + 128u) | ((u32)ex + 128u) | ((u32)en + 128u)) > 255u) {
-              if (e4_longer<1>(d0)) leaf16 |= 1u << (15 - 4 * b);
-              if (e4_longer<1>(d1)) leaf16 |= 1u << (14 - 4 * b);
-              if (e4_longer<1>(d2)) leaf16 |= 1u << (13 - 4 * b);
-              if (e4_longer<1>(d3)) leaf16 |= 1u << (12 - 4 * b);
-              if (e4_longer<1>(ex)) qx |= 1u << (3 - b);
-              if (e4_longer<1>(en)) qn |= 1u << (3 - b);
-              if ((((u32)d0 + 32768u) | ((u32)d1 + 32768u) | ((u32)d2 + 32768u) | ((u32)d3 + 32768u)) > 65535u) err |= EF_BAD_FORMAT;  // not eligible
-              leafw = e5_pack4(zigzag32(d0), zigzag32(d1), zigzag32(d2), zigzag32(d3));
-              ovx |= (zigzag32(ex) & 0xffu) << (8 * b);
-              ovn |= (zigzag32(en) & 0xffu) << (8 * b);
-              ovm |= 0xffu << (8 * b);
-            }
-            S.leaf[4 * a + b][tid] = leafw;
-            amax = max(amax, qmax); amin = min(amin, qmin);
-            if (b == 0) dfirst = d0;
-            aeq = aeq && e5 && d0 == dfirst;
+        for (int b = 0; b < 4; b++) {
+          const int4 t = q[b], sq = S.cell[4 * a + b][tid];
+          int qmax, qmin, sqmax, sqmin;
+          e4_qmm<FULL>(t, qmax, qmin);
+          e4_qmm<FULL>(sq, sqmax, sqmin);
+          const int d0 = e4_sub(t.x, sq.x), d1 = e4_sub(t.y, sq.y), d2 = e4_sub(t.z, sq.z), d3 = e4_sub(t.w, sq.w);  // None - None = 0 (log.rs:751)
+          const int ex = e5_dx<FULL>(qmax, sqmax), en = e5_dn(qmin, sqmin);
+          const bool e5 = (((d1 ^ d0) | (d2 ^ d0) | (d3 ^ d0)) == 0);  // all four leaf diffs equal (log.rs:780-806)
+          if (e4_unif<FULL>(qmax, qmin)) u5n |= 1u << (3 - b);
+          if (e5) e5n |= 1u << (3 - b);
+          u32 leafw = e5_zz4(e5_low4(d0, d1, d2, d3));
+          exw = __byte_perm(exw, (u32)ex, b == 0 ? 0x3214 : b == 1 ? 0x3240 : b == 2 ? 0x3410 : 0x4210);
+          enw = __byte_perm(enw, (u32)en, b == 0 ? 0x3214 : b == 1 ? 0x3240 : b == 2 ? 0x3410 : 0x4210);
+          // one test for "some entry of this quad needs two bytes" (zigzag code above 255  <=>  value outside -128..127)
+          if ((((u32)d0 + 128u) | ((u32)d1 + 128u) | ((u32)d2 + 128u) | ((u32)d3 + 128u) | ((u32)ex + 128u) | ((u32)en + 128u)) > 255u) {
+            if (e4_longer<1>(d0)) leaf16 |= 1u << (15 - 4 * b);
+            if (e4_longer<1>(d1)) leaf16 |= 1u << (14 - 4 * b);
+            if (e4_longer<1>(d2)) leaf16 |= 1u << (13 - 4 * b);
+            if (e4_longer<1>(d3)) leaf16 |= 1u << (12 - 4 * b);
+            if (e4_longer<1>(ex)) qx |= 1u << (3 - b);
+            if (e4_longer<1>(en)) qn |= 1u << (3 - b);
+            // not eligible (a forced Snapshot's image may be stale: nothing to check)
+            if (!forced && (((u32)d0 + 32768u) | ((u32)d1 + 32768u) | ((u32)d2 + 32768u) | ((u32)d3 + 32768u)) > 65535u) err |= EF_BAD_FORMAT;
+            leafw = e5_pack4(zigzag32(d0), zigzag32(d1), zigzag32(d2), zigzag32(d3));
+            ovx |= (zigzag32(ex) & 0xffu) << (8 * b);
+            ovn |= (zigzag32(en) & 0xffu) << (8 * b);
+            ovm |= 0xffu << (8 * b);
           }
-          const u32 zxw = (e5_zz4(exw) & ~ovm) | ovx, znw = (e5_zz4(enw) & ~ovm) | ovn;
-          S.qx[a][tid] = zxw;
-          S.qn[a][tid] = znw;
-          S.l4t[a][tid] = make_int2(amax, amin);
-          L.ml |= (u64)leaf16 << (48 - 16 * a);
-          L.mq |= (qx << (12 - 4 * a)) | (qn << (28 - 4 * a));
-          u5 |= u5n << (12 - 4 * a);
-          eq5 |= e5n << (12 - 4 * a);
-          if (e4_unif<FULL>(amax, amin)) u4 |= 1u << (3 - a);
-          if (aeq) eq4 |= 1u << (3 - a);
-          if (e4_longer<1>(e5_dx<FULL>(amax, s4.x))) L.mu |= 1u << (3 - a);
-          if (e4_longer<1>(e5_dn(amin, s4.y))) L.mu |= 1u << (7 - a);
-          t3max = max(t3max, amax); t3min = min(t3min, amin);
-          if (a == 0) diff3 = dfirst;
-          eq3 = eq3 && aeq && dfirst == diff3;
+          S.leaf[4 * a + b][tid] = leafw;
+          amax = max(amax, qmax); amin = min(amin, qmin);
+          if (b == 0) dfirst = d0;
+          aeq = aeq && e5 && d0 == dfirst;
         }
-        if (e4_longer<1>(e5_dx<FULL>(t3max, s3max))) L.mu |= 1u << 8;
-        if (e4_longer<1>(e5_dn(t3min, s3min))) L.mu |= 1u << 9;
-      } else {
-        // ---------------- Snapshot entry masks of levels 6 and 5 (snapshot.rs:122-147: parent_max - child_max,
-        // child_min - parent_min); the uniform flags and the level-4 records come out the same as in pass 0
-        C.ml = 0; C.mq = 0;
-#pragma unroll 1
-        for (int a = 0; a < 4; a++) {
-          int4 q[4];
-          e5_quads<FULL>(raw, scale2, q, E5_RL(a), E5_CL(a));
-          if (a < 3) e5_load_node<FULL>(e5_node_ptr(pt, sr, a + 1), sr, raw, E5_RL(a + 1), E5_CL(a + 1), vec);
-          int qmax[4], qmin[4];
-#pragma unroll
-          for (int b = 0; b < 4; b++) e4_qmm<FULL>(q[b], qmax[b], qmin[b]);
-          const int amax = max(max(qmax[0], qmax[1]), max(qmax[2], qmax[3])), amin = min(min(qmin[0], qmin[1]), min(qmin[2], qmin[3]));
-          u32 leaf16 = 0, qx = 0, qn = 0, u5n = 0;
-#pragma unroll
-          for (int b = 0; b < 4; b++) {
-            const int4 t = q[b];
-            if (e4_unif<FULL>(qmax[b], qmin[b])) u5n |= 1u << (3 - b);
-            // full tiles: every difference is >= 0 and below the quad's / node's range; clipped: a cell outside counts as 0
-            if (!FULL || ((u32)(qmax[b] - qmin[b]) | (u32)(amax - qmax[b]) | (u32)(qmin[b] - amin)) > 127u) {
-              if (e4_longer<1>(e5_dx<FULL>(qmax[b], t.x))) leaf16 |= 1u << (15 - 4 * b);
-              if (e4_longer<1>(e5_dx<FULL>(qmax[b], t.y))) leaf16 |= 1u << (14 - 4 * b);
-              if (e4_longer<1>(e5_dx<FULL>(qmax[b], t.z))) leaf16 |= 1u << (13 - 4 * b);
-              if (e4_longer<1>(e5_dx<FULL>(qmax[b], t.w))) leaf16 |= 1u << (12 - 4 * b);
-              if (e4_longer<1>(e5_dx<FULL>(amax, qmax[b]))) qx |= 1u << (3 - b);
-              if (e4_longer<1>(e5_dn(qmin[b], amin))) qn |= 1u << (3 - b);
-            }
+        const u32 zxw = (e5_zz4(exw) & ~ovm) | ovx, znw = (e5_zz4(enw) & ~ovm) | ovn;
+        S.qx[a][tid] = zxw;
+        S.qn[a][tid] = znw;
+        S.l4t[a][tid] = make_int2(amax, amin);
+        L.ml |= (u64)leaf16 << (48 - 16 * a);
+        L.mq |= (qx << (12 - 4 * a)) | (qn << (28 - 4 * a));
+        u5 |= u5n << (12 - 4 * a);
+        eq5 |= e5n << (12 - 4 * a);
+        if (e4_unif<FULL>(amax, amin)) u4 |= 1u << (3 - a);
+        if (aeq) eq4 |= 1u << (3 - a);
+        if (e4_longer<1>(e5_dx<FULL>(amax, s4.x))) L.mu |= 1u << (3 - a);
+        if (e4_longer<1>(e5_dn(amin, s4.y))) L.mu |= 1u << (7 - a);
+        t3max = max(t3max, amax); t3min = min(t3min, amin);
+        if (a == 0) diff3 = dfirst;
+        eq3 = eq3 && aeq && dfirst == diff3;
+        // ---------------- Snapshot entries of levels 6 and 5 (snapshot.rs:122-147): every one lies in 0 .. amax - amin,
+        // so one test per node proves them all short.  Clipped tiles: a cell outside the raster counts as 0, so a node
+        // the raster's edge cuts through takes the exact path; a node wholly outside has nothing but zero entries
+        {
+          const int rl = E5_RL(a), cl = E5_CL(a);
+          const bool inside = FULL || (rl >= 4 && cl >= 4), outside = !FULL && (rl <= 0 || cl <= 0);
+          if (!outside && (!inside || (u32)(amax - amin) > 127u)) {
+            const u32 m = e5_snap_long<FULL>(e5_node_ptr(pt, sr, a), sr, scale2, rl, cl, vec);
+            C.ml |= (u64)(m & 0xffffu) << (48 - 16 * a);
+            C.mq |= (((m >> 16) & 0xfu) << (12 - 4 * a)) | ((m >> 20) << (28 - 4 * a));
           }
-          S.l4t[a][tid] = make_int2(amax, amin);
-          C.ml |= (u64)leaf16 << (48 - 16 * a);
-          C.mq |= (qx << (12 - 4 * a)) | (qn << (28 - 4 * a));
-          u5 |= u5n << (12 - 4 * a);
-          if (e4_unif<FULL>(amax, amin)) u4 |= 1u << (3 - a);
-          t3max = max(t3max, amax); t3min = min(t3min, amin);
         }
-        if (t3max != E4_NONE && (u32)e4_sub(t3max, t3min) > 32767u) err |= EF_BAD_FORMAT;  // not eligible
       }
-      u3 = e4_unif<FULL>(t3max, t3min);
+      if (e4_longer<1>(e5_dx<FULL>(t3max, s3max))) L.mu |= 1u << 8;
+      if (e4_longer<1>(e5_dn(t3min, s3min))) L.mu |= 1u << 9;
+      if (t3max != E4_NONE && (u32)e4_sub(t3max, t3min) > 32767u) err |= EF_BAD_FORMAT;  // not eligible
+    }
+    u3 = e4_unif<FULL>(t3max, t3min);
 
-      // ---------------- levels 2 and 1 with shuffles (4 resp. 16 consecutive lanes)
-      t2max = max(t3max, shfl_xor(t3max, 1)); t2max = max(t2max, shfl_xor(t2max, 2));
-      t2min = min(t3min, shfl_xor(t3min, 1)); t2min = min(t2min, shfl_xor(t2min, 2));
-      const int diff2 = shfl(diff3, lane & ~3);
-      const u32 ok3 = __ballot_sync(0xffffffffu, eq3 && diff3 == diff2);
-      eq2 = ((ok3 >> (lane & ~3)) & 0xfu) == 0xfu;
-      u2 = e4_unif<FULL>(t2max, t2min);
-      t1max = max(t2max, shfl_xor(t2max, 4)); t1max = max(t1max, shfl_xor(t1max, 8));
-      t1min = min(t2min, shfl_xor(t2min, 4)); t1min = min(t1min, shfl_xor(t1min, 8));
-      const int diff1 = shfl(diff2, lane & ~15);
-      const u32 ok2 = __ballot_sync(0xffffffffu, eq2 && diff2 == diff1);
-      const bool eq1 = ((ok2 >> (lane & ~15)) & 0xffffu) == 0xffffu;
-      const bool u1 = e4_unif<FULL>(t1max, t1min);
+    // ---------------- levels 2 and 1 with shuffles (4 resp. 16 consecutive lanes)
+    t2max = max(t3max, shfl_xor(t3max, 1)); t2max = max(t2max, shfl_xor(t2max, 2));
+    t2min = min(t3min, shfl_xor(t3min, 1)); t2min = min(t2min, shfl_xor(t2min, 2));
+    const int diff2 = shfl(diff3, lane & ~3);
+    const u32 ok3 = __ballot_sync(0xffffffffu, eq3 && diff3 == diff2);
+    eq2 = ((ok3 >> (lane & ~3)) & 0xfu) == 0xfu;
+    u2 = e4_unif<FULL>(t2max, t2min);
+    t1max = max(t2max, shfl_xor(t2max, 4)); t1max = max(t1max, shfl_xor(t1max, 8));
+    t1min = min(t2min, shfl_xor(t2min, 4)); t1min = min(t1min, shfl_xor(t1min, 8));
+    const int diff1 = shfl(diff2, lane & ~15);
+    const u32 ok2 = __ballot_sync(0xffffffffu, eq2 && diff2 == diff1);
+    const bool eq1 = ((ok2 >> (lane & ~15)) & 0xffffu) == 0xffffu;
+    const bool u1 = e4_unif<FULL>(t1max, t1min);
 
-      // structure flags: snapshot internal = !uniform (snapshot.rs:133); log internal = !uniform && !equal (log.rs:137-152)
-      C.in5 = ~u5 & 0xffffu; C.in4 = ~u4 & 0xfu; C.in3 = !u3; C.in2 = !u2; C.in1 = !u1;
-      if (pass == 0) {
-        if (e4_longer<1>(e5_dx<FULL>(t2max, s2max))) L.mu |= 1u << 10;
-        if (e4_longer<1>(e5_dn(t2min, s2min))) L.mu |= 1u << 11;
-        L.in5 = ~u5 & ~eq5 & 0xffffu; L.in4 = ~u4 & ~eq4 & 0xfu; L.in3 = !u3 && !eq3; L.in2 = !u2 && !eq2; L.in1 = !u1 && !eq1;
-        e5_count(L, owner2, wl);
-      } else {
-        C.mu = 0;  // entry masks of the Snapshot above the quads
+    // structure flags: snapshot internal = !uniform (snapshot.rs:133); log internal = !uniform && !equal (log.rs:137-152)
+    C.in5 = ~u5 & 0xffffu; C.in4 = ~u4 & 0xfu; C.in3 = !u3; C.in2 = !u2; C.in1 = !u1;
+    if (e4_longer<1>(e5_dx<FULL>(t2max, s2max))) L.mu |= 1u << 10;
+    if (e4_longer<1>(e5_dn(t2min, s2min))) L.mu |= 1u << 11;
+    L.in5 = ~u5 & ~eq5 & 0xffffu; L.in4 = ~u4 & ~eq4 & 0xfu; L.in3 = !u3 && !eq3; L.in2 = !u2 && !eq2; L.in1 = !u1 && !eq1;
+    e5_count(L, owner2, wl);
+    // entry masks of the Snapshot above the quads
 #pragma unroll
-        for (int a = 0; a < 4; a++) {
-          const int2 n4 = S.l4t[a][tid];
-          if (e4_longer<1>(e5_dx<FULL>(t3max, n4.x))) C.mu |= 1u << (3 - a);
-          if (e4_longer<1>(e5_dn(n4.y, t3min))) C.mu |= 1u << (7 - a);
-        }
-        if (e4_longer<1>(e5_dx<FULL>(t2max, t3max))) C.mu |= 1u << 8;
-        if (e4_longer<1>(e5_dn(t3min, t2min))) C.mu |= 1u << 9;
-        if (e4_longer<1>(e5_dx<FULL>(t1max, t2max))) C.mu |= 1u << 10;
-        if (e4_longer<1>(e5_dn(t2min, t1min))) C.mu |= 1u << 11;
-      }
-      e5_count(C, owner2, ws);  // pass 0: structure only (the masks are still empty) -> the lower bound
+    for (int a = 0; a < 4; a++) {
+      const int2 n4 = S.l4t[a][tid];
+      if (e4_longer<1>(e5_dx<FULL>(t3max, n4.x))) C.mu |= 1u << (3 - a);
+      if (e4_longer<1>(e5_dn(n4.y, t3min))) C.mu |= 1u << (7 - a);
+    }
+    if (e4_longer<1>(e5_dx<FULL>(t2max, t3max))) C.mu |= 1u << 8;
+    if (e4_longer<1>(e5_dn(t3min, t2min))) C.mu |= 1u << 9;
+    if (e4_longer<1>(e5_dx<FULL>(t1max, t2max))) C.mu |= 1u << 10;
+    if (e4_longer<1>(e5_dn(t2min, t1min))) C.mu |= 1u << 11;
+    e5_count(C, owner2, ws);
 
-      // ---------------- per-warp totals and the four level-1 records go through shared memory
-      if (pass == 1 && !forced) e5_tile_sync<NW>(slot);  // the other warp may still be reading the totals of pass 0
+    // ---------------- per-warp totals and the four level-1 records go through shared memory
 #pragma unroll
-      for (int i = 0; i < 4; i++) {
-        const u32 rs = __reduce_add_sync(0xffffffffu, ws[i]);
-        if (lane == 0) S.wt[warp][0][i] = rs;
-        if (pass == 0) {
-          const u32 rl = __reduce_add_sync(0xffffffffu, wl[i]);
-          if (lane == 0) S.wt[warp][1][i] = rl;
-        }
-      }
-      if ((lane & 15) == 0) {
-        S.rec1[k1] = make_int4(t1max, t1min, diff1, eq1 ? 1 : 0);
-        if (pass == 0) S.ent1[k1] = make_int2(e5_dx<FULL>(t1max, s1max), e5_dn(t1min, s1min));
-      }
-      e5_tile_sync<NW>(slot);  // B1
+    for (int i = 0; i < 4; i++) {
+      const u32 rs = __reduce_add_sync(0xffffffffu, ws[i]);
+      const u32 rl = __reduce_add_sync(0xffffffffu, wl[i]);
+      if (lane == 0) { S.wt[warp][0][i] = rs; S.wt[warp][1][i] = rl; }
+    }
+    if ((lane & 15) == 0) {
+      S.rec1[k1] = make_int4(t1max, t1min, diff1, eq1 ? 1 : 0);
+      S.ent1[k1] = make_int2(e5_dx<FULL>(t1max, s1max), e5_dn(t1min, s1min));
+    }
+    e5_tile_sync<NW>(slot);  // B1
 
-      // ---------------- root from the level-1 records, one per lane (lane 1 + k: node k; the others hold neutral values)
-      {
-        const int4 r = S.rec1[(lane - 1) & 3];
-        n1max = is1 ? r.x : INT32_MIN; n1min = is1 ? r.y : INT32_MAX;
-        n1un = e4_unif<FULL>(r.x, r.y);
-        n1eq = r.w != 0;
-        t0max = __reduce_max_sync(0xffffffffu, n1max);
-        t0min = __reduce_min_sync(0xffffffffu, n1min);
-        const int dif0 = shfl(r.z, 1);
-        eq0 = __ballot_sync(0xffffffffu, is1 && n1eq && r.z == dif0) == 0x1eu;
-        // bit 1 + k of a ballot -> bit 3 - k
-        s_in1 = __brev(__ballot_sync(0xffffffffu, is1 && !n1un)) >> 27;
-        l_in1 = __brev(__ballot_sync(0xffffffffu, is1 && !n1un && !n1eq)) >> 27;
-        if (pass == 0) { const int2 e = S.ent1[(lane - 1) & 3]; l_e1max = e.x; l_e1min = e.y; }
-      }
-      u0 = t0max == t0min;
-      l_in0 = !u0 && !eq0; s_in0 = !u0;
+    // ---------------- root from the level-1 records, one per lane (lane 1 + k: node k; the others hold neutral values)
+    {
+      const int4 r = S.rec1[(lane - 1) & 3];
+      n1max = is1 ? r.x : INT32_MIN; n1min = is1 ? r.y : INT32_MAX;
+      n1un = e4_unif<FULL>(r.x, r.y);
+      n1eq = r.w != 0;
+      t0max = __reduce_max_sync(0xffffffffu, n1max);
+      t0min = __reduce_min_sync(0xffffffffu, n1min);
+      const int dif0 = shfl(r.z, 1);
+      eq0 = __ballot_sync(0xffffffffu, is1 && n1eq && r.z == dif0) == 0x1eu;
+      // bit 1 + k of a ballot -> bit 3 - k
+      s_in1 = __brev(__ballot_sync(0xffffffffu, is1 && !n1un)) >> 27;
+      l_in1 = __brev(__ballot_sync(0xffffffffu, is1 && !n1un && !n1eq)) >> 27;
+      const int2 e = S.ent1[(lane - 1) & 3]; l_e1max = e.x; l_e1min = e.y;
+    }
+    u0 = t0max == t0min;
+    l_in0 = !u0 && !eq0; s_in0 = !u0;
 
-      // ---------------- exact size of this pass's candidate (snapshot.rs:84-93, log.rs:92-98): one stream item per lane
-      const bool as_log = pass == 0;
-      E5Tot Tc;
-      u32 c_ntop, c_cnt;
-      {
+    // ---------------- exact sizes of both candidates (snapshot.rs:84-93, log.rs:92-98): one stream item per lane
+    {
+      auto cand_size = [&](bool as_log, E5Tot& Tc, u32& c_ntop, u32& c_cnt) {
         const bool c_in0 = as_log ? l_in0 : s_in0;
         const bool c_int1 = !n1un && !(as_log && n1eq);  // own level-1 node internal
         const int ex = lane == 0 ? (as_log ? t0max - s0max : t0max) : as_log ? l_e1max : e5_dx<FULL>(t0max, n1max);
@@ -670,23 +667,20 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
         const int lx = e5_len(lane == 0 || (c_in0 && is1), ex), ln = e5_len(c_in0 && (lane == 0 || (is1 && c_int1)), en);
         c_ntop = __reduce_add_sync(0xffffffffu, e5_nib(lx) | (e5_nib(ln) << 16));
         e5_totals(Tc, S, as_log ? 1 : 0, c_in0, as_log ? l_in1 : s_in1);
-      }
-      const u32 c_size = e5_item(c_cnt, Tc, as_log, c_ntop, lane);
-      const u32 size = 13u + __reduce_add_sync(0xffffffffu, c_size);
-      if (as_log) {
-        T = Tc;
-        ntop = c_ntop; item_cnt = c_cnt; item_size = c_size;
-        log_size = size; my_size = size;
-        // lower bound of the Snapshot: every entry takes at least one byte
-        const u32 st = s_in0 ? S.wt[0][0][0] + S.wt[1][0][0] : 0u;
-        const u32 s_upper = (s_in0 ? 1u + (u32)__popc(s_in1) : 0u) + e4_f2(st) + e4_f3(st) + e4_f4(st);
-        const u32 s_int = s_upper + e4_f5(st), s_nm = 1u + 4u * s_upper, s_nmax = 1u + 4u * s_int;
-        const u32 snap_lb = 13u + bitmap_size(s_nm) + 1u + bitmap_size(s_nmax) + s_nmax + (s_int ? 1u + bitmap_size(s_int) + s_int : 1u);
-        if (!(snap_lb <= log_size)) break;  // the Log wins without looking closer
-      } else {
-        as_snapshot = forced || size <= log_size;  // ties go to the snapshot (chunk.rs:62)
-        if (as_snapshot) { T = Tc; ntop = c_ntop; item_cnt = c_cnt; item_size = c_size; my_size = size; }
-      }
+        return e5_item(c_cnt, Tc, as_log, c_ntop, lane);
+      };
+      E5Tot Tl;
+      u32 l_ntop, l_cnt, s_ntop, s_cnt;
+      const u32 s_item = cand_size(false, T, s_ntop, s_cnt);
+      const u32 l_item = cand_size(true, Tl, l_ntop, l_cnt);
+      const u32 snap_size = 13u + __reduce_add_sync(0xffffffffu, s_item);
+      const u32 log_size = 13u + __reduce_add_sync(0xffffffffu, l_item);
+      as_snapshot = forced || snap_size <= log_size;  // ties go to the snapshot (chunk.rs:62)
+      if (!as_snapshot) T = Tl;
+      ntop = as_snapshot ? s_ntop : l_ntop;
+      item_cnt = as_snapshot ? s_cnt : l_cnt;
+      item_size = as_snapshot ? s_item : l_item;
+      my_size = as_snapshot ? snap_size : log_size;
     }
 
     // ---------------- the winner, generic from here on
