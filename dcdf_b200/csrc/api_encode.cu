@@ -158,7 +158,7 @@ void launch_encode_v4(dcdf_ctx* ctx, const EncParams& P, u32 grid) {
 template <int G, bool BULK>
 void launch_encode_v5_variant(dcdf_ctx* ctx, const EncParams& P, u32 grid) {
   const u32 stage_limit = std::min<u32>(ctx->opt.stage_limit, (u32)E5_POOL);
-  const size_t smem = (sizeof(E5Smem) + (BULK ? sizeof(E5Bulk) : 0)) * G;
+  const size_t smem = (sizeof(E5Smem<true>) + (BULK ? sizeof(E5Bulk) : 0)) * G;
   CK(cudaFuncSetAttribute(k_encode_v5<G, true, BULK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   k_encode_v5<G, true, BULK><<<(grid + G - 1) / G, E5_THREADS * G, smem, ctx->stream>>>(P, stage_limit, ctx->opt.fast_sync_mask);
   CK(cudaGetLastError());
@@ -171,7 +171,7 @@ void launch_encode_v5(dcdf_ctx* ctx, const EncParams& P, u32 grid) {
   if (FULL && ctx->opt.fast_variant == 2 && ((P.stride_r | P.stride_t) & 3) == 0 && (((uintptr_t)P.data + 4 * 0) & 15) == 0)
     return launch_encode_v5_variant<4, true>(ctx, P, grid);
   const u32 stage_limit = std::min<u32>(ctx->opt.stage_limit, (u32)E5_POOL);
-  const size_t smem = sizeof(E5Smem) * G;
+  const size_t smem = sizeof(E5Smem<FULL>) * G;
   CK(cudaFuncSetAttribute(k_encode_v5<G, FULL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   k_encode_v5<G, FULL><<<(grid + G - 1) / G, E5_THREADS * G, smem, FULL ? ctx->stream : ctx->aux_stream>>>(P, stage_limit, ctx->opt.fast_sync_mask);
   CK(cudaGetLastError());

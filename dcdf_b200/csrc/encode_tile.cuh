@@ -43,6 +43,7 @@ struct EncUnit {
   u32 piece_base;   // first entry of this unit in the piece table
   u32 slot;         // caller-defined (subchunk slot inside its slice)
   int row0, col0;   // origin of the tile inside its region (row-major order of the NaN quirk)
+  int fmin;         // units of k_encode_v5: the smallest fixed code of the unit (k_finalize_tree); full tiles code cells relative to it
 };
 enum : int { UF_ROUND = 1, UF_NARROW = 2, UF_SKIP = 4, UF_FULL = 8 /* 64x64, all in bounds */,
               UF_EXACT = 16 /* float unit whose values all have <= bits fractional bits and are finite: to_fixed never rounds */ };

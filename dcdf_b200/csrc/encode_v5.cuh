@@ -16,11 +16,15 @@
 //   * the same pass sizes the Snapshot candidate exactly, so the Log / Snapshot decision needs no second pass: a
 //     Snapshot's level-6 and level-5 entries all lie within their level-4 node's range, so one test per node proves
 //     them one byte long (nodes with a range above 127, and nodes the raster's edge cuts through, are re-read from L2);
-//   * a Snapshot (one instant in several, the first of a block among them) takes a pass over the tile from L2 for its
-//     emission, which also rewrites the snapshot image the following Logs refer to;
+//   * a Snapshot (one instant in several, the first of a block among them) takes a pass over the tile for its emission
+//     (clipped tiles: from L2), which also installs the snapshot image the following Logs refer to;
 //   * the emission image is placed so that byte 1 of the max DAC's level 0 is 4-byte aligned: every sibling group
 //     (BFS positions 1 + 4k .. 4 + 4k) is then one aligned 32-bit store; the copy to the arena re-aligns with funnel
 //     shifts.
+//   * full tiles hold their cells as 16-bit codes relative to the unit's smallest fixed code, two per register
+//     (e5_pack_node): the fused pass computes differences, quad max / min, flags, length classes and payload bytes of two
+//     cells per instruction, and keeps the instant's codes as a second image in shared memory that becomes the snapshot
+//     image when a Snapshot wins (its emission pass reads them from there instead of converting the tile again).
 // 36 KB of shared memory per tile and <= 168 registers: six tiles per SM (v4: four).
 // Reference functions restated: snapshot.rs:108-156 + 439-500, log.rs:112-165 + 725-817, bitmap.rs:66-113,
 // dac.rs:96-132, chunk.rs:55-78, serializers snapshot.rs:48-58 / log.rs:53-64 / dac.rs:37-44 / bitmap.rs:128-138.
@@ -37,11 +41,14 @@ constexpr int E5_POOL = 9 * 1024;
 // level-3 node with cells; its structures are at most about half as large
 constexpr int E5_POOL_EDGE = 5 * 1024;
 
-// TT threads per tile (one per level-3 node that can hold cells), POOL bytes of emission image
-template <int TT, int POOL>
+// TT threads per tile (one per level-3 node that can hold cells), POOL bytes of emission image.  PK (full tiles): cells
+// are held as 16-bit codes relative to the unit's smallest fixed code, two per word (e5_pack_node), in two images: the
+// block's snapshot and the instant being encoded, which becomes the snapshot by swapping the two
+template <int TT, int POOL, bool PK>
 struct E5SmemT {
   __align__(16) u8 pool[POOL + 16];  // emission image (+ room for the alignment shift)
-  int4 cell[16][TT];                 // cells of the block's snapshot: [quad q][thread]
+  // cells of the block's snapshot: PK [image][level-4 node a * 2 + quad pair h][thread] (e5_pack_node), else [quad q][thread]
+  std::conditional_t<PK, uint4[2][8][TT], int4[16][TT]> cell;
   int2 l4s[4][TT];                   // (max, min) of the snapshot's level-4 nodes
   int2 l4t[4][TT];                   // ... of the instant being encoded
   u32 leaf[16][TT];                  // Log payload: low bytes of the four leaf codes of quad q
@@ -54,8 +61,9 @@ struct E5SmemT {
   u32 n_bm;
   unsigned long long piece_off;
 };
-using E5Smem = E5SmemT<E5_THREADS, E5_POOL>;
-using E5SmemEdge = E5SmemT<32, E5_POOL_EDGE>;
+template <bool FULL>
+using E5Smem = E5SmemT<E5_THREADS, E5_POOL, FULL>;
+using E5SmemEdge = E5SmemT<32, E5_POOL_EDGE, false>;
 
 struct E5Cand {
   u32 in5, in4;        // internal flags: quad q = bit 15-q, level-4 node a = bit 3-a
@@ -256,6 +264,170 @@ DCDF_DEVINL int e5_dn(int a, int b) { return e4_sub(a, b); }
 DCDF_DEVINL u32 e5_low4(int a, int b, int c, int d) { return __byte_perm(__byte_perm((u32)a, (u32)b, 0x0040), __byte_perm((u32)c, (u32)d, 0x0040), 0x5410); }
 DCDF_DEVINL u32 e5_zz4(u32 p) { return ((p + p) & 0xfefefefeu) ^ (((p >> 7) & 0x01010101u) * 0xffu); }
 DCDF_DEVINL u32 e5_pack4(u32 z0, u32 z1, u32 z2, u32 z3) { return (z0 & 0xffu) | ((z1 & 0xffu) << 8) | ((z2 & 0xffu) << 16) | (z3 << 24); }
+// Full tiles (PK): cells as 16-bit codes relative to the unit's smallest fixed code fmin (k_finalize_tree: every code of
+// the unit lies in fmin .. fmin + 32767), two per word.  A level-4 node is two uint4, one per pair of quads 2h, 2h + 1
+// (h = 0: upper rows, 1: lower rows); word x / y / z / w holds cell x / y / z / w (e4_qmm's order) of quad 2h in bits
+// 15..0 and of quad 2h + 1 in bits 31..16.  Codes take 15 bits, so a - b + 0x00800080 holds d + 128 in each half with
+// no borrow across halves as long as d >= -128: the length class, the low byte and the zigzag code of every difference
+// come from that word, two cells per instruction.
+// to_fixed as in e5_conv_raw with 1 - fmin folded into the constant: the result's bits are 0x4B400000 + (f - fmin)
+DCDF_DEVINL u32 e5_conv_rel(u32 bits, float scale2, float cmag) { return __float_as_uint(__fmaf_rn(__uint_as_float(bits), scale2, cmag)); }
+DCDF_DEVINL u32 e5_rel_or_nan(u32 bits, u32 c, int fmin) { return (bits & 0x7fffffffu) > 0x7f800000u ? 0x4B400000u - (u32)fmin : c; }
+DCDF_DEVINL void e5_pack_node(const uint4 (&raw)[4], float scale2, float cmag, int fmin, uint4 (&w)[2], u32& err) {
+  uint4 c[4];
+#pragma unroll
+  for (int r = 0; r < 4; r++)
+    c[r] = make_uint4(e5_conv_rel(raw[r].x, scale2, cmag), e5_conv_rel(raw[r].y, scale2, cmag), e5_conv_rel(raw[r].z, scale2, cmag),
+                      e5_conv_rel(raw[r].w, scale2, cmag));
+  // every code in fmin .. fmin + 32767  <=>  bits 31..15 of every word are those of 0x4B400000: their OR and their AND
+  // tell.  A NaN (code 0, fixed.rs:35-37) comes out of the FMA as a NaN and fails the test as well
+  auto out_of_window = [&]() {
+    u32 o = 0u, n = ~0u;
+#pragma unroll
+    for (int r = 0; r < 4; r++) { o |= c[r].x | c[r].y | c[r].z | c[r].w; n &= c[r].x & c[r].y & c[r].z & c[r].w; }
+    return (((o & 0xffff8000u) ^ 0x4B400000u) | ((n & 0xffff8000u) ^ 0x4B400000u)) != 0u;
+  };
+  if (out_of_window()) {
+#pragma unroll
+    for (int r = 0; r < 4; r++)
+      c[r] = make_uint4(e5_rel_or_nan(raw[r].x, c[r].x, fmin), e5_rel_or_nan(raw[r].y, c[r].y, fmin), e5_rel_or_nan(raw[r].z, c[r].z, fmin),
+                        e5_rel_or_nan(raw[r].w, c[r].w, fmin));
+    if (out_of_window()) err |= EF_BAD_FORMAT;  // not eligible
+  }
+#pragma unroll
+  for (int h = 0; h < 2; h++) {
+    const uint4 u = c[2 * h], l = c[2 * h + 1];
+    w[h] = make_uint4(__byte_perm(u.x, u.z, 0x5410), __byte_perm(u.y, u.w, 0x5410), __byte_perm(l.x, l.z, 0x5410), __byte_perm(l.y, l.w, 0x5410));
+  }
+}
+// quad b of a node as absolute fixed codes; w: the node's word group of quad pair b >> 1
+DCDF_DEVINL int4 e5_unpack_quad(const uint4& w, int b, int fmin) {
+  const int s = 16 * (b & 1);
+  return make_int4(fmin + (int)((w.x >> s) & 0xffffu), fmin + (int)((w.y >> s) & 0xffffu), fmin + (int)((w.z >> s) & 0xffffu),
+                   fmin + (int)((w.w >> s) & 0xffffu));
+}
+// quad b of a level-4 node of the snapshot image (scell: the node's first entry of E5SmemT::cell, entries TT apart)
+template <bool PK, int TT>
+DCDF_DEVINL int4 e5_snap_quad(const void* scell, int b, int fmin) {
+  if constexpr (PK) return e5_unpack_quad(static_cast<const uint4*>(scell)[(b >> 1) * TT], b, fmin);
+  else return static_cast<const int4*>(scell)[b * TT];
+}
+// zigzag codes of four bytes e = d + 128 (d in -128..127): 2d for e >= 128, 255 - 2e below.  The sign of every byte
+// comes from prmt's sign-replicating selectors, which __byte_perm does not expose (it keeps 3 bits per selector)
+DCDF_DEVINL u32 e5_zz4_off(u32 e) {
+  u32 sgn;
+  asm("prmt.b32 %0, %1, 0, 0xBA98;" : "=r"(sgn) : "r"(e));
+  return ((e + e) & 0xfefefefeu) ^ ~sgn;
+}
+// four bytes of 0 / 1 -> bit 3 - i for byte i
+DCDF_DEVINL u32 e5_bits4(u32 b) { return (b * 0x08040201u) >> 24; }
+// bytes 0 and 2 of two words (halves 0 / 1 of each): quads 0..3 of a node from its two quad-pair words
+DCDF_DEVINL u32 e5_lo_bytes(u32 h0, u32 h1) { return __byte_perm(h0, h1, 0x6420); }
+
+// What the fused pass derives from one level-4 node of a Log: uniform / equal flags of the quads (quad b = bit 3 - b),
+// leaves / quad max / quad min entries longer than one byte, the zigzag low bytes of the quad max / min entries, the
+// node's max and min, the difference of its first cell and whether all sixteen differences are equal
+struct E5LogNode {
+  u32 u5n, e5n, leaf16, qx, qn, zxw, znw, err;
+  int amax, amin, dfirst;
+  bool aeq;
+};
+// ... cell by cell (q: the instant's quads; sq_of(b): the snapshot's quad b).  The low bytes of the four leaf codes of
+// quad b go to leaf[b * TT]
+template <bool FULL, int TT, class SQ>
+DCDF_DEVINL void e5_log_node(const int4 (&q)[4], SQ sq_of, u32* leaf, bool forced, u32& err, E5LogNode& R) {
+  int amax = INT32_MIN, amin = INT32_MAX, dfirst = 0;
+  bool aeq = true;
+  u32 leaf16 = 0, u5n = 0, e5n = 0, qx = 0, qn = 0;
+  u32 exw = 0, enw = 0;          // low bytes of the four quad max / min entries
+  u32 ovx = 0, ovn = 0, ovm = 0; // exact low bytes of the zigzag codes of entries outside -128..127
+#pragma unroll
+  for (int b = 0; b < 4; b++) {
+    const int4 t = q[b], sq = sq_of(b);
+    int qmax, qmin, sqmax, sqmin;
+    e4_qmm<FULL>(t, qmax, qmin);
+    e4_qmm<FULL>(sq, sqmax, sqmin);
+    const int d0 = e4_sub(t.x, sq.x), d1 = e4_sub(t.y, sq.y), d2 = e4_sub(t.z, sq.z), d3 = e4_sub(t.w, sq.w);  // None - None = 0 (log.rs:751)
+    const int ex = e5_dx<FULL>(qmax, sqmax), en = e5_dn(qmin, sqmin);
+    const bool e5 = (((d1 ^ d0) | (d2 ^ d0) | (d3 ^ d0)) == 0);  // all four leaf diffs equal (log.rs:780-806)
+    if (e4_unif<FULL>(qmax, qmin)) u5n |= 1u << (3 - b);
+    if (e5) e5n |= 1u << (3 - b);
+    u32 leafw = e5_zz4(e5_low4(d0, d1, d2, d3));
+    exw = __byte_perm(exw, (u32)ex, b == 0 ? 0x3214 : b == 1 ? 0x3240 : b == 2 ? 0x3410 : 0x4210);
+    enw = __byte_perm(enw, (u32)en, b == 0 ? 0x3214 : b == 1 ? 0x3240 : b == 2 ? 0x3410 : 0x4210);
+    // one test for "some entry of this quad needs two bytes" (zigzag code above 255  <=>  value outside -128..127)
+    if ((((u32)d0 + 128u) | ((u32)d1 + 128u) | ((u32)d2 + 128u) | ((u32)d3 + 128u) | ((u32)ex + 128u) | ((u32)en + 128u)) > 255u) {
+      if (e4_longer<1>(d0)) leaf16 |= 1u << (15 - 4 * b);
+      if (e4_longer<1>(d1)) leaf16 |= 1u << (14 - 4 * b);
+      if (e4_longer<1>(d2)) leaf16 |= 1u << (13 - 4 * b);
+      if (e4_longer<1>(d3)) leaf16 |= 1u << (12 - 4 * b);
+      if (e4_longer<1>(ex)) qx |= 1u << (3 - b);
+      if (e4_longer<1>(en)) qn |= 1u << (3 - b);
+      // not eligible (a forced Snapshot's image may be stale: nothing to check)
+      if (!forced && (((u32)d0 + 32768u) | ((u32)d1 + 32768u) | ((u32)d2 + 32768u) | ((u32)d3 + 32768u)) > 65535u) err |= EF_BAD_FORMAT;
+      leafw = e5_pack4(zigzag32(d0), zigzag32(d1), zigzag32(d2), zigzag32(d3));
+      ovx |= (zigzag32(ex) & 0xffu) << (8 * b);
+      ovn |= (zigzag32(en) & 0xffu) << (8 * b);
+      ovm |= 0xffu << (8 * b);
+    }
+    leaf[b * TT] = leafw;
+    amax = max(amax, qmax); amin = min(amin, qmin);
+    if (b == 0) dfirst = d0;
+    aeq = aeq && e5 && d0 == dfirst;
+  }
+  R.zxw = (e5_zz4(exw) & ~ovm) | ovx; R.znw = (e5_zz4(enw) & ~ovm) | ovn;
+  R.u5n = u5n; R.e5n = e5n; R.leaf16 = leaf16; R.qx = qx; R.qn = qn;
+  R.amax = amax; R.amin = amin; R.dfirst = dfirst; R.aeq = aeq;
+}
+// ... on packed cells (PK; tw / sw: the instant's and the snapshot's words).  false: some entry lies outside -128..127,
+// and R is not complete (the caller unpacks and takes e5_log_node, which rewrites the leaf words too)
+template <int TT>
+DCDF_DEVINL bool e5_log_packed(const uint4 (&tw)[2], const uint4 (&sw)[2], u32* leaf, int fmin, E5LogNode& R) {
+  u32 acc = 0u, mx[2], mn[2], ex[2], en[2], eqw[2], unw[2], d0[2];
+#pragma unroll
+  for (int h = 0; h < 2; h++) {
+    const uint4 t = tw[h], s = sw[h];
+    // leaf differences + 128, quads 2h (bits 15..0) and 2h + 1 (bits 31..16)
+    const u32 dx = t.x - s.x + 0x00800080u, dy = t.y - s.y + 0x00800080u, dz = t.z - s.z + 0x00800080u, dw = t.w - s.w + 0x00800080u;
+    const u32 xt = __vimax3_u16x2(t.x, t.y, __vmaxu2(t.z, t.w)), nt = __vimin3_u16x2(t.x, t.y, __vminu2(t.z, t.w));
+    const u32 xs = __vimax3_u16x2(s.x, s.y, __vmaxu2(s.z, s.w)), ns = __vimin3_u16x2(s.x, s.y, __vminu2(s.z, s.w));
+    ex[h] = xt - xs + 0x00800080u; en[h] = nt - ns + 0x00800080u;
+    acc |= dx | dy | dz | dw | ex[h] | en[h];
+    eqw[h] = __vminu2((dx ^ dy) | (dx ^ dz) | (dx ^ dw), 0x00010001u);  // 0: the quad's four differences are equal
+    unw[h] = __vminu2(xt ^ nt, 0x00010001u);                           // 0: the quad is uniform
+    const u32 a = e5_zz4_off(__byte_perm(dx, dy, 0x6240)), b = e5_zz4_off(__byte_perm(dz, dw, 0x6240));
+    leaf[2 * h * TT] = __byte_perm(a, b, 0x5410);
+    leaf[(2 * h + 1) * TT] = __byte_perm(a, b, 0x7632);
+    mx[h] = xt; mn[h] = nt; d0[h] = dx;
+  }
+  R.u5n = 0xfu & ~e5_bits4(e5_lo_bytes(unw[0], unw[1]));
+  R.e5n = 0xfu & ~e5_bits4(e5_lo_bytes(eqw[0], eqw[1]));
+  R.leaf16 = 0u; R.qx = 0u; R.qn = 0u;
+  R.zxw = e5_zz4_off(e5_lo_bytes(ex[0], ex[1]));
+  R.znw = e5_zz4_off(e5_lo_bytes(en[0], en[1]));
+  const u32 m = __vmaxu2(mx[0], mx[1]), k = __vminu2(mn[0], mn[1]);
+  R.err = 0u;
+  R.amax = fmin + (int)max(m & 0xffffu, m >> 16);
+  R.amin = fmin + (int)min(k & 0xffffu, k >> 16);
+  R.dfirst = (int)(d0[0] & 0xffffu) - 128;
+  R.aeq = (eqw[0] | eqw[1] | (d0[0] ^ d0[1]) | (d0[0] ^ __byte_perm(d0[0], 0u, 0x1032))) == 0u;
+  return (acc & 0xff00ff00u) == 0u;
+}
+// ... the rare case of e5_log_packed, out of line: e5_log_node on the unpacked codes
+template <int TT>
+__device__ __noinline__ E5LogNode e5_log_unpacked(uint4 t0, uint4 t1, uint4 s0, uint4 s1, u32* leaf, int fmin, bool forced) {
+  int4 q[4], sq[4];
+#pragma unroll
+  for (int b = 0; b < 4; b++) {
+    q[b] = e5_unpack_quad(b < 2 ? t0 : t1, b, fmin);
+    sq[b] = e5_unpack_quad(b < 2 ? s0 : s1, b, fmin);
+  }
+  E5LogNode R;
+  R.err = 0u;
+  e5_log_node<true, TT>(q, [&](int b) { return sq[b]; }, leaf, forced, R.err, R);
+  return R;
+}
+
 // ALIGNED: the staged image is shifted so that every group of four sibling entries starts on a word (the caller knows)
 template <bool ALIGNED = false>
 DCDF_DEVINL void e5_store_word(u8* p, u32 w) {
@@ -267,9 +439,9 @@ DCDF_DEVINL void e5_store_word(u8* p, u32 w) {
 // quads, then the four quad max entries, then the min entries of the internal quads -- the order in which their second
 // bytes sit in DAC level 1 (dac.rs:109-121).  Log: cells of the instant come from a second (L2-resident) read of the
 // node, the snapshot's from shared memory.  Snapshot: the emission pass has just stored the cells in shared memory.
-// scell: the node's quad 0 in E5SmemT::cell, whose quads lie TT apart
-template <bool FULL, int TT = E5_THREADS>
-__device__ __noinline__ void e5_long_node(bool as_snapshot, const float* pn, i64 sr, float scale2, const int4* scell, int2 n4, u32 in5a,
+// scell: the node's first entry in E5SmemT::cell (e5_snap_quad)
+template <bool FULL, int TT, bool PK>
+__device__ __noinline__ void e5_long_node(bool as_snapshot, const float* pn, i64 sr, float scale2, const void* scell, int fmin, int2 n4, u32 in5a,
                                           u8* xb1, u8* nb1, u32* pos /* lx1, rx1, rn1 */, int rl, int cl, int vec) {
   int4 q[4];
   if (!as_snapshot) {
@@ -281,7 +453,7 @@ __device__ __noinline__ void e5_long_node(bool as_snapshot, const float* pn, i64
   u32 zx[4], zn[4];
 #pragma unroll
   for (int b = 0; b < 4; b++) {
-    const int4 s = scell[b * TT];
+    const int4 s = e5_snap_quad<PK, TT>(scell, b, fmin);
     const int4 t = as_snapshot ? s : q[b];
     int qmax, qmin, sqmax, sqmin;
     e4_qmm<FULL>(t, qmax, qmin);
@@ -307,15 +479,14 @@ __device__ __noinline__ void e5_long_node(bool as_snapshot, const float* pn, i64
 }
 
 // Snapshot entries of one level-4 node that take two bytes (snapshot.rs:122-147: quad max - cell, node max - quad max,
-// quad min - node min), cell by cell from a second (L2-resident) read of the node: leaves (bits 15..0, cell m of the node
-// = bit 15 - m), quad max entries (bits 19..16, quad b = bit 19 - b), quad min entries (bits 23..20).  Rare: only for
-// nodes whose range does not prove every entry short, and for nodes the raster's edge cuts through
+// quad min - node min), cell by cell: leaves (bits 15..0, cell m of the node = bit 15 - m), quad max entries (bits
+// 19..16, quad b = bit 19 - b), quad min entries (bits 23..20).  Nodes the raster's edge cuts through take them from the
+// cells the fused pass holds in registers; nodes whose range does not prove every entry short (rare) from a second
+// (L2-resident) read of the node (e5_snap_long)
+// ... from the node's quads q0..q3 (e5_quads)
 template <bool FULL>
-__device__ __noinline__ u32 e5_snap_long(const float* pn, i64 sr, float scale2, int rl, int cl, int vec) {
-  uint4 raw[4];
-  int4 q[4];
-  e5_load_node<FULL>(pn, sr, raw, rl, cl, vec);
-  e5_quads<FULL>(raw, scale2, q, rl, cl);
+DCDF_DEVINL u32 e5_snap_cells(int4 q0, int4 q1, int4 q2, int4 q3) {
+  const int4 q[4] = {q0, q1, q2, q3};
   int qmax[4], qmin[4];
 #pragma unroll
   for (int b = 0; b < 4; b++) e4_qmm<FULL>(q[b], qmax[b], qmin[b]);
@@ -332,6 +503,14 @@ __device__ __noinline__ u32 e5_snap_long(const float* pn, i64 sr, float scale2, 
     if (e4_longer<1>(e5_dn(qmin[b], amin))) m |= 1u << (23 - b);
   }
   return m;
+}
+template <bool FULL>
+__device__ __noinline__ u32 e5_snap_long(const float* pn, i64 sr, float scale2, int rl, int cl, int vec) {
+  uint4 raw[4];
+  int4 q[4];
+  e5_load_node<FULL>(pn, sr, raw, rl, cl, vec);
+  e5_quads<FULL>(raw, scale2, q, rl, cl);
+  return e5_snap_cells<FULL>(q[0], q[1], q[2], q[3]);
 }
 
 // mbarrier + bulk copy (the TMA unit's 1-D form) for the BULK variant of the kernel
@@ -395,7 +574,8 @@ template <int G, bool FULL, bool BULK, int NW>
 DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sync_mask) {
   static_assert(NW == 2 || (NW == 1 && !FULL && !BULK), "one-warp tiles are clipped edge tiles");
   constexpr int TT = 32 * NW;  // threads per tile
-  using Smem = std::conditional_t<NW == 2, E5Smem, E5SmemEdge>;
+  using Smem = std::conditional_t<NW == 2, E5Smem<FULL>, E5SmemEdge>;
+  constexpr bool PK = FULL;  // 16-bit packed cells (e5_pack_node)
   // every row of four cells is 16-byte aligned -> 128-bit loads; BULK (host checked the alignment): loads from the staged tile
   const int vec = BULK ? 2 : (((P.stride_r | P.stride_t) & 3) == 0 && (((uintptr_t)P.data) & 15) == 0) ? 1 : 0;
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -421,6 +601,7 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
   // the thread's level-3 node (NW = 1: the top half of the tree when the unit has at most 32 rows, else the left half)
   const int node = NW == 2 ? tid : unit.rows <= 32 ? lane : lane < 16 ? lane : lane + 16;
   const float scale2 = (float)((i64)2 << unit.bits);
+  const float cmag = (float)(12582912 + 1 - unit.fmin);  // PK: e5_conv_rel
   const i64 sr = BULK ? 64 : P.stride_r;
   // the thread's 8x8 block
   const float* const base = BULK ? SB.raw + (8 * (int)morton_row(tid)) * 64 + 8 * (int)morton_col(tid)
@@ -451,7 +632,7 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
     uint4* z = reinterpret_cast<uint4*>(S.pool);
     for (int i = tid; i < (int)(sizeof(S.pool) / 16); i += TT) z[i] = make_uint4(0, 0, 0, 0);
   }
-  if (!FULL) {  // cells outside the raster are None in the snapshot image from the start
+  if constexpr (!FULL) {  // cells outside the raster are None in the snapshot image from the start
     for (int q = 0; q < 16; q++) S.cell[q][tid] = make_int4(E4_NONE, E4_NONE, E4_NONE, E4_NONE);
     for (int a = 0; a < 4; a++) S.l4s[a][tid] = make_int2(E4_NONE, INT32_MAX);
   }
@@ -470,6 +651,7 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
   u32 err = 0;
   int s3max = 0, s3min = 0, s2max = 0, s2min = 0, s1max = 0, s1min = 0, s0max = 0, s0min = 0;
   u32 n_logs = 0, n_snap = 0, n_log_total = 0;
+  int simg = 0;  // PK: which of S.cell's images is the snapshot
   u64 total_bytes = 0;
 
 #pragma unroll 1
@@ -516,57 +698,38 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
       eq3 = true;
 #pragma unroll 1
       for (int a = 0; a < 4; a++) {
-        int4 q[4];
-        e5_quads<FULL>(raw, scale2, q, E5_RL(a), E5_CL(a));
-        if (a < 3) e5_load_node<FULL>(e5_node_ptr(pt, sr, a + 1), sr, raw, E5_RL(a + 1), E5_CL(a + 1), vec);
-        const int2 s4 = S.l4s[a][tid];
-        int amax = INT32_MIN, amin = INT32_MAX, dfirst = 0;
-        bool aeq = true;
-        u32 leaf16 = 0, u5n = 0, e5n = 0, qx = 0, qn = 0;
-        u32 exw = 0, enw = 0;          // low bytes of the four quad max / min entries
-        u32 ovx = 0, ovn = 0, ovm = 0; // exact low bytes of the zigzag codes of entries outside -128..127
-#pragma unroll
-        for (int b = 0; b < 4; b++) {
-          const int4 t = q[b], sq = S.cell[4 * a + b][tid];
-          int qmax, qmin, sqmax, sqmin;
-          e4_qmm<FULL>(t, qmax, qmin);
-          e4_qmm<FULL>(sq, sqmax, sqmin);
-          const int d0 = e4_sub(t.x, sq.x), d1 = e4_sub(t.y, sq.y), d2 = e4_sub(t.z, sq.z), d3 = e4_sub(t.w, sq.w);  // None - None = 0 (log.rs:751)
-          const int ex = e5_dx<FULL>(qmax, sqmax), en = e5_dn(qmin, sqmin);
-          const bool e5 = (((d1 ^ d0) | (d2 ^ d0) | (d3 ^ d0)) == 0);  // all four leaf diffs equal (log.rs:780-806)
-          if (e4_unif<FULL>(qmax, qmin)) u5n |= 1u << (3 - b);
-          if (e5) e5n |= 1u << (3 - b);
-          u32 leafw = e5_zz4(e5_low4(d0, d1, d2, d3));
-          exw = __byte_perm(exw, (u32)ex, b == 0 ? 0x3214 : b == 1 ? 0x3240 : b == 2 ? 0x3410 : 0x4210);
-          enw = __byte_perm(enw, (u32)en, b == 0 ? 0x3214 : b == 1 ? 0x3240 : b == 2 ? 0x3410 : 0x4210);
-          // one test for "some entry of this quad needs two bytes" (zigzag code above 255  <=>  value outside -128..127)
-          if ((((u32)d0 + 128u) | ((u32)d1 + 128u) | ((u32)d2 + 128u) | ((u32)d3 + 128u) | ((u32)ex + 128u) | ((u32)en + 128u)) > 255u) {
-            if (e4_longer<1>(d0)) leaf16 |= 1u << (15 - 4 * b);
-            if (e4_longer<1>(d1)) leaf16 |= 1u << (14 - 4 * b);
-            if (e4_longer<1>(d2)) leaf16 |= 1u << (13 - 4 * b);
-            if (e4_longer<1>(d3)) leaf16 |= 1u << (12 - 4 * b);
-            if (e4_longer<1>(ex)) qx |= 1u << (3 - b);
-            if (e4_longer<1>(en)) qn |= 1u << (3 - b);
-            // not eligible (a forced Snapshot's image may be stale: nothing to check)
-            if (!forced && (((u32)d0 + 32768u) | ((u32)d1 + 32768u) | ((u32)d2 + 32768u) | ((u32)d3 + 32768u)) > 65535u) err |= EF_BAD_FORMAT;
-            leafw = e5_pack4(zigzag32(d0), zigzag32(d1), zigzag32(d2), zigzag32(d3));
-            ovx |= (zigzag32(ex) & 0xffu) << (8 * b);
-            ovn |= (zigzag32(en) & 0xffu) << (8 * b);
-            ovm |= 0xffu << (8 * b);
-          }
-          S.leaf[4 * a + b][tid] = leafw;
-          amax = max(amax, qmax); amin = min(amin, qmin);
-          if (b == 0) dfirst = d0;
-          aeq = aeq && e5 && d0 == dfirst;
+        int2 s4;
+        u32 mcut = 0;  // clipped tiles: the Snapshot's two-byte masks of a node the raster's edge cuts (e5_snap_cells)
+        E5LogNode R;
+        u32* const leaf = &S.leaf[4 * a][tid];
+        if constexpr (PK) {
+          uint4 tw[2];
+          e5_pack_node(raw, scale2, cmag, unit.fmin, tw, err);
+          if (a < 3) e5_load_node<FULL>(e5_node_ptr(pt, sr, a + 1), sr, raw, E5_RL(a + 1), E5_CL(a + 1), vec);
+          s4 = S.l4s[a][tid];
+          S.cell[simg ^ 1][2 * a][tid] = tw[0];  // the instant's image: the snapshot image if a Snapshot wins
+          S.cell[simg ^ 1][2 * a + 1][tid] = tw[1];
+          const uint4 sw[2] = {S.cell[simg][2 * a][tid], S.cell[simg][2 * a + 1][tid]};
+          if (!e5_log_packed<TT>(tw, sw, leaf, unit.fmin, R))  // some entry takes two bytes (rare): cell by cell
+            R = e5_log_unpacked<TT>(tw[0], tw[1], sw[0], sw[1], leaf, unit.fmin, forced);
+          err |= R.err;
+        } else {
+          int4 q[4];
+          e5_quads<FULL>(raw, scale2, q, E5_RL(a), E5_CL(a));
+          if (a < 3) e5_load_node<FULL>(e5_node_ptr(pt, sr, a + 1), sr, raw, E5_RL(a + 1), E5_CL(a + 1), vec);
+          s4 = S.l4s[a][tid];
+          if (!FULL && E5_RL(a) > 0 && E5_CL(a) > 0 && (E5_RL(a) < 4 || E5_CL(a) < 4)) mcut = e5_snap_cells<FULL>(q[0], q[1], q[2], q[3]);
+          e5_log_node<FULL, TT>(q, [&](int b) { return S.cell[4 * a + b][tid]; }, leaf, forced, err, R);
         }
-        const u32 zxw = (e5_zz4(exw) & ~ovm) | ovx, znw = (e5_zz4(enw) & ~ovm) | ovn;
-        S.qx[a][tid] = zxw;
-        S.qn[a][tid] = znw;
+        const int amax = R.amax, amin = R.amin, dfirst = R.dfirst;
+        const bool aeq = R.aeq;
+        S.qx[a][tid] = R.zxw;
+        S.qn[a][tid] = R.znw;
         S.l4t[a][tid] = make_int2(amax, amin);
-        L.ml |= (u64)leaf16 << (48 - 16 * a);
-        L.mq |= (qx << (12 - 4 * a)) | (qn << (28 - 4 * a));
-        u5 |= u5n << (12 - 4 * a);
-        eq5 |= e5n << (12 - 4 * a);
+        L.ml |= (u64)R.leaf16 << (48 - 16 * a);
+        L.mq |= (R.qx << (12 - 4 * a)) | (R.qn << (28 - 4 * a));
+        u5 |= R.u5n << (12 - 4 * a);
+        eq5 |= R.e5n << (12 - 4 * a);
         if (e4_unif<FULL>(amax, amin)) u4 |= 1u << (3 - a);
         if (aeq) eq4 |= 1u << (3 - a);
         if (e4_longer<1>(e5_dx<FULL>(amax, s4.x))) L.mu |= 1u << (3 - a);
@@ -576,12 +739,12 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
         eq3 = eq3 && aeq && dfirst == diff3;
         // ---------------- Snapshot entries of levels 6 and 5 (snapshot.rs:122-147): every one lies in 0 .. amax - amin,
         // so one test per node proves them all short.  Clipped tiles: a cell outside the raster counts as 0, so a node
-        // the raster's edge cuts through takes the exact path; a node wholly outside has nothing but zero entries
+        // the raster's edge cuts through takes the exact masks (mcut); a node wholly outside has nothing but zero entries
         {
           const int rl = E5_RL(a), cl = E5_CL(a);
           const bool inside = FULL || (rl >= 4 && cl >= 4), outside = !FULL && (rl <= 0 || cl <= 0);
           if (!outside && (!inside || (u32)(amax - amin) > 127u)) {
-            const u32 m = e5_snap_long<FULL>(e5_node_ptr(pt, sr, a), sr, scale2, rl, cl, vec);
+            const u32 m = inside ? e5_snap_long<FULL>(e5_node_ptr(pt, sr, a), sr, scale2, rl, cl, vec) : mcut;
             C.ml |= (u64)(m & 0xffffu) << (48 - 16 * a);
             C.mq |= (((m >> 16) & 0xfu) << (12 - 4 * a)) | ((m >> 20) << (28 - 4 * a));
           }
@@ -896,7 +1059,7 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
       u8* dst5 = xb0 + Pn5 + 4u * R4;
       u8* dmn = nb0 + Mn5 + R5;
       uint4 raw[4];
-      if (as_snapshot) e5_load_node<FULL>(e5_node_ptr(pt, sr, 0), sr, raw, E5_RL(0), E5_CL(0), vec);
+      if (!PK && as_snapshot) e5_load_node<FULL>(e5_node_ptr(pt, sr, 0), sr, raw, E5_RL(0), E5_CL(0), vec);
 #pragma unroll 1
       for (int a = 0; a < 4; a++) {
         const int2 n4 = S.l4t[a][tid];
@@ -906,10 +1069,32 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
         if (as_snapshot) {
           // quads and leaves of the Snapshot from a pass over the tile, which also installs the instant as the snapshot
           // image the following Logs are built against (even when nothing can be emitted: the sizes must stay exact)
+          S.l4s[a][tid] = n4;
+          if constexpr (PK) {
+            // the cells come from the image the fused pass wrote.  Every entry is a non-negative difference of two codes
+            // (quad max - cell, node max - quad max, quad min - node min): its zigzag code is twice it, whose low byte
+            // is twice the low byte
+            const uint4 tw[2] = {S.cell[simg ^ 1][2 * a][tid], S.cell[simg ^ 1][2 * a + 1][tid]};
+            const u32 nx = (u32)(n4.x - unit.fmin) * 0x00010001u, nn = (u32)(n4.y - unit.fmin) * 0x00010001u;
+            u32 vx[2], vn[2];
+#pragma unroll
+            for (int h = 0; h < 2; h++) {
+              const uint4 t = tw[h];
+              const u32 xt = __vimax3_u16x2(t.x, t.y, __vmaxu2(t.z, t.w)), nt = __vimin3_u16x2(t.x, t.y, __vminu2(t.z, t.w));
+              vx[h] = nx - xt; vn[h] = nt - nn;
+              u32 lu = __byte_perm(xt - t.x, xt - t.y, 0x6240), ll = __byte_perm(xt - t.z, xt - t.w, 0x6240);
+              lu = (lu + lu) & 0xfefefefeu; ll = (ll + ll) & 0xfefefefeu;
+              if (alive && ((in5a >> (3 - 2 * h)) & 1u))
+                e5_store_word<decltype(in_shared)::value>(dst6 + 4u * (u32)__popc(in5a >> (4 - 2 * h)), __byte_perm(lu, ll, 0x5410));
+              if (alive && ((in5a >> (2 - 2 * h)) & 1u))
+                e5_store_word<decltype(in_shared)::value>(dst6 + 4u * (u32)__popc(in5a >> (3 - 2 * h)), __byte_perm(lu, ll, 0x7632));
+            }
+            zxw = e5_lo_bytes(vx[0], vx[1]); zxw = (zxw + zxw) & 0xfefefefeu;
+            znw = e5_lo_bytes(vn[0], vn[1]); znw = (znw + znw) & 0xfefefefeu;
+          } else {
           int4 q[4];
           e5_quads<FULL>(raw, scale2, q, E5_RL(a), E5_CL(a));
           if (a < 3) e5_load_node<FULL>(e5_node_ptr(pt, sr, a + 1), sr, raw, E5_RL(a + 1), E5_CL(a + 1), vec);
-          S.l4s[a][tid] = n4;
           zxw = 0; znw = 0;
 #pragma unroll
           for (int b = 0; b < 4; b++) {
@@ -923,6 +1108,7 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
               e5_store_word<decltype(in_shared)::value>(dst6 + 4u * (u32)__popc(in5a >> (4 - b)),
                             e5_pack4(zigzag32(e5_dx<FULL>(qmax, t.x)), zigzag32(e5_dx<FULL>(qmax, t.y)), zigzag32(e5_dx<FULL>(qmax, t.z)),
                                      zigzag32(e5_dx<FULL>(qmax, t.w))));
+          }
           }
         } else {
           // quads and leaves of the Log from the payload of the fused pass
@@ -942,8 +1128,13 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
           if ((in5a >> (3 - b)) & 1u) *dmn++ = (u8)(znw >> (8 * b));
         const u32 ml16 = (u32)(W.ml >> (48 - 16 * a)) & 0xffffu;
         const u32 lq = ((W.mq >> (12 - 4 * a)) & 0xfu) | (((W.mq >> (28 - 4 * a)) & 0xfu) & in5a);
-        if ((ml16 & (e4_expand4(in5a) & 0xffffu)) | lq)
-          e5_long_node<FULL, TT>(as_snapshot, e5_node_ptr(pt, sr, a), sr, scale2, &S.cell[4 * a][tid], n4, in5a, xb1, nb1, pos, E5_RL(a), E5_CL(a), vec);
+        if ((ml16 & (e4_expand4(in5a) & 0xffffu)) | lq) {
+          const void* scell;  // Log: the snapshot's cells; Snapshot: the instant's
+          if constexpr (PK) scell = &S.cell[as_snapshot ? simg ^ 1 : simg][2 * a][tid];
+          else scell = &S.cell[4 * a][tid];
+          e5_long_node<FULL, TT, PK>(as_snapshot, e5_node_ptr(pt, sr, a), sr, scale2, scell, PK ? unit.fmin : 0, n4, in5a, xb1, nb1, pos, E5_RL(a),
+                                     E5_CL(a), vec);
+        }
       }
     }
     if (emit) {
@@ -1083,6 +1274,7 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
       s3max = t3max; s3min = t3min; s2max = t2max; s2min = t2min; s1max = t1max; s1min = t1min; s0max = t0max; s0min = t0min;
       n_snap++;
       n_logs = 0;
+      simg ^= 1;  // PK: the instant's image is the snapshot from here on
       total_bytes += 1;  // Block's n_instants byte (block.rs:88-95)
     } else {
       n_logs++;

@@ -1005,6 +1005,7 @@ __global__ void __launch_bounds__(256) k_finalize_tree(const TreeParams P, u32 n
         // k_encode_v5 (encode_v5.cuh): f32 tiles with a 64-side tree whose to_fixed is exact, every fixed value below
         // 2^22 in magnitude and all of them within 32767 of each other -> every entry below the root takes <= 2 bytes
         bool fast = false;
+        unit.fmin = 0;
         if (P.allow_fast && !can_elide && unit.lo == 0 && narrow && P.encoding == 32 && (flags & UF_EXACT) && has) {
           const double sc = ldexp(1.0, cbits + 1);
           // fixed = 2 v 2^bits + 1 for values, 0 for NaN: every code of the unit within 32767 of every other one
@@ -1013,6 +1014,7 @@ __global__ void __launch_bounds__(256) k_finalize_tree(const TreeParams P, u32 n
           fast = hi - lo <= 32767.0 && fabs(hi) < 4194303.0 && fabs(lo) < 4194303.0;
           // clipped tiles: an entry next to a cell outside the raster is the max itself (snapshot.rs:122-130 with None => 0)
           if (!full) fast = fast && fabs(hi) <= 32767.0 && fabs(lo) <= 32767.0;
+          unit.fmin = (int)lo;  // exact: codes are integers below 2^22 in magnitude
         }
         unit.bits = cbits;
         unit.flags = flags;
