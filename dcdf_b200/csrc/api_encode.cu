@@ -140,8 +140,8 @@ void launch_encode_one(dcdf_ctx* ctx, const EncParams& P, u32 grid) {
   ctx->launches++;
 }
 // Full 64x64 tiles with 31-bit values: 64-thread CTAs, 64 cells per thread (encode_v4.cuh).
-// Option "encode_tiles256" routes them through k_encode_tiles instead; option "stage_limit" lowers the size above
-// which a structure is emitted straight into the arena (tests use it to cover that path).
+// Option "stage_limit" lowers the size above which a structure is emitted straight into the arena (tests use it to
+// cover that path).
 template <typename InT, bool FULL>
 void launch_encode_v4(dcdf_ctx* ctx, const EncParams& P, u32 grid) {
   constexpr int MINB = 4;
@@ -153,27 +153,13 @@ void launch_encode_v4(dcdf_ctx* ctx, const EncParams& P, u32 grid) {
   ctx->launches++;
 }
 // Full f32 tiles that qualify for the small fast-path kernel (encode_v5.cuh; list 5, filled by k_finalize_tree).
-// Measurement variants (ctx option fast_variant): 1 = four tiles per CTA, 2 = four tiles per CTA with the instant's tile
-// staged in shared memory by bulk copies behind an mbarrier (the TMA unit's 1-D form).
-template <int G, bool BULK>
-void launch_encode_v5_variant(dcdf_ctx* ctx, const EncParams& P, u32 grid) {
-  const u32 stage_limit = std::min<u32>(ctx->opt.stage_limit, (u32)E5_POOL);
-  const size_t smem = (sizeof(E5Smem<true>) + (BULK ? sizeof(E5Bulk) : 0)) * G;
-  CK(cudaFuncSetAttribute(k_encode_v5<G, true, BULK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  k_encode_v5<G, true, BULK><<<(grid + G - 1) / G, E5_THREADS * G, smem, ctx->stream>>>(P, stage_limit, ctx->opt.fast_sync_mask);
-  CK(cudaGetLastError());
-  ctx->launches++;
-}
 template <bool FULL>
 void launch_encode_v5(dcdf_ctx* ctx, const EncParams& P, u32 grid) {
   constexpr int G = 6;  // tiles per CTA, one CTA per SM
-  if (FULL && ctx->opt.fast_variant == 1) return launch_encode_v5_variant<4, false>(ctx, P, grid);
-  if (FULL && ctx->opt.fast_variant == 2 && ((P.stride_r | P.stride_t) & 3) == 0 && (((uintptr_t)P.data + 4 * 0) & 15) == 0)
-    return launch_encode_v5_variant<4, true>(ctx, P, grid);
   const u32 stage_limit = std::min<u32>(ctx->opt.stage_limit, (u32)E5_POOL);
   const size_t smem = sizeof(E5Smem<FULL>) * G;
   CK(cudaFuncSetAttribute(k_encode_v5<G, FULL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  k_encode_v5<G, FULL><<<(grid + G - 1) / G, E5_THREADS * G, smem, FULL ? ctx->stream : ctx->aux_stream>>>(P, stage_limit, ctx->opt.fast_sync_mask);
+  k_encode_v5<G, FULL><<<(grid + G - 1) / G, E5_THREADS * G, smem, FULL ? ctx->stream : ctx->aux_stream>>>(P, stage_limit, E5_SYNC_MASK);
   CK(cudaGetLastError());
   ctx->launches++;
 }
@@ -185,7 +171,7 @@ void launch_encode_v5_edge(dcdf_ctx* ctx, const EncParams& P, u32 grid) {
   const u32 stage_limit = std::min<u32>(ctx->opt.stage_limit, (u32)E5_POOL_EDGE);
   const size_t smem = sizeof(E5SmemEdge) * G;
   CK(cudaFuncSetAttribute(k_encode_v5_edge<G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  k_encode_v5_edge<G><<<(grid + G - 1) / G, 32 * G, smem, ctx->aux_stream>>>(P, stage_limit, ctx->opt.fast_sync_mask);
+  k_encode_v5_edge<G><<<(grid + G - 1) / G, 32 * G, smem, ctx->aux_stream>>>(P, stage_limit, E5_SYNC_MASK);
   CK(cudaGetLastError());
   ctx->launches++;
 }
@@ -202,12 +188,10 @@ void launch_encode(dcdf_ctx* ctx, const EncParams& P, u32 grid, int list) {
     }
     return;
   }
-  const bool force_v2 = ctx->opt.encode_tiles256 != 0;
-  if (list == 0 && !force_v2) { launch_encode_v4<InT, true>(ctx, P, grid); return; }
-  if (list == 4 && !force_v2) { launch_encode_v4<InT, false>(ctx, P, grid); return; }
+  if (list == 0) { launch_encode_v4<InT, true>(ctx, P, grid); return; }
+  if (list == 4) { launch_encode_v4<InT, false>(ctx, P, grid); return; }
   switch (list) {
-    case 0: launch_encode_one<InT, int32_t, true, 2>(ctx, P, grid); break;
-    case 1: case 4: launch_encode_one<InT, int32_t, false, 2>(ctx, P, grid); break;
+    case 1: launch_encode_one<InT, int32_t, false, 2>(ctx, P, grid); break;
     case 2: launch_encode_one<InT, i64, true, 1>(ctx, P, grid); break;
     default: launch_encode_one<InT, i64, false, 1>(ctx, P, grid); break;
   }
@@ -901,10 +885,7 @@ int32_t dcdf_ctx_set_option(dcdf_ctx* ctx, const char* name, int64_t value) {
   const std::string n(name);
   if (n == "stage_limit") ctx->opt.stage_limit = value < 0 ? 0xffffffffu : (uint32_t)std::min<int64_t>(value, 0xffffffffll);
   else if (n == "arena_hint") ctx->arena_hint = value < 0 ? 0 : (size_t)value;
-  else if (n == "encode_tiles256") ctx->opt.encode_tiles256 = value != 0;
   else if (n == "no_fast_encode") ctx->opt.no_fast_encode = value != 0;
-  else if (n == "fast_sync_mask") ctx->opt.fast_sync_mask = (int)value;
-  else if (n == "fast_variant") ctx->opt.fast_variant = (int)value;
   else if (n == "search_share_min") ctx->opt.search_share_min = (uint32_t)std::max<int64_t>(value, 0);
   else if (n == "cell_tile_min") ctx->opt.cell_tile_min = (uint32_t)std::max<int64_t>(value, 0);
   else if (n == "window_cells") ctx->opt.window_cells = value != 0;

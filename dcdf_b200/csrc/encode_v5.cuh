@@ -190,10 +190,7 @@ DCDF_DEVINL void e5_load_node(const float* pn, i64 sr, uint4 (&raw)[4], int rl, 
   for (int r = 0; r < 4; r++) {
     if (FULL || (r < rl && cl >= 4)) {
       const float* pr = pn + (i64)r * sr;
-      if (vec == 2) {  // the instant's tile sits in shared memory (bulk-copy variant)
-        asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(raw[r].x), "=r"(raw[r].y), "=r"(raw[r].z), "=r"(raw[r].w)
-                     : "r"((u32)__cvta_generic_to_shared(pr)));
-      } else if (vec) {
+      if (vec) {
         raw[r] = __ldg(reinterpret_cast<const uint4*>(pr));
       } else {  // rows that are not 16-byte aligned (e.g. 1405 columns): four 32-bit loads
         raw[r] = make_uint4(__float_as_uint(__ldg(pr)), __float_as_uint(__ldg(pr + 1)), __float_as_uint(__ldg(pr + 2)), __float_as_uint(__ldg(pr + 3)));
@@ -513,35 +510,6 @@ __device__ __noinline__ u32 e5_snap_long(const float* pn, i64 sr, float scale2, 
   return e5_snap_cells<FULL>(q[0], q[1], q[2], q[3]);
 }
 
-// mbarrier + bulk copy (the TMA unit's 1-D form) for the BULK variant of the kernel
-DCDF_DEVINL u32 e5_smem_u32(const void* p) { return (u32)__cvta_generic_to_shared(p); }
-DCDF_DEVINL void e5_mbar_init(unsigned long long* b, u32 count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(e5_smem_u32(b)), "r"(count) : "memory");
-}
-DCDF_DEVINL void e5_mbar_expect_tx(unsigned long long* b, u32 bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(e5_smem_u32(b)), "r"(bytes) : "memory");
-}
-DCDF_DEVINL void e5_mbar_wait(unsigned long long* b, u32 parity) {
-  asm volatile(
-      "{\n\t.reg .pred P1;\n\t"
-      "E5_WAIT:\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 P1, [%0], %1;\n\t"
-      "@P1 bra E5_DONE;\n\t"
-      "bra E5_WAIT;\n\t"
-      "E5_DONE:\n\t}" ::"r"(e5_smem_u32(b)), "r"(parity) : "memory");
-}
-DCDF_DEVINL void e5_bulk_g2s(void* smem, const void* g, u32 bytes, unsigned long long* b) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(e5_smem_u32(smem)),
-               "l"(g), "r"(bytes), "r"(e5_smem_u32(b))
-               : "memory");
-}
-// BULK variant: the instant's 64x64 f32 tile, row-major, filled by 64 bulk copies (one row each) behind an mbarrier
-struct E5Bulk {
-  __align__(16) float raw[64 * 64];
-  __align__(8) unsigned long long mbar;
-  unsigned long long pad_;
-};
-
 // barrier over the threads of one tile: named barrier 1 + tile slot for a two-warp tile (barrier 0 stays the CTA-wide
 // one), the warp itself for a one-warp tile
 template <int NW>
@@ -560,29 +528,33 @@ DCDF_DEVINL void e5_tile_sync(int slot) {
 // each group of 16 lanes is still one level-1 node.  The missing half is two all-None level-1 nodes; what the NW = 2
 // kernel computes for such a node is a constant: no internal node below it (all its counters are 0), record
 // (None, INT32_MAX, diff 0, equal) and Log entries (0, 0), set once below.
-template <int G, bool FULL, bool BULK, int NW = 2>
+// The tiles of a CTA take the CTA-wide barrier every (E5_SYNC_MASK + 1) instants.  Measured in round 2 on a B200
+// (profiles/prof_v5.py, 704x1408 raster): every instant / every second / every fourth / never = 46.1 / 47.0 / 48.0 / 45.9
+// k tile-instants per ms.  The host passes it as the kernels' sync_mask argument: compiled in as an immediate, it
+// changes k_encode_v5_edge's register allocation (32 / 60 bytes of spill stores / loads instead of 24 / 44) and the
+// kernel takes 5.81 instead of 5.66 ms per C2 build (one B200, 1000 W; profiles/r3_encode_ab_removal.txt)
+constexpr int E5_SYNC_MASK = 3;
+template <int G, bool FULL, int NW = 2>
 DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sync_mask);
-template <int G, bool FULL, bool BULK = false>
+template <int G, bool FULL>
 __global__ void __launch_bounds__(E5_THREADS * G, 1) k_encode_v5(const EncParams P, const u32 stage_limit, const int sync_mask) {
-  e5_body<G, FULL, BULK>(P, stage_limit, sync_mask);
+  e5_body<G, FULL>(P, stage_limit, sync_mask);
 }
 template <int G>
 __global__ void __launch_bounds__(32 * G, 1) k_encode_v5_edge(const EncParams P, const u32 stage_limit, const int sync_mask) {
-  e5_body<G, false, false, 1>(P, stage_limit, sync_mask);
+  e5_body<G, false, 1>(P, stage_limit, sync_mask);
 }
-template <int G, bool FULL, bool BULK, int NW>
+template <int G, bool FULL, int NW>
 DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sync_mask) {
-  static_assert(NW == 2 || (NW == 1 && !FULL && !BULK), "one-warp tiles are clipped edge tiles");
+  static_assert(NW == 2 || (NW == 1 && !FULL), "one-warp tiles are clipped edge tiles");
   constexpr int TT = 32 * NW;  // threads per tile
   using Smem = std::conditional_t<NW == 2, E5Smem<FULL>, E5SmemEdge>;
   constexpr bool PK = FULL;  // 16-bit packed cells (e5_pack_node)
-  // every row of four cells is 16-byte aligned -> 128-bit loads; BULK (host checked the alignment): loads from the staged tile
-  const int vec = BULK ? 2 : (((P.stride_r | P.stride_t) & 3) == 0 && (((uintptr_t)P.data) & 15) == 0) ? 1 : 0;
+  // every row of four cells is 16-byte aligned -> 128-bit loads
+  const int vec = (((P.stride_r | P.stride_t) & 3) == 0 && (((uintptr_t)P.data) & 15) == 0) ? 1 : 0;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int slot = threadIdx.x / TT;
-  constexpr size_t kSlab = sizeof(Smem) + (BULK ? sizeof(E5Bulk) : 0);
-  Smem& S = *reinterpret_cast<Smem*>(smem_raw + (size_t)slot * kSlab);
-  E5Bulk& SB = *reinterpret_cast<E5Bulk*>(smem_raw + (size_t)slot * kSlab + sizeof(Smem));  // only touched when BULK
+  Smem& S = *reinterpret_cast<Smem*>(smem_raw + (size_t)slot * sizeof(Smem));
 
   const u32 n_order = *P.order_count;
   if (blockIdx.x * (u32)G >= n_order) return;
@@ -602,24 +574,9 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
   const int node = NW == 2 ? tid : unit.rows <= 32 ? lane : lane < 16 ? lane : lane + 16;
   const float scale2 = (float)((i64)2 << unit.bits);
   const float cmag = (float)(12582912 + 1 - unit.fmin);  // PK: e5_conv_rel
-  const i64 sr = BULK ? 64 : P.stride_r;
+  const i64 sr = P.stride_r;
   // the thread's 8x8 block
-  const float* const base = BULK ? SB.raw + (8 * (int)morton_row(tid)) * 64 + 8 * (int)morton_col(tid)
-                                 : static_cast<const float*>(P.data) + unit.base + (i64)(8 * (int)morton_row(node)) * sr + 8 * (int)morton_col(node);
-  // BULK: thread r fetches row r of the tile (256 bytes) of one instant
-  const float* const my_row = static_cast<const float*>(P.data) + unit.base + (i64)tid * P.stride_r;
-  auto fetch_instant = [&](int t) {
-    if (tid == 0) e5_mbar_expect_tx(&SB.mbar, 64u * 256u);
-    e5_bulk_g2s(SB.raw + 64 * tid, my_row + (i64)t * P.stride_t, 256u, &SB.mbar);
-  };
-  if (BULK) {
-    if (tid == 0) {
-      e5_mbar_init(&SB.mbar, 1u);
-      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    e5_tile_sync<NW>(slot);
-    if (unit.instants > 0) fetch_instant(0);
-  }
+  const float* const base = static_cast<const float*>(P.data) + unit.base + (i64)(8 * (int)morton_row(node)) * sr + 8 * (int)morton_col(node);
   const bool owner2 = (lane & 3) == 0;
   const bool is1 = (u32)(lane - 1) < 4u;  // lane 1 + k holds level-1 node k at the top of the tree
   const int k1 = node >> 4;  // own level-1 node
@@ -659,9 +616,8 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
     if ((inst & sync_mask) == 0) __syncthreads();  // all tiles of the CTA start the instant together (shared instruction stream)
     if (inst >= unit.instants) continue;
     const bool first = inst == 0;
-    const float* const pt = BULK ? base : base + (i64)inst * P.stride_t;
-    if (BULK) e5_mbar_wait(&SB.mbar, (u32)inst & 1u);  // the instant's tile has landed
-    if (!BULK && inst + 1 < unit.instants) {  // the next instant's cells on their way into L2 (the tiles of a CTA all load at once)
+    const float* const pt = base + (i64)inst * P.stride_t;
+    if (inst + 1 < unit.instants) {  // the next instant's cells on their way into L2 (the tiles of a CTA all load at once)
 #pragma unroll
       for (int r = 0; r < 8; r++)
         if (FULL || (r < rl8 && cl8 > 0)) asm volatile("prefetch.global.L2 [%0];" ::"l"(pt + P.stride_t + (i64)r * sr));
@@ -1204,8 +1160,6 @@ DCDF_DEVINL void e5_body(const EncParams& P, const u32 stage_limit, const int sy
       }
     }
     e5_tile_sync<NW>(slot);  // B2
-    // BULK: nobody reads the staged tile any more -> the next instant's rows start coming in behind the rank directories
-    if (BULK && inst + 1 < unit.instants) fetch_instant(inst + 1);
 
     if (emit) {
       // ================= bitmap headers and rank directories: index[b] = ones in bits [0, 128(b+1))  (bitmap.rs:97-104)

@@ -114,9 +114,6 @@ struct dcdf_ctx {
   struct Options {
     uint32_t stage_limit = 0xffffffffu;  // encoder: structures above this many bytes are emitted straight into the arena
     int no_fast_encode = 0;              // keep eligible tiles away from the fast-path encoder (k_encode_v5)
-    int fast_variant = 0;                // k_encode_v5 A/B launches (api_encode.cu: launch_encode_v5_variant)
-    int fast_sync_mask = 3;              // k_encode_v5: the tiles of a CTA re-align every (mask + 1) instants (measured: 0 / 1 / 3 / never = 46.1 / 47.0 / 48.0 / 45.9 k tile-instants per ms)
-    int encode_tiles256 = 0;             // full tiles through the 256-thread tile encoder instead of the 64-thread one
     uint32_t cell_tile_min = 64;         // cell series: tiles with at least this many series of a batch are decoded by the tile decoder (0: never)
     int window_cells = 0;                // windows through the 4x4-block walker (the path of trees larger than 64x64)
     int window_wide = 0;                 // 64-bit expansion even when every DAC code fits three bytes

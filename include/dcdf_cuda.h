@@ -84,13 +84,11 @@ int32_t dcdf_ctx_destroy(dcdf_ctx* ctx);
 int32_t dcdf_ctx_set_stream(dcdf_ctx* ctx, void* cuda_stream);
 /* Per-context knobs (the reference has no configuration system: all knobs are arguments, SURVEY section 5; these
  * select between code paths that produce identical bytes / results and exist for tests and A/B measurements):
- *   "stage_limit" <bytes>   encoder: structures larger than this are emitted straight into the arena (default 16384)
+ *   "stage_limit" <bytes>   encoder: structures larger than this are emitted straight into the arena (default: no limit
+ *                           below the kernel's own shared-memory image: 16 KB for k_encode_v4, 9 KB for k_encode_v5,
+ *                           5 KB for k_encode_v5_edge; < 0 restores the default)
  *   "arena_hint"  <bytes>   first size of the encoder's output arena (grown and retried when it overflows)
  *   "no_fast_encode" 0|1    eligible full f32 tiles through the general encoder instead of the fast-path kernel
- *   "encode_tiles256" 0|1   full 64x64 tiles through the 256-thread tile encoder
- *   "fast_variant" 0|1|2    fast-path kernel launches for A/B runs: 1 = four tiles per CTA (255 registers), 2 = four tiles
- *                           per CTA with every instant's tile staged in shared memory by bulk copies behind an mbarrier
- *   "fast_sync_mask" <m>    fast-path kernel: the tiles of a CTA re-align every (m + 1) instants (default 3)
  *   "cell_tile_min" <n>     cell series: a tile that at least n series of a batch fall into is decoded once per instant by
  *                           the tile decoder instead of one root-to-leaf walk per (series, instant) (default 64, the measured break-even; 0 = never)
  *   "window_cells" 0|1      windows through the 4x4-block walker k_window_blocks (the path of trees larger than 64x64)

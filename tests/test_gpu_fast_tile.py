@@ -12,22 +12,32 @@ from test_gpu_parity import _check_superchunk
 pytestmark = pytest.mark.gpu
 
 
-@pytest.fixture(scope="module", params=["staged", "direct", "general", "bulk"])
+@pytest.fixture(scope="module", params=["staged", "direct", "general"])
 def ctx(request):
     """staged: default; direct: stage_limit = 0 sends every structure straight into the arena; general: the same
-    inputs through the general encoder (no_fast_encode), which must give the same bytes; bulk: the measurement variant
-    that stages every instant's tile in shared memory with bulk copies behind an mbarrier (fast_variant = 2)."""
+    inputs through the general encoder (no_fast_encode), which must give the same bytes."""
     from dcdf_b200 import Context
     c = Context(0)
     if request.param == "direct":
         c.set_option("stage_limit", 0)
     if request.param == "general":
         c.set_option("no_fast_encode", 1)
-    if request.param == "bulk":
-        c.set_option("fast_variant", 2)
     c.general = request.param == "general"
     yield c
     c.close()
+
+
+def test_removed_encoder_options_are_refused():
+    """fast_variant, fast_sync_mask and encode_tiles256 select no encoder path: set_option refuses them like any unknown
+    name."""
+    from dcdf_b200 import Context, DcdfError
+    c = Context(0)
+    try:
+        for name in ("fast_variant", "fast_sync_mask", "encode_tiles256"):
+            with pytest.raises(DcdfError, match=f"BAD_ARG: unknown option {name}"):
+                c.set_option(name, 1)
+    finally:
+        c.close()
 
 
 def _tiles(frames, bits=4, offset=0.0):

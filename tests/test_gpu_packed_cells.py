@@ -10,15 +10,13 @@ from test_gpu_parity import _check_superchunk
 pytestmark = pytest.mark.gpu
 
 
-@pytest.fixture(scope="module", params=["staged", "direct", "bulk"])
+@pytest.fixture(scope="module", params=["staged", "direct"])
 def ctx(request):
-    """staged: default; direct: every structure straight into the arena; bulk: instants staged by bulk copies."""
+    """staged: default; direct: every structure straight into the arena."""
     from dcdf_b200 import Context
     c = Context(0)
     if request.param == "direct":
         c.set_option("stage_limit", 0)
-    if request.param == "bulk":
-        c.set_option("fast_variant", 2)
     yield c
     c.close()
 
